@@ -16,6 +16,9 @@ call (three kernels) per rank and, at N > 1, the one all-reduce of the batch sum
 
 `--impl reference` times the reference's CPU path (the oracle port: the reference EMD has no CPU
 implementation and pytorch3d is absent) on the host cores, on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller (see dump_outputs) as DIR/<name>.npy; the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -201,10 +204,7 @@ def run_reference(args):
     if rank != 0:
         return
     sample = 16
-    # K steps as asked, unless that would take more than about two minutes on this host (one step of the sample is ~0.2 s on
-    # 16 cores): then as many as fit; the line reports the number actually timed
-    t1 = max(cpu_baseline(sample, 1, 1)["ms_per_step"] * 1e-3, 1e-3)
-    steps, warm = max(1, min(args.steps, int(120.0 / t1))), max(1, min(args.warmup, 2))
+    steps, warm = args.steps, max(1, min(args.warmup, 2))
     cb = cpu_baseline(sample, steps, warm)
     line = {"metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": steps, "warmup": warm,
             "ms_per_step": cb["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -285,19 +285,38 @@ def reference_gpu_step(torch, pool, ev, emd_ms_ours):
     return out
 
 
+def dump_outputs(out_dir, step):
+    """What the caller of the timed step holds after its last call (rank 0's shard), as float32 arrays:
+    losses       the first 7 entries of the `losses` vector of pcl_chamfer_emd_step (include/pcl.h; [2:6] all-reduced over the ranks),
+    grad_chamfer (B,N,3) d Chamfer loss / d pred,
+    grad_emd     (B,N,3) d EMD loss / d pred."""
+    import numpy as np
+    step.wait()
+    arrays = {"losses": step.out[:7], "grad_chamfer": step.grad_chamfer, "grad_emd": step.grad_emd}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy().astype(np.float32))
+
+
 # ------------------------------------------------------------------------------------------------ main arm
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=300)
+    ap.add_argument("--steps", type=int, default=300, help="timed steps of the measured step (`value`)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile", action="store_true", help="value leg only (short command for ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU step; the reference arm has none")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference(args)
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)  # before the run: an unusable DIR fails in a second, not after it
 
     import numpy as np
     import torch
@@ -366,9 +385,12 @@ def main():
     #      NCCL all-reduce of the four batch sums, INSIDE the timed region --------------------------------------------------------
     step = pcl.ShardedChamferEmdStep(B_PER_GPU, NPTS, device, EPS, ITERS)
     t_wall0 = time.time()
+    # the last timed step sees pool[(W + K - 1) % n_sets]: tests/test_bench_gpu.py recomputes it to check --dump-outputs
     ms_total = timed(lambda i: step.step(*pool[i % n_sets][:2]), K, W)
     t_wall1 = time.time()
     clocks = sampler.stop(t_wall0, t_wall1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step)
     ms_per_step = ms_total / K
     value = world * B_PER_GPU * K / (ms_total * 1e-3)
     if args.profile:

@@ -1,4 +1,4 @@
-"""Shared helpers for the GPU parity tests."""
+"""Shared helpers of the tests."""
 import numpy as np
 import torch
 
@@ -61,3 +61,24 @@ def npy(t):
 def sqdist_to_match(x1, x2, asg):
     m = np.take_along_axis(np.asarray(x2), np.asarray(asg).astype(np.int64)[..., None], 1)
     return ((np.asarray(x1, dtype=np.float64) - m) ** 2).sum(-1)
+
+
+CLASSES = ['env', 'cube', 'arm', 'base', 'gripper']           # robosuite_envs/envs.py:79 (scene 'Cube')
+
+
+class LitProtocol(torch.nn.Module):
+    """The four lines of Lit.training_step (train.py:30-35) around a model that returns the recorded prediction."""
+
+    def __init__(self, prediction, loss_fn):
+        super().__init__()
+        self.prediction, self.loss_fn, self.logged = prediction, loss_fn, {}
+
+    def log(self, name, value):
+        self.logged[name] = float(value)
+
+    def training_step(self, batch, batch_idx):
+        x, y = batch
+        prediction = self.prediction
+        loss = self.loss_fn(prediction, y)
+        self.log('train_loss', loss)
+        return loss

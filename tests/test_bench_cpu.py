@@ -23,6 +23,16 @@ def test_reference_arm_json_line():
     assert line["vs_baseline"] is None and line["gpu_launches"] == 0 and "workload" in line["config"]
 
 
+def test_steps_sets_the_timed_steps_and_bad_arguments_are_refused():
+    run = lambda *a: subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *a], capture_output=True, text=True, timeout=600, cwd=ROOT)
+    out = run("--impl", "reference", "--steps", "3", "--warmup", "1")
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == 3
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        out = run(*bad)
+        assert out.returncode == 2 and "error" in out.stderr, bad
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU behaviour")
 def test_default_arm_needs_a_gpu():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1"], capture_output=True, text=True, timeout=300, cwd=ROOT)

@@ -1,9 +1,9 @@
-"""GPU side of the drop-in contract with the reference's caller (train.py:19-35,71-163).  The GPU box has no
-/root/reference, so the vectors were recorded in the build container from the REAL `create_model` + `Lit.training_step`
-with the reference's own models and losses (tests/golden/make_train_golden.py); here the recorded prediction goes
-through the caller protocol -- `loss_fn(prediction, y)`, `.log` assigned after construction (train.py:161), the loss
-logged as 'train_loss' (train.py:34) -- into the CUDA loss classes, plain and wrapped in ShardedLoss.
-tests/test_dropin_train_cpu.py runs the unmodified train.py itself where the reference is present."""
+"""GPU side of the drop-in contract with the reference's caller (train.py:19-35,71-163).  The vectors were recorded
+from the REAL `create_model` + `Lit.training_step` with the reference's own models and losses
+(tests/golden/make_train_golden.py); here the recorded prediction goes through the caller protocol --
+`loss_fn(prediction, y)`, `.log` assigned after construction (train.py:161), the loss logged as 'train_loss'
+(train.py:34) -- into the CUDA loss classes, plain and wrapped in ShardedLoss.
+tests/test_dropin_train_cpu.py replays the same vectors on any host."""
 import os
 
 import numpy as np
@@ -11,29 +11,10 @@ import pytest
 import torch
 
 import pointcloud_b200 as pcl
-from helpers import npy
+from helpers import CLASSES, LitProtocol, npy
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CLASSES = ['env', 'cube', 'arm', 'base', 'gripper']           # robosuite_envs/envs.py:79 (scene 'Cube')
-
-
-class LitProtocol(torch.nn.Module):
-    """The four lines of Lit.training_step (train.py:30-35) around a model that returns the recorded prediction."""
-
-    def __init__(self, prediction, loss_fn):
-        super().__init__()
-        self.prediction, self.loss_fn, self.logged = prediction, loss_fn, {}
-
-    def log(self, name, value):
-        self.logged[name] = float(value)
-
-    def training_step(self, batch, batch_idx):
-        x, y = batch
-        prediction = self.prediction
-        loss = self.loss_fn(prediction, y)
-        self.log('train_loss', loss)
-        return loss
 
 
 @pytest.fixture(scope="module")

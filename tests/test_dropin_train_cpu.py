@@ -1,33 +1,36 @@
-"""Drop-in test against the reference's OWN caller: /root/reference/pointcloud_vision/train.py is imported unmodified
-(`Lit`, train.py:19-68; `create_model`, train.py:71-163) with its absent third-party imports stubbed
-(tests/golden/ref_train_stubs.py), and the loss classes of this package are put where train.py:15 imports them from
-(INTEGRATION.md route 1).  `create_model` then constructs them exactly as the reference does (train.py:82,100,125),
-assigns `model.loss_fn.log = model.log` (train.py:161), and `Lit.training_step` (train.py:30-35) runs the reference's
-real PointNet2 / PointNet models into the new loss.  The same models with the same weights run into the reference's own
-loss classes; loss value, every logged scalar and the gradient of every model parameter must agree.
+"""Drop-in test against the reference's OWN caller, `Lit.training_step` + `create_model` of pointcloud_vision/train.py
+(train.py:19-35,71-163).  tests/golden/make_train_golden.py ran that caller unmodified, with the reference's real
+PointNet2 / PointNet models and its own loss classes, and recorded per model type the batch, the model's prediction, the
+loss, everything `.log` received and d loss / d prediction (tests/golden/train_golden.npz).  Here the recorded prediction
+goes through the same caller protocol -- `loss_fn(prediction, y)`, `.log` assigned after construction (train.py:161), the
+loss logged as 'train_loss' (train.py:34) -- into the loss classes of this package, constructed as train.py:82,100,125
+constructs them.  Loss value, every logged scalar and d loss / d prediction must agree; every model parameter's gradient
+is d loss / d prediction chained through the same model, so the training step is the reference's.
 
-Runs only where /root/reference exists (this container); on this CPU-only host the three CUDA entry points of the
-product classes are served by the CPU oracle (the test-only subclass used by test_sharded_cpu.py) -- the GPU side of
-the same contract is tests/test_dropin_gpu.py, against golden vectors recorded here from the reference's `Lit`."""
-import copy
+Without a CUDA device the three CUDA entry points of the product classes are served by the CPU oracle (the test-only
+subclasses of test_sharded_cpu.py); tests/test_dropin_gpu.py replays the same vectors on the CUDA losses, plain and
+wrapped in ShardedLoss."""
+import inspect
 import os
-import sys
 
 import numpy as np
 import pytest
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-import ref_train_stubs  # noqa: E402
+from helpers import CLASSES, LitProtocol
+from pointcloud_b200 import cfg
 
-pytestmark = pytest.mark.skipif(not ref_train_stubs.available(), reason="/root/reference is not present on this host")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+# The module-level surface the reference's utils.py calls (INTEGRATION.md route 2): emdModule.forward and
+# emdFunction.forward of pointcloud_vision/loss/emd/emd_module.py:74-79 and :33-61.
+REF_EMD_MODULE_FORWARD = ["self", "input1", "input2", "eps", "iters"]
+REF_EMD_FUNCTION_FORWARD = ["ctx", "xyz1", "xyz2", "eps", "iters"]
 
 
 @pytest.fixture(scope="module")
-def ref():
-    train, utils = ref_train_stubs.install()
-    return train, utils
+def tg():
+    return np.load(os.path.join(ROOT, "tests", "golden", "train_golden.npz"))
 
 
 def _product_classes():
@@ -49,55 +52,46 @@ def _batch(model_type, b, n):
     return x, target
 
 
-@pytest.mark.parametrize("model_type,backbone", [("Autoencoder", "PointNet2"), ("Segmenter", "PointNet"), ("MultiSegmenter", "PointNet")])
-def test_training_step_of_the_reference_lit_with_the_new_losses(ref, model_type, backbone, monkeypatch):
-    train, utils = ref
+@pytest.mark.parametrize("model_type", [pytest.param("Autoencoder", id="Autoencoder-PointNet2"),  # id: + the reference model that
+                                        pytest.param("Segmenter", id="Segmenter-PointNet"),        # made the recorded prediction
+                                        pytest.param("MultiSegmenter", id="MultiSegmenter-PointNet")])
+def test_training_step_of_the_reference_lit_with_the_new_losses(tg, model_type):
     emd_cls, msc_cls = _product_classes()
-    torch.manual_seed(0)
-    ref_model, _ = train.create_model(model_type, backbone, "Cube")           # the reference's own losses
-    monkeypatch.setattr(train, "EarthMoverDistance", emd_cls)                  # what `from pointcloud_b200 import ...` does
-    monkeypatch.setattr(train, "SegmentingChamferDistance", msc_cls)
-    new_model, _ = train.create_model(model_type, backbone, "Cube")
-    new_model.model.load_state_dict(copy.deepcopy(ref_model.model.state_dict()))
-    assert type(new_model).__name__ == "Lit" and isinstance(new_model.loss_fn, (emd_cls, msc_cls))
-    assert new_model.loss_fn.log == new_model.log                              # train.py:161
-    if model_type != "MultiSegmenter":                                         # ctor arguments of train.py:82,100
-        assert new_model.loss_fn.eps == train.cfg.emd_eps and new_model.loss_fn.iterations == train.cfg.emd_iterations
-        assert new_model.loss_fn.C == (None if model_type == "Autoencoder" else 5)
+    if model_type == "MultiSegmenter":                                         # train.py:116-125
+        loss_fn = msc_cls({n: CLASSES.index(n) for n in ("cube", "arm", "gripper")})
+    else:                                                                      # train.py:82,100
+        loss_fn = emd_cls(eps=cfg.emd_eps, its=cfg.emd_iterations, num_classes=None if model_type == "Autoencoder" else len(CLASSES))
+        assert loss_fn.eps == 0.005 and loss_fn.iterations == 50 and loss_fn.C == (None if model_type == "Autoencoder" else 5)
 
     x, y = _batch(model_type, 2, 2048)
-    out = []
-    for m in (ref_model, new_model):
-        m.train()
-        torch.manual_seed(1)                                                   # same dropout masks in both models
-        loss = m.training_step((x, y), 0)                                      # train.py:30-35
-        assert loss.dim() == 0
-        m.zero_grad()
-        loss.backward()
-        out.append((float(loss), {k: float(v) for k, v in m.logged.items()},
-                    {k: p.grad.clone() for k, p in m.model.named_parameters() if p.grad is not None}))
-    (l0, log0, g0), (l1, log1, g1) = out
-    assert l1 == pytest.approx(l0, rel=1e-5)
-    assert set(log1) == set(log0) and "train_loss" in log1
-    for k in log0:
-        assert log1[k] == pytest.approx(log0[k], rel=1e-5, abs=1e-9), k
-    assert set(g1) == set(g0) and len(g0) > 4
-    gmax = max(float(g.abs().max()) for g in g0.values())
-    for k in g0:  # biases in front of a BatchNorm have a mathematically zero gradient (1e-8 rounding noise): absolute floor
-        np.testing.assert_allclose(g1[k].numpy(), g0[k].numpy(), rtol=2e-4, atol=2e-5 * float(g0[k].abs().max()) + 1e-5 * gmax, err_msg=k)
+    np.testing.assert_array_equal(y.numpy(), tg[f"{model_type}_y"])            # the recorded batch is the one synth draws
+    dev = "cuda" if torch.cuda.is_available() else "cpu"
+    names = [k[len(model_type) + 6:] for k in tg.files if k.startswith(f"{model_type}_pred_")]
+    preds = {n: torch.from_numpy(tg[f"{model_type}_pred_{n}"]).to(dev).requires_grad_() for n in names}
+    lit = LitProtocol(preds[""] if names == [""] else preds, loss_fn)
+    lit.loss_fn.log = lit.log                                                  # train.py:161
+    assert lit.loss_fn.log == lit.log
+    loss = lit.training_step((x.to(dev), y.to(dev)), 0)                        # train.py:30-35
+    assert loss.dim() == 0
+    loss.backward()
+
+    assert float(loss) == pytest.approx(float(tg[f"{model_type}_loss"]), rel=1e-5)
+    want = {k[len(model_type) + 5:].replace(".", "/"): float(tg[k]) for k in tg.files if k.startswith(f"{model_type}_log_")}
+    assert set(lit.logged) == set(want) and "train_loss" in want
+    for k, v in want.items():
+        assert lit.logged[k] == pytest.approx(v, rel=1e-5, abs=1e-9), k
+    for n, p in preds.items():
+        np.testing.assert_allclose(p.grad.cpu().numpy(), tg[f"{model_type}_grad_{n}"], rtol=1e-5, atol=1e-10, err_msg=n)
 
 
-def test_module_level_route_names_resolve(ref):
+def test_module_level_route_names_resolve():
     """INTEGRATION.md route 2: utils.py stays, `emd_module` and `pytorch3d.loss` are re-exported from this package --
     the names and call surfaces the reference's utils.py uses must exist with the reference's signatures."""
-    import inspect
     import pointcloud_b200.chamfer as new_p3d_loss
     import pointcloud_b200.emd_module as new_emd
-    _, utils = ref
-    ref_emd = sys.modules["pointcloud_vision.loss.emd.emd_module"]
-    assert list(inspect.signature(new_emd.emdModule.forward).parameters) == list(inspect.signature(ref_emd.emdModule.forward).parameters)
-    assert list(inspect.signature(new_emd.emdFunction.forward).parameters) == list(inspect.signature(ref_emd.emdFunction.forward).parameters)
-    params = inspect.signature(new_p3d_loss.chamfer_distance).parameters
-    assert list(params)[:4] == ["x", "y", "x_lengths", "y_lengths"]           # utils.py:211,228
-    src = inspect.getsource(utils.FilteringChamferDistance.__call__) + inspect.getsource(utils.ChamferDistance.__call__)
-    assert "pytorch3d_loss.chamfer_distance(" in src and "y_lengths=" in src  # the only surface the reference touches
+    assert list(inspect.signature(new_emd.emdModule.forward).parameters) == REF_EMD_MODULE_FORWARD
+    assert list(inspect.signature(new_emd.emdFunction.forward).parameters) == REF_EMD_FUNCTION_FORWARD
+    sig = inspect.signature(new_p3d_loss.chamfer_distance)
+    assert list(sig.parameters)[:4] == ["x", "y", "x_lengths", "y_lengths"]  # utils.py:211,228
+    sig.bind("pred", "target")                                                 # ChamferDistance (utils.py:211)
+    sig.bind("pred", "target", y_lengths="num_points")                         # FilteringChamferDistance (utils.py:228)

@@ -1,9 +1,12 @@
 """GPU parity tests of the auction EMD kernels (through the C ABI) against
   (1) the CPU oracle (bit-exact, always),
-  (2) the UNMODIFIED reference extension built from /root/reference (oracle/_ref/emd.so) -- exact on clouds
-      where the reference's GetMax race cannot fire (oracle race_events == 0), statistical otherwise,
+  (2) the UNMODIFIED reference extension (oracle/_ref/emd.so, see oracle/build_ref.py) -- exact on clouds
+      where the reference's GetMax race cannot fire (oracle race_events == 0), statistical otherwise; where that
+      extension cannot be built, against its recorded runs (tests/golden/reference_envelope.npz),
   (3) golden vectors that went through the reference's own emd_module.py,
   (4) size-independent properties at BASELINE.json's full size (B=32, N=2048)."""
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -202,6 +205,26 @@ def test_emd_deviation_lies_inside_the_reference_nondeterminism_envelope(ref_ext
         assert (dev <= 5.0 * np.maximum(sigma, pooled) + 1e-12).all(), (dev, sigma, pooled)
         batch = runs.mean(1)                                             # the loss value of the batch, per reference run
         assert abs(ours.mean() - batch.mean()) <= 5.0 * batch.std(ddof=1) + 1e-12
+
+
+def test_emd_deviation_lies_inside_the_recorded_reference_envelope():
+    """The per-cloud statements of the test above against the reference's recorded runs instead of live ones:
+    tests/golden/reference_envelope.npz holds, per cloud of the same two batches, the mean and the spread (ddof=1) of the
+    reference's 12 runs, restored by tests/golden/make_envelope_golden.py from profiles/r2_s1_envelope.txt.  Every cloud
+    without a race event must equal the reference; the others must lie within 5 sigma of its runs.  (The batch-level
+    statement needs each run's batch value, which the recording does not keep.)"""
+    env = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_envelope.npz"))
+    b, n = 32, 2048
+    for regime in ("independent", "noisy"):
+        x1, t = synth.table_clouds(b, n, seed=0, regime=regime)
+        d, _, _ = pcl.emd_forward_raw(x1.cuda(), t[:, :, :3].contiguous().cuda(), 0.005, 50)
+        ours = np.sqrt(npy(d).astype(np.float64)).mean(1)
+        racy = env[f"{regime}_race_events"] > 0
+        sigma = env[f"{regime}_ref_std"]
+        pooled = float(np.sqrt((sigma[racy] ** 2).mean())) if racy.any() else 0.0
+        dev = np.abs(ours - env[f"{regime}_ref_mean"])
+        assert (dev[~racy] <= 1e-12).all(), regime
+        assert (dev <= 5.0 * np.maximum(sigma, pooled) + 1e-12).all(), (regime, dev, sigma, pooled)
 
 
 def test_emd_backward_matches_reference_and_oracle(ref_ext):
