@@ -113,11 +113,16 @@ PCL_API int pcl_chamfer_bwd(const void *x, int x_dtype, int64_t x_bs, int64_t x_
  * The GetMax race of the reference (emd_cuda.cu:188-191) is resolved deterministically: the
  * largest bidder index inside the +-1e-6 window wins.
  *
- * Two kernels implement the same auction bit for bit (stats[3] tells which one ran: cluster size, or 0 for the team kernel):
+ * Three paths implement the same auction bit for bit (stats[3] tells which kind ran: cluster size, or 0 for the team path):
  *   cluster path: one thread-block cluster of 1..16 CTAs per cloud for the whole auction (pcl_emd.cu);
  *   team path:    one owner CTA per cloud + worker CTAs on all other SMs that execute Bid tasks of whichever cloud is
- *                 furthest behind (pcl_emd_team.cu); needs N <= 3584, B < SM count and a workspace of pcl_emd_workspace_bytes.
- * pcl_emd_set_path picks one for the calls that follow (process-wide); AUTO = the team path wherever it is possible.
+ *                 furthest behind (pcl_emd_team.cu);
+ *   tickets path: the cluster kernel, whose many-bidder iterations are shared as tasks with worker CTAs on the SMs the
+ *                 clusters leave free and with the clusters that are already done (pcl_emd.cu + pcl_emd_team.cu).
+ * The team and tickets paths need N <= 3584, B < SM count and a workspace of pcl_emd_workspace_bytes.  Where they are possible,
+ * AUTO takes the team path for N >= 3072 and B >= 8, else the tickets path for N >= 1536 when the clusters have at most 2 CTAs,
+ * else the cluster path.  pcl_emd_set_path forces one path for the calls that follow (process-wide; for parity tests and A/B
+ * timing); a forced team or tickets path that is not possible fails with PCL_E_UNSUPPORTED.
  */
 enum { PCL_EMD_PATH_AUTO = 0, PCL_EMD_PATH_CLUSTER = 1, PCL_EMD_PATH_TEAM = 2, PCL_EMD_PATH_TICKETS = 3 };
 PCL_API int pcl_emd_set_path(int path);

@@ -734,13 +734,9 @@ inline PruneWs prune_ws(unsigned char *base, int B, int P1, int P2) {
 }
 // smallest min(P1, P2) that takes the pruned path (0: never).  Measured on B200 (profiles/r2_s2_chamfer_pruned.txt): the brute-force
 // kernel evaluates a pair in 2.5 instructions, the pruned scan in ~12 (oracle arithmetic) on the ~30 % / 6 % of the pairs that survive
-// at N = 2048 / 16384 -- the crossover is near 6000 points.  pcl_chamfer_set_prune_min / PCL_CHAMFER_PRUNE_MIN override it.
+// at N = 2048 / 16384 -- the crossover is near 6000 points.  pcl_chamfer_set_prune_min overrides it.
 int g_prune_min = -1;
-inline int prune_min() {
-    if (g_prune_min >= 0) return g_prune_min;
-    static const int v = [] { const char *e = getenv("PCL_CHAMFER_PRUNE_MIN"); return e ? atoi(e) : 6144; }();
-    return v;
-}
+inline int prune_min() { return g_prune_min >= 0 ? g_prune_min : 6144; }
 
 inline int nblk_for(int P1, int P2) {
     const int maxP = P1 > P2 ? P1 : P2;

@@ -44,8 +44,6 @@
 namespace pcl {
 namespace {
 
-// PROF: per-phase clock64() totals of thread 0 of every CTA -> prof[blockIdx.x*8 + phase] (development aid,
-// reached through the PCL_EMD_PROFILE environment variable; the product path instantiates PROF=false).
 // EXPORT: the lane-per-bidder iterations run as TICKETS (pcl_emd_tasks.cuh): the bidders' records go to the cloud's L2 region, the
 // CTAs of the cluster claim tasks dynamically (no static dealing, no waiting for the slowest CTA of the cluster), worker CTAs of a
 // second launch (emd_worker_kernel) claim them too -- they take work from the clouds that are furthest behind, which is what
@@ -54,21 +52,13 @@ namespace {
 // THREADS: 512, or 640 for clusters of at most 4 CTAs (their iterations are dominated by the lane-per-bidder scan, which gains from 20
 // warps at 80 registers: -4..9 % on early-training inputs for B >= 16; bigger clusters spend their time in the latency-bound
 // warp-per-bidder mode, where the 16-warp / 103-register build is 2-6 % faster -- profiles/r2_s2_auction_experiments.txt).
-template <bool PROF, bool EXPORT, int THREADS>
+template <bool EXPORT, int THREADS>
 __global__ void __launch_bounds__(THREADS, 1)
 emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, int pcap, int wpb_max, int items_target,
                    float *__restrict__ dist,
-                   int *__restrict__ assignment, int *__restrict__ stats, long long *__restrict__ prof,
+                   int *__restrict__ assignment, int *__restrict__ stats,
                    unsigned char *__restrict__ cold_ws, float grad_scale, float *__restrict__ grad_xyz1,
                    double *__restrict__ part, unsigned *__restrict__ ticket, float *__restrict__ sums_out, TeamWs W, int tasks_target, int export_pct, int lag_min_q, int lag_slope) {
-    long long pt[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0}, pc = 0, bid0 = 0;
-#define PCL_TICK(i)                                              \
-    if constexpr (PROF) {                                        \
-        const long long now_ = clock64();                        \
-        pt[i] += now_ - pc;                                      \
-        pc = now_;                                               \
-    }
-    if constexpr (PROF) pc = clock64();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     cg::cluster_group cluster = cg::this_cluster();
     const int cs = (int)cluster.num_blocks(), rank = (int)cluster.block_rank(), csl = __ffs(cs) - 1;  // cs is a power of two
@@ -98,7 +88,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
     unsigned tk_limit = 0;       // tickets published so far (identical in every CTA of the cluster)
     bool told_workers = false;   // this cloud has no more exported iterations: said so once (rank 0)
     cluster.sync();  // every CTA's arrays exist before anyone writes remote bids
-    PCL_TICK(0)
 
     auto pred_xyz = [&](int jp) -> float3 {
         if (S.x1) { const float4 q = S.x1[jp]; return make_float3(q.x, q.y, q.z); }
@@ -187,8 +176,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
         __syncthreads();
         sum_u += U;
         iters_run = t + 1;
-        PCL_TICK(1)
-        if constexpr (PROF) bid0 = pc;
 
         // ---- 2. Bid (emd_cuda.cu:95-179) for this CTA's share of the bidders ----------------------------
         // A warp owns 32 consecutive (= spatially close) bidders and one interleaved slice of the target tiles;
@@ -280,7 +267,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                         st_release_u64(&ctl->avail, ((unsigned long long)(unsigned)(t + 1) << 32) | (unsigned long long)tk_limit);
                     }
                 }
-                PCL_TICK(10)
             }
         }
         if (wpb) {
@@ -293,8 +279,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                 const float3 a = pred_xyz(jp);
                 unsigned lp = S.last[jp], lp34 = S.last34[jp];
                 if (flags & EMD_F_SORT) first_seeds(jp, N, lp, lp34);
-                long long wb0 = 0; int ncand = 0, nrounds = 0, nsteps = 0;
-                if constexpr (PROF) wb0 = clock64();
                 float tm = -1e9f;
                 {
                     const int k1 = (int)(lp & 0xffffu), k2 = (int)(lp >> 16);
@@ -319,7 +303,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                     bool cand = false;
                     if (tl < NT) cand = !tile_skippable(S.tlo[tl], S.thi[tl], a.x, a.y, a.z, tm);
                     unsigned cm = __ballot_sync(0xffffffffu, cand);
-                    if constexpr (PROF) ncand += __popc(cm);
                     constexpr int WC = PCL_WPB_CHUNK;
                     while (cm) {  // up to WC candidate tiles per step: WC independent filter chains per lane, one vote
                         int tix[WC];
@@ -346,7 +329,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
 #pragma unroll
                             for (int i = 0; i < WC; i++) my_evals += have[i] ? TILE : 0;
                         }
-                        if constexpr (PROF) nsteps++;
                         if (!__any_sync(0xffffffffu, any)) continue;
                         // Every lane takes ITS first surviving slot, so that one pass through the sqrt/F2F/DADD chain serves
                         // all lanes (a lane rarely has two survivors among its 4 targets; leftovers loop).
@@ -364,7 +346,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                             int ko = 0;
                             if (sel >= 0) { v = bid_value_exact(ssel, S.pf[ksel]); ko = S.tperm ? (int)S.tperm[ksel] : ksel; }
                             unsigned pm = __ballot_sync(0xffffffffu, sel >= 0);
-                            if constexpr (PROF) nrounds += 1 + (__popc(pm) << 8);
                             if (__popc(pm) > 3) {
                                 // Many survivors (a weak threshold, e.g. after an eviction): only the two largest of them can change
                                 // (best, better), so pick those with warp reductions instead of folding every survivor serially.
@@ -417,17 +398,9 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                 }
                 if (lane == 0) publish(jp, best, better, (unsigned)(bi & 0xffff) | ((unsigned)(bi2 & 0xffff) << 16),
                                        (unsigned)(k3 & 0xffff) | ((unsigned)(k4 & 0xffff) << 16));
-                if constexpr (PROF) {  // slowest warp-per-bidder scan of this CTA and iteration: cycles | candidate tiles | steps | exact rounds | survivors
-                    if (lane == 0 && prof && blockIdx.x < 4 && t < 50) {
-                        const unsigned long long v = ((unsigned long long)(clock64() - wb0) << 40) | ((unsigned long long)(ncand & 0xff) << 32) |
-                                                     ((unsigned long long)(nsteps & 0xff) << 24) | ((unsigned long long)(nrounds & 0xff) << 16) | (unsigned long long)((nrounds >> 8) & 0xffff);
-                        atomicMax((unsigned long long *)&prof[(size_t)gridDim.x * 16 + 256 + blockIdx.x * 50 + t], v);
-                    }
-                }
                 if (lane == 0) b = atomicAdd(work_ctr, 1);  // next bidder of this warp
                 b = __shfl_sync(0xffffffffu, b, 0);
             }
-            PCL_TICK(8)
         } else {
         // seed thresholds once per bidder (not once per slice item): parked in the increment field of the bidder's own
         // bid slot, which nobody else touches before this CTA publishes that bid
@@ -439,7 +412,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
             pub_cur[jp].y = __float_as_uint(seed_threshold(S, lp, lp34, N, a.x, a.y, a.z));
         }
         __syncthreads();
-        PCL_TICK(6)
         for (int it = wid;;) {
             if (it >= Gn * KS) break;
             const int g = it % Gn, sl = it / Gn;
@@ -469,7 +441,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
             if (lane == 0) it = atomicAdd(work_ctr, 1);  // next work item of this warp
             it = __shfl_sync(0xffffffffu, it, 0);
         }
-        PCL_TICK(2)
         }
         if (!wpb && KS > 1) {
             __syncthreads();
@@ -509,17 +480,8 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                 }
                 __syncthreads();
             }
-            PCL_TICK(9)
             for (int b = tid; b < Uc; b += T) publish(S.unass[pos(b)], S.pbest[b], S.pbetter[b], S.pbi[b], S.pbi34[b]);
         }
-        if constexpr (PROF) {
-            if (blockIdx.x == 0 && tid == 0 && prof && t < 50) {
-                prof[(size_t)gridDim.x * 16 + t * 4] = U;
-                prof[(size_t)gridDim.x * 16 + t * 4 + 1] = clock64() - bid0;
-                prof[(size_t)gridDim.x * 16 + t * 4 + 2] = KS * 1000 + Gn;
-            }
-        }
-        PCL_TICK(7)
         if constexpr (EXPORT) {
             if (!wpb && rank == 0 && wid == NW - 1 && W.nworkers > 0) {  // export share of the NEXT iteration from the mean lag (in iterations)
                 const int nb = (int)gridDim.x / cs;
@@ -554,7 +516,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                     __syncthreads();
                     if (tid == 0) { __threadfence(); atomicAdd(&ctl->done, 1u); }
                 }
-                PCL_TICK(11)
                 if (rank == 0 && tid == 0) {  // the tickets other CTAs hold (the barrier below makes the whole cluster wait with this thread)
                     for (unsigned spin = 0; ld_acquire_u32(&ctl->done) < tk_limit; spin++) {
                         if (spin > PCL_SPIN_LIMIT) __trap();
@@ -564,10 +525,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
             }
         }
         cluster.sync();  // all bids of this iteration are visible in every CTA
-        if constexpr (PROF) {
-            if (blockIdx.x == 0 && tid == 0 && prof && t < 50) prof[(size_t)gridDim.x * 16 + t * 4 + 3] = clock64() - pc;
-        }
-        PCL_TICK(3)
         if constexpr (EXPORT) {
             if (ticketed) {  // all bids of the iteration are in the cloud's L2 region: bring them home, indexed by bidder
                 const uint4 *const g_pub = reinterpret_cast<const uint4 *>(cl + W.o_pub);
@@ -578,7 +535,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                     S.last34[jp] = rec.z;
                 }
                 __syncthreads();
-                PCL_TICK(9)
             }
         }
 
@@ -643,7 +599,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
         }
         __syncthreads();
         cur ^= 1;
-        PCL_TICK(4)
     }
 
     if constexpr (EXPORT) {
@@ -704,12 +659,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
             }
         }
     }
-    PCL_TICK(5)
-    if constexpr (PROF) {
-        if (tid == 0 && prof)
-            for (int i = 0; i < 16; i++) prof[(size_t)blockIdx.x * 16 + i] = pt[i];
-    }
-#undef PCL_TICK
     if (stats) {  // uniform over the grid
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {
@@ -737,7 +686,7 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
         // and by now that cloud exports a large share of its iterations) until every cloud is past its exported iterations.
         if (W.nworkers > 0) {
             __syncthreads();
-            team_worker<THREADS>(S, W, (int)gridDim.x / cs, N, eps, (int)blockIdx.x, 0, nullptr);
+            team_worker<THREADS>(S, W, (int)gridDim.x / cs, N, eps, (int)blockIdx.x, 0);
         }
     }
 }
@@ -851,9 +800,8 @@ int sm_count_or_default() {
     return di.sm_count;
 }
 
-struct EmdEnv;
-const EmdEnv &emd_env();
-int pick_cluster_impl(int B, int N, int sm_count, size_t smem, cudaStream_t st, int forced_cs) {
+// cluster size of the launch: cluster_size_for, halved until B clusters of it are resident at once with `smem` bytes per CTA
+int pick_cluster(int B, int sm_count, size_t smem, cudaStream_t st) {
     // the occupancy query costs a few microseconds of host time: remembered per (device, B, shared-memory size)
     struct Memo { int dev, B; size_t smem; int cs; };
     static thread_local Memo memo[8];
@@ -863,7 +811,6 @@ int pick_cluster_impl(int B, int N, int sm_count, size_t smem, cudaStream_t st, 
     for (int i = 0; i < memo_n; i++)
         if (memo[i].dev == dev && memo[i].B == B && memo[i].smem == smem) return memo[i].cs;
     int cs = cluster_size_for(B, sm_count);
-    if (forced_cs > 0) cs = forced_cs;  // development aid (PCL_EMD_CS)
     // Are B clusters of this size resident at the same time with this much shared memory?  A cluster lives inside one GPC, so
     // fewer clusters than B * cs <= SM count suggests may fit (8 clusters of 16 never do on a B200); a second wave would
     // double the time of the launch, half the cluster size costs far less.
@@ -875,44 +822,19 @@ int pick_cluster_impl(int B, int N, int sm_count, size_t smem, cudaStream_t st, 
         at[0].val.clusterDim.x = cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
         cfg.attrs = at; cfg.numAttrs = 1;
         int ncl = 0;
-        cudaError_t e = cudaOccupancyMaxActiveClusters(&ncl, emd_auction_kernel<false, false, EMD_THREADS>, &cfg);
+        cudaError_t e = cudaOccupancyMaxActiveClusters(&ncl, emd_auction_kernel<false, EMD_THREADS>, &cfg);
         if (e == cudaSuccess && ncl >= B) break;
         (void)cudaGetLastError();
         cs >>= 1;
     }
-    (void)N;
     memo[memo_n < 8 ? memo_n++ : (memo_n = 8, 7)] = Memo{dev, B, smem, cs};
     return cs;
 }
 
-// development aids, read once per process: PCL_EMD_NO_SORT, PCL_EMD_PCAP, PCL_EMD_WPB, PCL_EMD_ITEMS, PCL_EMD_PROFILE, PCL_EMD_TEAM*
-struct EmdEnv { bool no_sort, profile; int pcap, wpb, items, cs, threads, path, team_tasks, team_local, team_wpb, team_grid, team_idle, team_export, team_lagmin, team_slope; };
-const EmdEnv &emd_env() {
-    static const EmdEnv e = [] {
-        EmdEnv v;
-        v.no_sort = getenv("PCL_EMD_NO_SORT") != nullptr;
-        v.profile = getenv("PCL_EMD_PROFILE") != nullptr;
-        const char *s;
-        v.pcap = (s = getenv("PCL_EMD_PCAP")) ? atoi(s) * 32 : 0;
-        v.wpb = (s = getenv("PCL_EMD_WPB")) ? atoi(s) : -1;
-        v.items = (s = getenv("PCL_EMD_ITEMS")) ? atoi(s) : 0;
-        v.cs = (s = getenv("PCL_EMD_CS")) ? atoi(s) : 0;
-        v.threads = (s = getenv("PCL_EMD_THREADS")) ? atoi(s) : 0;  // 512: never the 640-thread build
-        v.path = (s = getenv("PCL_EMD_PATH")) ? atoi(s) : 0;               // PCL_EMD_PATH_* of include/pcl.h when pcl_emd_set_path says AUTO
-        v.team_export = (s = getenv("PCL_EMD_TEAM_EXPORT")) ? atoi(s) : -1;  // percent of a lane-per-bidder iteration's bidders exported as tickets
-        v.team_lagmin = (s = getenv("PCL_EMD_TEAM_LAGMIN")) ? atoi(s) : -1;  // quarter iterations behind the mean from which a cloud exports
-        v.team_slope = (s = getenv("PCL_EMD_TEAM_SLOPE")) ? atoi(s) : -1;    // exported percent per iteration of lag
-        v.team_idle = (s = getenv("PCL_EMD_TEAM_IDLE")) ? atoi(s) : 0;     // cycles without a ticket after which a worker of the ticket path leaves
-        v.team_tasks = (s = getenv("PCL_EMD_TEAM_TASKS")) ? atoi(s) : 0;   // tasks per cloud and iteration the owner aims at
-        v.team_local = (s = getenv("PCL_EMD_TEAM_LOCAL")) ? atoi(s) : -1;  // the owner works alone with at most this many bidders
-        v.team_wpb = (s = getenv("PCL_EMD_TEAM_WPB")) ? atoi(s) : -1;      // warp-per-bidder tasks with at most this many bidders
-        v.team_grid = (s = getenv("PCL_EMD_TEAM_GRID")) ? atoi(s) : 0;     // CTAs of the team launch / clusters + workers of the ticket path (default: one per SM; -1: no workers)
-        return v;
-    }();
-    return e;
-}
-
-int pick_cluster(int B, int N, int sm_count, size_t smem, cudaStream_t st) { return pick_cluster_impl(B, N, sm_count, smem, st, emd_env().cs); }
+// the instantiations of the cluster kernel, by [EXPORT][THREADS == EMD_THREADS_WIDE]
+using AuctionKernel = decltype(&emd_auction_kernel<false, EMD_THREADS>);
+const AuctionKernel auction_kernels[2][2] = {{emd_auction_kernel<false, EMD_THREADS>, emd_auction_kernel<false, EMD_THREADS_WIDE>},
+                                             {emd_auction_kernel<true, EMD_THREADS>, emd_auction_kernel<true, EMD_THREADS_WIDE>}};
 
 }  // namespace
 
@@ -920,10 +842,9 @@ int pick_cluster(int B, int N, int sm_count, size_t smem, cudaStream_t st) { ret
 size_t emd_team_workspace_bytes(int B, int N);
 int emd_team_launch(const Pts &p1, const Pts &p2, int B, int N, float eps, int iters, int flags, int pcap, int wpb_max, int tasks_target,
                     int local_max, int grid, size_t smem, float *dist, int *assignment, int *stats, void *team_ws, float grad_scale,
-                    float *grad_xyz1, double *part, unsigned *ticket, float *sums, long long *prof, cudaStream_t st);
+                    float *grad_xyz1, double *part, unsigned *ticket, float *sums, cudaStream_t st);
 
-int emd_worker_launch(void *team_ws, int B, int N, float eps, int flags, int pcap, int nworkers, size_t smem, long long idle_limit,
-                      long long *prof, cudaStream_t st);
+int emd_worker_launch(void *team_ws, int B, int N, float eps, int flags, int pcap, int nworkers, size_t smem, cudaStream_t st);
 
 static int g_emd_path = PCL_EMD_PATH_AUTO;  // pcl_emd_set_path
 
@@ -959,22 +880,21 @@ extern "C" int pcl_emd_set_path(int path) {
     return PCL_OK;
 }
 
-// workspace layout: [ticket, 256 B][per-CTA partial sums of the fused epilogue, fp64][the rest: reduction partials of
-// pcl_emd_weighted_reduce | profile counters | cold auction state for large N]
+// workspace layout: [ticket, 256 B][per-CTA partial sums of the fused epilogue, fp64][reduction partials of
+// pcl_emd_weighted_reduce | cold auction state for large N][task workspace of the team / ticket paths]
 static size_t emd_fused_bytes(int B) {
     const size_t ctas = (size_t)(B > 256 ? B : 256);  // grid = B * cs <= max(SM count, B)
     return 256 + align_up(ctas * sizeof(double), 256);
 }
 
 extern "C" size_t pcl_emd_workspace_bytes(int B, int N) {
-    const size_t red = (size_t)RED_BLOCKS * 2 * sizeof(double), prof = ((size_t)(B > 16 ? B : 16) * 16 * 16 + 512) * sizeof(long long);  // >= 16 counters for each of up to 256 CTAs
+    const size_t red = (size_t)RED_BLOCKS * 2 * sizeof(double);
     size_t cold = 0;
     if (N > EMD_SMEM_ONLY_N && B > 0) {  // large clouds: per-CTA global region for the cold state, sized for the largest cluster
         const int cs = cluster_size_for(B, sm_count_or_default());  // the same rule pick_cluster starts from (it can only go down)
         cold = (size_t)B * cs * ((emd_cold_bytes(N) + 255) / 256 * 256);
     }
-    const size_t m = red > prof ? red : prof;
-    return emd_fused_bytes(B) + align_up(m > cold ? m : cold, 256) + emd_team_workspace_bytes(B, N);  // the team region is the tail
+    return emd_fused_bytes(B) + align_up(red > cold ? red : cold, 256) + emd_team_workspace_bytes(B, N);  // the team region is the tail
 }
 
 static int emd_check(const void *xyz1, int dtype1, const void *xyz2, int dtype2, int B, int N, const char *who) {
@@ -1030,33 +950,29 @@ int pcl::emd_fwd_fused_impl(const void *xyz1, int dtype1, int64_t bs1, int64_t r
     }
     if (N >= 1024 && N <= EMD_SMEM_ONLY_N && emd_smem_bytes(N, EMD_F_SORT) <= (size_t)di.max_smem_optin) flags |= EMD_F_SORT;
     if (N <= EMD_SMEM_ONLY_N && emd_smem_bytes(N, flags | EMD_F_X1) <= (size_t)di.max_smem_optin) flags |= EMD_F_X1;
-    const EmdEnv &env = emd_env();
-    if (env.no_sort) flags &= ~EMD_F_SORT;  // development aid: natural order (no spatial pruning benefit)
     static thread_local int attr_dev = -1;
     int dev = 0;
     PCL_CUDA(cudaGetDevice(&dev));
     if (attr_dev != dev) {
-        const void *kernels[6] = {(const void *)emd_auction_kernel<false, false, EMD_THREADS>, (const void *)emd_auction_kernel<true, false, EMD_THREADS>,
-                                  (const void *)emd_auction_kernel<false, true, EMD_THREADS>, (const void *)emd_auction_kernel<true, true, EMD_THREADS>,
-                                  (const void *)emd_auction_kernel<false, false, EMD_THREADS_WIDE>, (const void *)emd_auction_kernel<false, true, EMD_THREADS_WIDE>};
-        for (const void *k : kernels) {
-            PCL_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, di.max_smem_optin));
-            PCL_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-            // The largest shared-memory carveout (228 KB) instead of the smallest that holds the 183 KB state (196 KB): the 44 KB that are
-            // left let one CTA of another kernel (Chamfer in the composite step: 17 KB, 96 registers) share the SM with an auction CTA.
-            // Late-training steps, where Chamfer on the 20 free SMs ends the step, 376 -> 357 us; early-training steps 1514 -> 1529 us
-            // (the guest competes for issue slots).  Training spends most of its steps in the late regime.  PCL_EMD_NO_CARVEOUT: off.
-            if (!getenv("PCL_EMD_NO_CARVEOUT")) PCL_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        for (const auto &by_threads : auction_kernels) {
+            for (const AuctionKernel k : by_threads) {
+                PCL_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, di.max_smem_optin));
+                PCL_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+                // The largest shared-memory carveout (228 KB) instead of the smallest that holds the 183 KB state (196 KB): the 44 KB that
+                // are left let one CTA of another kernel (Chamfer in the composite step: 17 KB, 96 registers) share the SM with an auction
+                // CTA.  Late-training steps, where Chamfer on the 20 free SMs ends the step, 376 -> 357 us; early-training steps
+                // 1514 -> 1529 us (the guest competes for issue slots).  Training spends most of its steps in the late regime.
+                PCL_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+            }
         }
         attr_dev = dev;
     }
     // cluster size first (with the 512-thread configuration), then the CTA size that goes with it
     int pcap = 2 * EMD_THREADS;  // room for 32 work items with partials; fall back to 16 when shared memory is tight
-    if (env.pcap > 0) pcap = env.pcap;  // development aid: work items with partials
     while (pcap > EMD_THREADS && emd_smem_bytes(N, flags, pcap) > (size_t)di.max_smem_optin) pcap -= EMD_THREADS;
     size_t smem = emd_smem_bytes(N, flags, pcap);
     if (smem > (size_t)di.max_smem_optin) { set_error("emd_fwd: N=%d needs %zu B shared memory (> %d)", N, smem, di.max_smem_optin); return PCL_E_UNSUPPORTED; }
-    const int cs = pick_cluster(B, N, di.sm_count, smem, st);
+    const int cs = pick_cluster(B, di.sm_count, smem, st);
     const int pcap512 = pcap;  // the team kernel always runs 512 threads
     const size_t smem512 = smem;
     int threads = EMD_THREADS;
@@ -1064,12 +980,11 @@ int pcl::emd_fwd_fused_impl(const void *xyz1, int dtype1, int64_t bs1, int64_t r
     double *part = sums ? (double *)((unsigned char *)workspace + 256) : nullptr;
     if (sums) PCL_CUDA(cudaMemsetAsync(ticket, 0, sizeof(unsigned), st));
     const Pts p1{xyz1, bs1, rs1, dtype1}, p2{xyz2, bs2, rs2, dtype2};
-    // Which kernel (include/pcl.h, pcl_emd_set_path; development aid PCL_EMD_PATH):
+    // Which kernel (include/pcl.h, pcl_emd_set_path):
     //   tickets: cluster kernel whose lane-per-bidder iterations run as tickets + worker CTAs on the SMs the clusters leave free;
     //   team:    one owner CTA per cloud + workers (pcl_emd_team.cu);
     //   cluster: the plain cluster kernel (the only one for large clouds, B >= SM count or without a workspace).
     int path = g_emd_path;
-    if (path == PCL_EMD_PATH_AUTO && env.path > 0) path = env.path;
     const size_t team_bytes = emd_team_workspace_bytes(B, N), all_bytes = pcl_emd_workspace_bytes(B, N);
     const bool can = !(flags & EMD_F_COLD) && B < di.sm_count && team_bytes > 0 && workspace && workspace_bytes >= all_bytes;
     if ((path == PCL_EMD_PATH_TEAM || path == PCL_EMD_PATH_TICKETS) && !can) {
@@ -1087,26 +1002,21 @@ int pcl::emd_fwd_fused_impl(const void *xyz1, int dtype1, int64_t bs1, int64_t r
         else if (can && N >= 1536 && cs <= 2) path = PCL_EMD_PATH_TICKETS;  // (clusters of 4 with many free SMs gain 1-3 % on the mix: not worth the second launch)
     }
     // CTA size: 640 threads where the lane-per-bidder scan dominates (plain clusters of <= 4 CTAs, ticket path with clusters of <= 2)
-    if (!(flags & EMD_F_COLD) && env.threads != 512 && !env.profile && env.pcap <= 0 &&
-        ((path == PCL_EMD_PATH_CLUSTER && cs <= 4) || (path == PCL_EMD_PATH_TICKETS && cs <= 2))) {
+    if (!(flags & EMD_F_COLD) && ((path == PCL_EMD_PATH_CLUSTER && cs <= 4) || (path == PCL_EMD_PATH_TICKETS && cs <= 2))) {
         const int pc = 2 * EMD_THREADS_WIDE;
         if (emd_smem_bytes(N, flags, pc) <= (size_t)di.max_smem_optin) { threads = EMD_THREADS_WIDE; pcap = pc; smem = emd_smem_bytes(N, flags, pcap); }
     }
     const int warps = threads / 32;
-    int wpb_max = 6 * warps;  // at most this many bidders per CTA: warp-per-bidder scan (swept on config 2: 48..128 at 16 warps)
-    if (env.wpb >= 0) wpb_max = env.wpb;  // development aid
-    int items_target = 2 * warps;  // work items per CTA and iteration in the lane-per-bidder mode (dynamic queue; swept 8..128 on config 2)
-    if (env.items > 0) items_target = env.items;  // development aid
+    const int wpb_max = 6 * warps;  // at most this many bidders per CTA: warp-per-bidder scan (swept on config 2: 48..128 at 16 warps)
+    const int items_target = 2 * warps;  // work items per CTA and iteration in the lane-per-bidder mode (dynamic queue; swept 8..128 on config 2)
     void *team_ws = can ? (unsigned char *)workspace + (all_bytes - team_bytes) : nullptr;
-    long long *prof_team = env.profile && workspace ? (long long *)((unsigned char *)workspace + emd_fused_bytes(B)) : nullptr;  // 16 int64 per CTA, <= 256 CTAs
     if (path == PCL_EMD_PATH_TEAM) {
-        int grid = env.team_grid > 0 ? env.team_grid : di.sm_count;
-        if (grid < B) grid = B;
-        const int tasks_target = env.team_tasks > 0 ? env.team_tasks : (3 * grid / B + 1) / 2;  // ~1.5 tasks per CTA that can work on a cloud
-        const int local_max = env.team_local >= 0 ? env.team_local : 32;
-        const int team_wpb = env.team_wpb >= 0 ? env.team_wpb : 4 * EMD_WPB_MAX;
+        const int grid = max(di.sm_count, B);
+        const int tasks_target = (3 * grid / B + 1) / 2;  // ~1.5 tasks per CTA that can work on a cloud
+        const int local_max = 32;                         // the owner works alone with at most this many bidders
+        const int team_wpb = 4 * EMD_WPB_MAX;             // warp-per-bidder tasks with at most this many bidders
         return emd_team_launch(p1, p2, B, N, eps, iters, flags, pcap512, team_wpb, tasks_target, local_max, grid, smem512, dist, (int *)assignment,
-                               (int *)stats, team_ws, grad_scale, grad_xyz1, part, ticket, sums, prof_team, st);
+                               (int *)stats, team_ws, grad_scale, grad_xyz1, part, ticket, sums, st);
     }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(B * cs); cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = smem; cfg.stream = st;
@@ -1114,58 +1024,39 @@ int pcl::emd_fwd_fused_impl(const void *xyz1, int dtype1, int64_t bs1, int64_t r
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
-    unsigned char *rest = workspace ? (unsigned char *)workspace + emd_fused_bytes(B) : nullptr;  // behind the fused-epilogue header
-    const size_t rest_bytes = workspace_bytes > emd_fused_bytes(B) ? workspace_bytes - emd_fused_bytes(B) : 0;
-    const bool prof_ok = env.profile && !(flags & EMD_F_COLD) && rest && rest_bytes >= ((size_t)B * cs * 16 + 512) * sizeof(long long);
-    if (path == PCL_EMD_PATH_TICKETS) {
+    unsigned char *cold_ws = (flags & EMD_F_COLD) ? (unsigned char *)workspace + emd_fused_bytes(B) : nullptr;  // behind the fused-epilogue header
+    const bool exported = path == PCL_EMD_PATH_TICKETS;
+    TeamWs W = {};  // zero for the plain cluster kernel, like the four ticket-path parameters below
+    int tasks_target = 0, export_pct = 0, lag_min_q = 0, lag_slope = 0, nworkers = 0;
+    WorkerStream *ws = nullptr;
+    if (exported) {
         // dedicated worker CTAs (a second launch) on the SMs the clusters leave free; besides them, the CTAs of every cluster whose
         // auction is over serve tickets until the last cloud is done (W.nworkers > 0 switches the export machinery on)
-        int nworkers = env.team_grid > 0 ? env.team_grid - B * cs : di.sm_count - B * cs;
-        if (nworkers < 0 || env.team_grid == -1 || worker_policy == EMD_WORKERS_NONE_DEDICATED) nworkers = 0;
-        const int tasks_target = env.team_tasks > 0 ? env.team_tasks : max(4, (2 * (nworkers > 0 ? nworkers : di.sm_count - B * cs) + B - 1) / B);  // exported tickets per cloud and iteration: ~2 per worker that serves the cloud, at least 4 (swept 2..8 at B=32)
-                int export_pct = env.team_export >= 0 ? env.team_export : 50;  // upper limit of the exported share (percent)
-        if (export_pct > 60) export_pct = 60;
-        const int lag_min_q = env.team_lagmin >= 0 ? env.team_lagmin : 4;   // a cloud exports when it lags >= this many quarter iterations behind the mean
-        const int lag_slope = env.team_slope >= 0 ? env.team_slope : 5;     // exported percent = 20 + slope * lag
-        const TeamWs W = team_ws_make(team_ws, B, N, nworkers > 0 ? nworkers : 1);
+        nworkers = di.sm_count - B * cs;
+        if (nworkers < 0 || worker_policy == EMD_WORKERS_NONE_DEDICATED) nworkers = 0;
+        tasks_target = max(4, (2 * (nworkers > 0 ? nworkers : di.sm_count - B * cs) + B - 1) / B);  // exported tickets per cloud and iteration: ~2 per worker that serves the cloud, at least 4 (swept 2..8 at B=32)
+        export_pct = 50;  // upper limit of the exported share (percent; the kernel needs <= 60)
+        lag_min_q = 4;    // a cloud exports when it lags >= this many quarter iterations behind the mean
+        lag_slope = 5;    // exported percent = 20 + slope * lag
+        W = team_ws_make(team_ws, B, N, nworkers > 0 ? nworkers : 1);
         PCL_CUDA(cudaMemsetAsync(team_ws, 0, team_ctl_bytes(B), st));
-        WorkerStream *ws = nullptr;
         if (nworkers > 0) {
             int rc2 = worker_stream(&ws);
             if (rc2) return rc2;
             PCL_CUDA(cudaEventRecord(ws->fork, st));  // the workers need the zeroed control block, nothing else
         }
-        if (prof_ok) {
-            PCL_CUDA(cudaLaunchKernelEx(&cfg, emd_auction_kernel<true, true, EMD_THREADS>, p1, p2, N, eps, iters, flags, pcap, wpb_max, items_target, dist, (int *)assignment, (int *)stats, (long long *)rest, (unsigned char *)nullptr, grad_scale, grad_xyz1, part, ticket, sums, W, tasks_target, export_pct, lag_min_q, lag_slope));
-        } else {
-            if (threads == EMD_THREADS_WIDE) {
-                PCL_CUDA(cudaLaunchKernelEx(&cfg, emd_auction_kernel<false, true, EMD_THREADS_WIDE>, p1, p2, N, eps, iters, flags, pcap, wpb_max, items_target, dist, (int *)assignment, (int *)stats, (long long *)nullptr, (unsigned char *)nullptr, grad_scale, grad_xyz1, part, ticket, sums, W, tasks_target, export_pct, lag_min_q, lag_slope));
-            } else {
-                PCL_CUDA(cudaLaunchKernelEx(&cfg, emd_auction_kernel<false, true, EMD_THREADS>, p1, p2, N, eps, iters, flags, pcap, wpb_max, items_target, dist, (int *)assignment, (int *)stats, (long long *)nullptr, (unsigned char *)nullptr, grad_scale, grad_xyz1, part, ticket, sums, W, tasks_target, export_pct, lag_min_q, lag_slope));
-            }
-        }
-        if (nworkers > 0) {
-            // Launched AFTER the clusters (they must not find their SMs taken) on a stream of their own; a worker leaves when every
-            // cloud is past its exported iterations, or after ~100 us without a ticket (so it can never starve a cluster of its SM).
-            PCL_CUDA(cudaStreamWaitEvent(ws->side, ws->fork, 0));
-            int rc2 = emd_worker_launch(team_ws, B, N, eps, flags, pcap, nworkers, smem, env.team_idle > 0 ? (long long)env.team_idle : 200000LL,
-                                        prof_ok ? (long long *)rest + (size_t)B * cs * 16 + 512 : nullptr, ws->side);
-            if (rc2) return rc2;
-            PCL_CUDA(cudaEventRecord(ws->join, ws->side));
-            PCL_CUDA(cudaStreamWaitEvent(st, ws->join, 0));  // the caller's next operation on `stream` comes after the workers
-        }
-        return PCL_OK;
     }
-    const TeamWs W0 = {};
-    // development aid: PCL_EMD_PROFILE=1 makes the workspace receive per-phase clock totals (B*cs*16 int64)
-    if (prof_ok) {
-        PCL_CUDA(cudaLaunchKernelEx(&cfg, emd_auction_kernel<true, false, EMD_THREADS>, p1, p2, N, eps, iters, flags, pcap, wpb_max, items_target, dist, (int *)assignment, (int *)stats, (long long *)rest, (unsigned char *)nullptr, grad_scale, grad_xyz1, part, ticket, sums, W0, 0, 0, 0, 0));
-    } else {
-        if (threads == EMD_THREADS_WIDE) {
-            PCL_CUDA(cudaLaunchKernelEx(&cfg, emd_auction_kernel<false, false, EMD_THREADS_WIDE>, p1, p2, N, eps, iters, flags, pcap, wpb_max, items_target, dist, (int *)assignment, (int *)stats, (long long *)nullptr, (unsigned char *)((flags & EMD_F_COLD) ? rest : nullptr), grad_scale, grad_xyz1, part, ticket, sums, W0, 0, 0, 0, 0));
-        } else {
-            PCL_CUDA(cudaLaunchKernelEx(&cfg, emd_auction_kernel<false, false, EMD_THREADS>, p1, p2, N, eps, iters, flags, pcap, wpb_max, items_target, dist, (int *)assignment, (int *)stats, (long long *)nullptr, (unsigned char *)((flags & EMD_F_COLD) ? rest : nullptr), grad_scale, grad_xyz1, part, ticket, sums, W0, 0, 0, 0, 0));
-        }
+    PCL_CUDA(cudaLaunchKernelEx(&cfg, auction_kernels[exported][threads == EMD_THREADS_WIDE], p1, p2, N, eps, iters, flags, pcap, wpb_max,
+                                items_target, dist, (int *)assignment, (int *)stats, cold_ws, grad_scale, grad_xyz1, part, ticket, sums, W,
+                                tasks_target, export_pct, lag_min_q, lag_slope));
+    if (nworkers > 0) {
+        // Launched AFTER the clusters (they must not find their SMs taken) on a stream of their own; a worker leaves when every
+        // cloud is past its exported iterations, or after ~100 us without a ticket (so it can never starve a cluster of its SM).
+        PCL_CUDA(cudaStreamWaitEvent(ws->side, ws->fork, 0));
+        int rc2 = emd_worker_launch(team_ws, B, N, eps, flags, pcap, nworkers, smem, ws->side);
+        if (rc2) return rc2;
+        PCL_CUDA(cudaEventRecord(ws->join, ws->side));
+        PCL_CUDA(cudaStreamWaitEvent(st, ws->join, 0));  // the caller's next operation on `stream` comes after the workers
     }
     return PCL_OK;
 }

@@ -22,7 +22,7 @@ struct __align__(128) TeamCtl {  // one per cloud; zeroed by the host call befor
 };
 static_assert(sizeof(TeamCtl) == 128, "TeamCtl is one 128-byte line");
 
-struct TeamWs {
+struct __align__(16) TeamWs {  // 16-byte aligned: as a kernel parameter, pairs of its fields are read with one 128-bit constant load
     TeamCtl *ctl;          // B control lines
     unsigned *finished;    // number of owners that are done
     unsigned char *clouds; // per-cloud mirror regions
@@ -310,15 +310,13 @@ __device__ __forceinline__ void team_run_task(const EmdSmem &S, int NT, float ep
 
 // widx: index of this worker (home cloud = widx mod B); idle_limit: leave after this many cycles without a ticket (0: never)
 template <int THREADS>
-__device__ void team_worker(const EmdSmem &S, const TeamWs &W, int B, int N, float eps, int widx, long long idle_limit, long long *prof) {
+__device__ void team_worker(const EmdSmem &S, const TeamWs &W, int B, int N, float eps, int widx, long long idle_limit) {
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const int n8 = (N + 7) / 8 * 8, n32 = (N + 31) / 32 * 32, NT = n32 / TILE;
     int cached_c = -1, cached_t = -1;
     const int home = widx % B;
     long long last_work = clock64();
     unsigned long long my_evals = 0ull;
-    long long pt[8] = {0, 0, 0, 0, 0, 0, 0, 0}, pc = prof ? clock64() : 0;  // development aid: idle, load, run, finish cycles; tasks, reloads
-#define PCL_WTICK(i) if (prof) { const long long now_ = clock64(); pt[i] += now_ - pc; pc = now_; }
     for (;;) {
         if (wid == 0) {
             // Which task next?  First the worker's HOME cloud (workers are dealt to the clouds round-robin: one control line, no
@@ -373,11 +371,7 @@ __device__ void team_worker(const EmdSmem &S, const TeamWs &W, int B, int N, flo
         }
         __syncthreads();
         const int c = S.wsum[56];
-        PCL_WTICK(0)
-        if (c < 0) {
-            if (prof && tid == 0) for (int i = 0; i < 8; i++) prof[i] = pt[i];
-            return;
-        }
+        if (c < 0) return;
         const unsigned ticket = (unsigned)S.wsum[57];
         last_work = clock64();
         const TeamCtl *ctl = &W.ctl[c];
@@ -414,15 +408,11 @@ __device__ void team_worker(const EmdSmem &S, const TeamWs &W, int B, int N, flo
                 }
             }
             cached_c = c; cached_t = t;
-            pt[5]++;
             __syncthreads();
         }
-        pt[4]++;
-        PCL_WTICK(1)
         // (team_run_task starts with a block barrier: the copies are visible to every warp before the first scan)
         team_run_task<THREADS>(S, NT, eps, h, (int)ticket - base, reinterpret_cast<const float4 *>(cl + W.o_brec),
                       reinterpret_cast<const unsigned short *>(cl + W.o_jp), reinterpret_cast<uint4 *>(const_cast<unsigned char *>(cl) + W.o_pub), my_evals);
-        PCL_WTICK(2)
         // statistics: evaluations executed for cloud c (before the task counts as done: the owner reads the total at the end)
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) my_evals += __shfl_xor_sync(0xffffffffu, my_evals, o);
@@ -431,9 +421,7 @@ __device__ void team_worker(const EmdSmem &S, const TeamWs &W, int B, int N, flo
         __threadfence();   // this thread's bids are visible device-wide ...
         __syncthreads();   // ... for every thread of the CTA, before the task counts as done
         if (tid == 0) { __threadfence(); atomicAdd(&W.ctl[c].done, 1u); }
-        PCL_WTICK(3)
     }
-#undef PCL_WTICK
 }
 
 }  // namespace

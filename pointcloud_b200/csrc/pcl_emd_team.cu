@@ -26,15 +26,13 @@ namespace {
 __global__ void __launch_bounds__(EMD_THREADS, 1)
 emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flags, int pcap, int wpb_max, int tasks_target, int local_max,
                 float *__restrict__ dist, int *__restrict__ assignment, int *__restrict__ stats, TeamWs W, float grad_scale,
-                float *__restrict__ grad_xyz1, double *__restrict__ part, unsigned *__restrict__ ticket, float *__restrict__ sums_out,
-                long long *__restrict__ prof) {
+                float *__restrict__ grad_xyz1, double *__restrict__ part, unsigned *__restrict__ ticket, float *__restrict__ sums_out) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int tid = threadIdx.x, T = EMD_THREADS, lane = tid & 31, wid = tid >> 5;
+    // each branch carves its own view of shared memory: one carve before the branch keeps values live into the worker loop, which
+    // runs at the 128-register limit and would spill them
+    if ((int)blockIdx.x >= B) { team_worker<EMD_THREADS>(carve(smem_raw, nullptr, N, flags, pcap), W, B, N, eps, (int)blockIdx.x - B, 0); return; }
     const EmdSmem S = carve(smem_raw, nullptr, N, flags, pcap);
-    if ((int)blockIdx.x >= B) { team_worker<EMD_THREADS>(S, W, B, N, eps, (int)blockIdx.x - B, 0, prof ? prof + (size_t)blockIdx.x * 16 : nullptr); return; }
-    // development aid (PCL_EMD_PROFILE): clock totals of thread 0 per phase -> prof[blockIdx.x * 16 + phase]
-    long long pt[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0}, pc = prof ? clock64() : 0;
-#define PCL_TICK(i) if (prof) { const long long now_ = clock64(); pt[i] += now_ - pc; pc = now_; }
 
     const int cloud = blockIdx.x;
     int *const work_ctr = S.wsum + 48;
@@ -53,7 +51,6 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
     copy16_out(g_tgt, S.tgt, n32);
     copy16_out(g_pf, S.pf, n8 / 4);
     if (S.tperm) copy16_out(cl + W.o_tperm, S.tperm, n8 / 8);
-    PCL_TICK(0)
 
     auto pred_xyz = [&](int jp) -> float3 {
         if (S.x1) { const float4 q = S.x1[jp]; return make_float3(q.x, q.y, q.z); }
@@ -141,7 +138,6 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
         __syncthreads();
         sum_u += U;
         iters_run = t + 1;
-        PCL_TICK(1)
 
         // ---- 2. Bid (emd_cuda.cu:95-179) ------------------------------------------------------------------------
         const bool team = U > local_max;
@@ -178,7 +174,6 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
                 b = __shfl_sync(0xffffffffu, b, 0);
             }
             __syncthreads();
-            PCL_TICK(7)
         } else {
             // bidder records {x, y, z, seed threshold} by list position + the internal index (scan start hint) ...
             for (int b = tid; b < U; b += T) {
@@ -202,7 +197,6 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
             }
             const unsigned base = limit;
             limit += (unsigned)ntasks;
-            PCL_TICK(2)
             // serve own tickets while any is left, then wait for the tasks the workers took
             for (;;) {
                 if (tid == 0) {
@@ -221,10 +215,7 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
                 __threadfence();
                 __syncthreads();
                 if (tid == 0) { __threadfence(); atomicAdd(&ctl->done, 1u); }
-                pt[9]++;
             }
-            pt[10] += ntasks;
-            PCL_TICK(3)
             if (tid == 0) {
                 for (unsigned spin = 0; ld_acquire_u32(&ctl->done) < limit; spin++) {
                     if (spin > PCL_SPIN_LIMIT) __trap();
@@ -232,7 +223,6 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
                 }
             }
             __syncthreads();
-            PCL_TICK(4)
             // all bids of the iteration are in the mirror: bring them home, indexed by bidder as GetMax / Assign expect them
             for (int q = tid; q < U; q += T) {
                 const uint4 rec = __ldcg(&g_pub[q]);
@@ -241,7 +231,6 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
                 S.last34[jp] = rec.z;
             }
             __syncthreads();
-            PCL_TICK(5)
         }
 
         // ---- 3. GetMax + Assign (emd_cuda.cu:181-215) -------------------------------------------------------------
@@ -297,7 +286,6 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
             if (lane == 0) S.wsum[40] = __popc(lose) + __popc(evic);
         }
         __syncthreads();
-        PCL_TICK(6)
     }
 
     // ---- CalcDist (emd_cuda.cu:217-226) + outputs in ORIGINAL index order + fused loss epilogue (see pcl_emd.cu) ----
@@ -371,24 +359,20 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
         }
     }
     __syncthreads();
-    PCL_TICK(8)
-    if (prof && tid == 0) for (int i = 0; i < 12; i++) prof[(size_t)blockIdx.x * 16 + i] = pt[i];
-#undef PCL_TICK
     if (tid == 0) { __threadfence(); atomicAdd(W.finished, 1u); }  // the workers leave when every owner is here
 }
 
 // Worker CTAs for the cluster kernel's exported iterations (pcl_emd.cu, EXPORT): launched next to it on a second stream.
 __global__ void __launch_bounds__(EMD_THREADS, 1)
-emd_worker_kernel(TeamWs W, int B, int N, float eps, int flags, int pcap, long long idle_limit, long long *__restrict__ prof) {
+emd_worker_kernel(TeamWs W, int B, int N, float eps, int flags, int pcap, long long idle_limit) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const EmdSmem S = carve(smem_raw, nullptr, N, flags, pcap);
-    team_worker<EMD_THREADS>(S, W, B, N, eps, (int)blockIdx.x, idle_limit, prof ? prof + (size_t)blockIdx.x * 16 : nullptr);
+    team_worker<EMD_THREADS>(S, W, B, N, eps, (int)blockIdx.x, idle_limit);
 }
 
 }  // namespace
 
-int emd_worker_launch(void *team_ws, int B, int N, float eps, int flags, int pcap, int nworkers, size_t smem, long long idle_limit,
-                      long long *prof, cudaStream_t st) {
+int emd_worker_launch(void *team_ws, int B, int N, float eps, int flags, int pcap, int nworkers, size_t smem, cudaStream_t st) {
     static thread_local int attr_dev = -1;
     int dev = 0;
     PCL_CUDA(cudaGetDevice(&dev));
@@ -399,7 +383,8 @@ int emd_worker_launch(void *team_ws, int B, int N, float eps, int flags, int pca
         PCL_CUDA(cudaFuncSetAttribute(emd_worker_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, di.max_smem_optin));
         attr_dev = dev;
     }
-    emd_worker_kernel<<<nworkers, EMD_THREADS, smem, st>>>(team_ws_make(team_ws, B, N, nworkers), B, N, eps, flags, pcap, idle_limit, prof);
+    emd_worker_kernel<<<nworkers, EMD_THREADS, smem, st>>>(team_ws_make(team_ws, B, N, nworkers), B, N, eps, flags, pcap,
+                                                           200000LL);  // a worker leaves after ~100 us without a ticket
     PCL_CUDA(cudaGetLastError());
     return PCL_OK;
 }
@@ -412,7 +397,7 @@ size_t emd_team_workspace_bytes(int B, int N) {
 // Launches the team kernel on `st`.  team_ws: emd_team_workspace_bytes(B, N) bytes.  Everything else as emd_auction_kernel.
 int emd_team_launch(const Pts &p1, const Pts &p2, int B, int N, float eps, int iters, int flags, int pcap, int wpb_max, int tasks_target,
                     int local_max, int grid, size_t smem, float *dist, int *assignment, int *stats, void *team_ws, float grad_scale,
-                    float *grad_xyz1, double *part, unsigned *ticket, float *sums, long long *prof, cudaStream_t st) {
+                    float *grad_xyz1, double *part, unsigned *ticket, float *sums, cudaStream_t st) {
     const TeamWs W = team_ws_make(team_ws, B, N, grid - B);
     const size_t ctl_bytes = team_ctl_bytes(B);
     PCL_CUDA(cudaMemsetAsync(team_ws, 0, ctl_bytes, st));
@@ -427,7 +412,7 @@ int emd_team_launch(const Pts &p1, const Pts &p2, int B, int N, float eps, int i
         attr_dev = dev;
     }
     emd_team_kernel<<<grid, EMD_THREADS, smem, st>>>(p1, p2, B, N, eps, iters, flags, pcap, wpb_max, tasks_target, local_max, dist, assignment,
-                                                      stats, W, grad_scale, grad_xyz1, part, ticket, sums, prof);
+                                                      stats, W, grad_scale, grad_xyz1, part, ticket, sums);
     PCL_CUDA(cudaGetLastError());
     return PCL_OK;
 }

@@ -1,10 +1,16 @@
-"""Development aid: Chamfer forward time over N for the current PCL_CHAMFER_PRUNE_MIN (B from argv, default 32 and 64)."""
+"""Development aid: Chamfer forward time over N (B = 32 and 64) with the pruned path taken from MIN_POINTS points per cloud on
+(pcl_chamfer_set_prune_min: 1 = always, 0 = never, -1 = the library's default of 6144).  Running it with 1 and with 0 shows where
+the pruned scan overtakes the brute-force kernel, which is how the default was chosen.
+
+  python tools/chamfer_prune_time.py MIN_POINTS"""
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import pointcloud_b200 as pcl
 from pointcloud_b200 import _lib, synth
 L = _lib.lib()
-tag = sys.argv[1] if len(sys.argv) > 1 else ""
+prune_min = int(sys.argv[1])
+L.pcl_chamfer_set_prune_min(prune_min)
+tag = f"prune_min={prune_min}"
 for b in (32, 64):
     row = []
     for n in (1024, 2048, 4096, 8192, 16384):

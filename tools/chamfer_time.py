@@ -23,4 +23,4 @@ def timeit(fn, iters=200):
     a.record()
     for _ in range(iters): fn()
     c.record(); torch.cuda.synchronize(); return a.elapsed_time(c) / iters * 1e3
-print(f"N={n} QPT={os.environ.get('PCL_CHAMFER_QPT')}: fwd unfused {timeit(lambda: fwd(0)):.1f} us, fwd fma {timeit(lambda: fwd(1)):.1f} us, bwd {timeit(bwd):.1f} us")
+print(f"N={n}: fwd unfused {timeit(lambda: fwd(0)):.1f} us, fwd fma {timeit(lambda: fwd(1)):.1f} us, bwd {timeit(bwd):.1f} us")

@@ -1,5 +1,5 @@
 """Development aid: time the auction kernel on the bench regimes (B=32, N=2048) and print output checksums, so
-that A/B variants (PCL_LIB_OVERRIDE, PCL_EMD_WPB, PCL_EMD_ITEMS) can be compared in one GPU call."""
+that A/B builds (tools/build_variant.py, selected with PCL_LIB_OVERRIDE) can be compared in one GPU call."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch

@@ -1,4 +1,6 @@
-"""Development aid: time the auction (current path selection / env knobs) on the bench regimes; prints checksums."""
+"""Development aid: time the auction on the bench regimes through one path (pcl_emd_set_path; default 2 = team); prints checksums.
+
+  python tools/team_time.py [TAG] [B] [PATH]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
