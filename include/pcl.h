@@ -248,6 +248,36 @@ PCL_API int pcl_ball_query(const void *xyz, int dtype, int64_t bs, int64_t rs,
                    const void *new_xyz, int ndtype, int64_t nbs, int64_t nrs,
                    int B, int N, int S, float radius2, int nsample, int32_t *group_idx, void *stream);
 
+/* ------------------------------------------------------------------ k nearest neighbours ------------------ */
+/*
+ * Replaces pytorch3d.ops.knn_points(p1, p2, lengths1, lengths2, norm=2, K) forward and knn_points_backward (third-party
+ * code, restated from memory: parity with pytorch3d itself is unpinned).  p1 (B,P1,D) queries, p2 (B,P2,D) targets,
+ * 1 <= D <= 8, len1 / len2 nullable int64[B] (entries clamped to [0,P]); 1 <= K <= pcl_knn_max_k() (64); K > P2 is allowed.
+ *   dists (B,P1,K) fp32: squared L2 distances, rounded as `mode` says (PCL_CHAMFER_UNFUSED or PCL_CHAMFER_FMA);
+ *   idx (B,P1,K) int32.
+ * For a query i < len1[n] the result is the K smallest targets j < len2[n] under the key (distance, index), sorted
+ * ascending by that key: exact ties go to the lower index, and a NaN distance ranks after +inf (its dists entry is the
+ * NaN 0x7fffffff).  Slots k >= min(K, len2[n]) and rows i >= len1[n] are dist 0, idx 0.  The result does not depend on
+ * the order in which the kernel visits the targets; for finite inputs K = 1 is bit-identical to dist_x / idx_x of
+ * pcl_chamfer_fwd.
+ * No workspace.
+ */
+PCL_API int pcl_knn_max_k(void);
+PCL_API int pcl_knn_fwd(const void *p1, int dtype1, int64_t bs1, int64_t rs1, const int64_t *len1,
+                const void *p2, int dtype2, int64_t bs2, int64_t rs2, const int64_t *len2,
+                int B, int P1, int P2, int D, int K, int mode,
+                float *dists, int32_t *idx, void *stream);
+/*
+ * Backward through dists (idx is not differentiable): for every i < len1[n] and k < min(K, len2[n]), with j = idx[n,i,k],
+ *   diff = 2*grad_dists[n,i,k] * (p1[n,i] - p2[n,j]);  grad_p1[n,i] += diff;  grad_p2[n,j] -= diff.
+ * grad_dists is a DEVICE (B,P1,K) fp32 array (no host sync).  grad_p1 (B,P1,D) and grad_p2 (B,P2,D) are dense fp32 and are
+ * overwritten: grad_p1 is summed over k in ascending order by one thread, grad_p2 is accumulated with fp32 atomics.
+ */
+PCL_API int pcl_knn_bwd(const void *p1, int dtype1, int64_t bs1, int64_t rs1, const int64_t *len1,
+                const void *p2, int dtype2, int64_t bs2, int64_t rs2, const int64_t *len2,
+                int B, int P1, int P2, int D, int K, const int32_t *idx,
+                const float *grad_dists, float *grad_p1, float *grad_p2, void *stream);
+
 /* ------------------------------------------------------------------ composite step ------------------------ */
 /*
  * One pass of the whole hot path over a batch that is already on the device: Chamfer fwd+bwd (upstream gradient 1)

@@ -8,6 +8,7 @@ hand-written CUDA kernels behind the C ABI of include/pcl.h (libpcl_b200.so).  N
 from . import cfg
 from .chamfer import chamfer_distance, chamfer_forward_raw
 from .emd_module import emdFunction, emdModule, emd_forward_raw, set_emd_path
+from .knn import knn_forward_raw, knn_gather, knn_points
 from .losses import (ChamferDistance, EarthMoverDistance, FilterClasses, FilteringChamferDistance,
                      SegmentingChamferDistance, chamfer_emd_loss)
 from .sampling import farthest_point_sample, query_ball_point, sample_farthest_points
@@ -17,5 +18,5 @@ __all__ = [
     "cfg", "chamfer_distance", "chamfer_forward_raw", "emdFunction", "emdModule", "emd_forward_raw", "set_emd_path",
     "ChamferDistance", "FilteringChamferDistance", "SegmentingChamferDistance", "EarthMoverDistance",
     "FilterClasses", "chamfer_emd_loss", "ShardedLoss", "ShardedChamferEmdStep", "shard_bounds",
-    "farthest_point_sample", "sample_farthest_points", "query_ball_point",
+    "farthest_point_sample", "sample_farthest_points", "query_ball_point", "knn_points", "knn_gather", "knn_forward_raw",
 ]

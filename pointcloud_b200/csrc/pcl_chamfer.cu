@@ -60,13 +60,6 @@ __device__ __forceinline__ float sqdist3(float qx, float qy, float qz, const flo
     else return __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz));
 }
 
-// length of cloud n, clamped to [0, P]: pytorch3d raises on lengths > P; a kernel cannot, but it must not read past the cloud
-__device__ __forceinline__ int len_of(const int64_t *len, int n, int P) {
-    if (!len) return P;
-    const int64_t v = len[n];
-    return (int)(v < 0 ? 0 : (v > P ? P : v));
-}
-
 // Tail of both forward kernels: the CTA's partial sum goes to the workspace; the CTA that takes the LAST ticket of the grid
 // (zeroed by the host call) then forms  loss_xy[dir] = sum_n (sum_i dist / clamp(len,1)) / max(B,1)  from all partials in a
 // fixed order (deterministic scalar, fp64) -- no memset of the partials and no second launch.  Needs >= 64 threads per CTA.

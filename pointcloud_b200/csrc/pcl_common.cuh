@@ -55,6 +55,14 @@ __device__ __forceinline__ float3 ld_xyz(const Pts &a, int64_t b, int64_t row) {
     return make_float3(ld_any(a, o), ld_any(a, o + 1), ld_any(a, o + 2));
 }
 
+// length of cloud n (len nullable: P), clamped to [0, P]: pytorch3d raises on lengths > P; a kernel cannot, but it must not
+// read past the cloud
+__device__ __forceinline__ int len_of(const int64_t *len, int n, int P) {
+    if (!len) return P;
+    const int64_t v = len[n];
+    return (int)(v < 0 ? 0 : (v > P ? P : v));
+}
+
 // Chamfer backward with the upstream gradients either on the device (grad_out != nullptr) or as immediates (pcl_chamfer.cu)
 int chamfer_bwd_impl(const void *x, int x_dtype, int64_t x_bs, int64_t x_rs, const int64_t *x_len, const void *y, int y_dtype,
                      int64_t y_bs, int64_t y_rs, const int64_t *y_len, int B, int P1, int P2, int D, const int32_t *idx_x,
