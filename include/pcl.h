@@ -235,10 +235,27 @@ PCL_API int pcl_class_filter(const void *target, int dtype, int64_t bs, int64_t 
  * part of the reference tree; semantics = the torch algorithm kept as a comment in pointnet2_utils.py:64-86 with
  * start index 0 (or start_idx[b]) and the lowest index on ties.  idx_out: int32 (B, npoint).
  * skip_origin != 0: points with x*x+y*y+z*z <= 1e-3 are never selected (pointnet2_ops' padding convention).
+ * start_idx[b] is clamped to [0, N-1].  npoint > N is allowed: once every running minimum is 0, index 0 repeats.
+ * N may be up to pcl_fps_max_points() = 262144: one thread-block cluster of 1..16 CTAs per cloud keeps the cloud
+ * and its running minima on chip (16384 points per CTA); the cluster size is chosen per launch (pcl_sampling.cu).
+ * N above the bound gives PCL_E_UNSUPPORTED.
  */
 PCL_API int pcl_fps_max_points(void);
 PCL_API int pcl_fps(const void *xyz, int dtype, int64_t bs, int64_t rs, int B, int N, int npoint,
             const int32_t *start_idx /* nullable */, int skip_origin, int32_t *idx_out, void *stream);
+/*
+ * Farthest point sampling of a ragged batch (pytorch3d's sample_farthest_points(points, lengths, K)).  For cloud b:
+ * n_b = lengths[b] clamped to [0, N] (N without lengths), k_b = K[b] clamped to [0, npoint] (npoint without K),
+ * s_b = min(n_b, k_b).  idx_out[b, j < s_b] is the FPS sequence over the first n_b points only (the arithmetic, start
+ * (start_idx[b] clamped to [0, n_b-1]), skip_origin and tie rule of pcl_fps; points at index >= n_b never influence
+ * it); idx_out[b, s_b <= j < npoint] = -1.  Without lengths and K the result equals pcl_fps whenever npoint <= N.
+ * lengths and K are int64 DEVICE arrays of B entries, read on the device (no host synchronisation).
+ * cluster: 0 = the automatic cluster size; 1, 2, 4, 8 or 16 force one (tests and timing only; a cluster of c CTAs
+ * holds at most 16384 * c points, larger N gives PCL_E_UNSUPPORTED).  Other values give PCL_E_ARG.
+ */
+PCL_API int pcl_fps_ragged(const void *xyz, int dtype, int64_t bs, int64_t rs, const int64_t *lengths /* nullable */,
+            int B, int N, const int64_t *K /* nullable */, int npoint, const int32_t *start_idx /* nullable */,
+            int skip_origin, int cluster, int32_t *idx_out /* (B, npoint) */, void *stream);
 /*
  * Ball query: replaces query_ball_point(radius, nsample, xyz, new_xyz) (models/pointnet2_utils.py:93-113): for every
  * centroid the first `nsample` point indices (ascending) with squared distance <= radius2, padded with the first

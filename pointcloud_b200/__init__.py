@@ -11,12 +11,12 @@ from .emd_module import emdFunction, emdModule, emd_forward_raw, set_emd_path
 from .knn import knn_forward_raw, knn_gather, knn_points
 from .losses import (ChamferDistance, EarthMoverDistance, FilterClasses, FilteringChamferDistance,
                      SegmentingChamferDistance, chamfer_emd_loss)
-from .sampling import farthest_point_sample, query_ball_point, sample_farthest_points
+from .sampling import farthest_point_sample, fps_forward_raw, query_ball_point, sample_farthest_points
 from .sharded import ShardedChamferEmdStep, ShardedLoss, shard_bounds
 
 __all__ = [
     "cfg", "chamfer_distance", "chamfer_forward_raw", "emdFunction", "emdModule", "emd_forward_raw", "set_emd_path",
     "ChamferDistance", "FilteringChamferDistance", "SegmentingChamferDistance", "EarthMoverDistance",
     "FilterClasses", "chamfer_emd_loss", "ShardedLoss", "ShardedChamferEmdStep", "shard_bounds",
-    "farthest_point_sample", "sample_farthest_points", "query_ball_point", "knn_points", "knn_gather", "knn_forward_raw",
+    "farthest_point_sample", "sample_farthest_points", "fps_forward_raw", "query_ball_point", "knn_points", "knn_gather", "knn_forward_raw",
 ]

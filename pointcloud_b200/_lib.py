@@ -45,6 +45,7 @@ _SIGNATURES = {
     "pcl_class_filter": (c_int, _PTS + [c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "pcl_fps_max_points": (c_int, []),
     "pcl_fps": (c_int, _PTS + [c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p]),
+    "pcl_fps_ragged": (c_int, _PTS + [c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "pcl_ball_query": (c_int, _PTS + _PTS + [c_int, c_int, c_int, c_float, c_int, c_void_p, c_void_p]),
     "pcl_knn_max_k": (c_int, []),
     "pcl_knn_fwd": (c_int, _PTS + [c_void_p] + _PTS + [c_void_p] + [c_int] * 6 + [c_void_p] * 2 + [c_void_p]),
