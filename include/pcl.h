@@ -289,8 +289,36 @@ PCL_API int pcl_knn_fwd(const void *p1, int dtype1, int64_t bs1, int64_t rs1, co
  *   diff = 2*grad_dists[n,i,k] * (p1[n,i] - p2[n,j]);  grad_p1[n,i] += diff;  grad_p2[n,j] -= diff.
  * grad_dists is a DEVICE (B,P1,K) fp32 array (no host sync).  grad_p1 (B,P1,D) and grad_p2 (B,P2,D) are dense fp32 and are
  * overwritten: grad_p1 is summed over k in ascending order by one thread, grad_p2 is accumulated with fp32 atomics.
+ * A slot whose idx is -1 contributes nothing (pcl_knn_fwd never writes -1; pcl_ball_query_fwd pads with it).
  */
 PCL_API int pcl_knn_bwd(const void *p1, int dtype1, int64_t bs1, int64_t rs1, const int64_t *len1,
+                const void *p2, int dtype2, int64_t bs2, int64_t rs2, const int64_t *len2,
+                int B, int P1, int P2, int D, int K, const int32_t *idx,
+                const float *grad_dists, float *grad_p1, float *grad_p2, void *stream);
+
+/* ------------------------------------------------------------------ ball query ---------------------------- */
+/*
+ * Replaces pytorch3d.ops.ball_query(p1, p2, lengths1, lengths2, K, radius) forward and its backward (third-party code,
+ * restated from memory [3P-memory]: parity with pytorch3d itself is unpinned).  Inputs as for pcl_knn_fwd: p1 (B,P1,D)
+ * queries, p2 (B,P2,D) targets, 1 <= D <= 8, len1 / len2 nullable int64[B] (entries clamped to [0,P]); K >= 1 with no
+ * upper bound (K > P2 is allowed); radius2 is the fp32 comparison value.
+ *   dists (B,P1,K) fp32, idx (B,P1,K) int32.
+ * For a query i < len1[n], the targets j = 0, 1, ..., len2[n]-1 are visited in ascending order and j is kept when
+ * d(i,j) < radius2 (strict; a NaN or infinite d is never kept).  The first c <= K kept targets fill slots 0..c-1 with
+ * (d, j); slots c..K-1 are dist 0, idx -1.  Rows i >= len1[n] are dist 0, idx -1 (pcl_knn_fwd writes 0 / 0 there).
+ * d is the arithmetic of `mode` (PCL_CHAMFER_UNFUSED or PCL_CHAMFER_FMA), so a kept distance is bit-identical to the one
+ * pcl_knn_fwd reports for the same pair.  The result does not depend on how the kernel splits the scan.
+ * Unlike pcl_ball_query (pointnet2's query_ball_point: xyz only, <=, padding with the first hit) this takes lengths,
+ * D <= 8, returns distances and has a backward.  No workspace.
+ */
+PCL_API int pcl_ball_query_fwd(const void *p1, int dtype1, int64_t bs1, int64_t rs1, const int64_t *len1,
+                const void *p2, int dtype2, int64_t bs2, int64_t rs2, const int64_t *len2,
+                int B, int P1, int P2, int D, int K, float radius2, int mode,
+                float *dists, int32_t *idx, void *stream);
+/*
+ * Backward through dists: pcl_knn_bwd's formula and kernel (the -1 pads contribute nothing) without its bound on K.
+ */
+PCL_API int pcl_ball_query_bwd(const void *p1, int dtype1, int64_t bs1, int64_t rs1, const int64_t *len1,
                 const void *p2, int dtype2, int64_t bs2, int64_t rs2, const int64_t *len2,
                 int B, int P1, int P2, int D, int K, const int32_t *idx,
                 const float *grad_dists, float *grad_p1, float *grad_p2, void *stream);

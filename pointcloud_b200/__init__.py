@@ -6,6 +6,7 @@ Python host layer (this package) mirrors the reference's loss interface
 hand-written CUDA kernels behind the C ABI of include/pcl.h (libpcl_b200.so).  No CPU fallback.
 """
 from . import cfg
+from .ball_query import ball_query, ball_query_forward_raw
 from .chamfer import chamfer_distance, chamfer_forward_raw
 from .emd_module import emdFunction, emdModule, emd_forward_raw, set_emd_path
 from .knn import knn_forward_raw, knn_gather, knn_points
@@ -19,4 +20,5 @@ __all__ = [
     "ChamferDistance", "FilteringChamferDistance", "SegmentingChamferDistance", "EarthMoverDistance",
     "FilterClasses", "chamfer_emd_loss", "ShardedLoss", "ShardedChamferEmdStep", "shard_bounds",
     "farthest_point_sample", "sample_farthest_points", "fps_forward_raw", "query_ball_point", "knn_points", "knn_gather", "knn_forward_raw",
+    "ball_query", "ball_query_forward_raw",
 ]

@@ -18,6 +18,8 @@
 // sorted lists (insertion, threshold refreshed after each key).  Draining together bounds the time a warp spends in the
 // divergent insertion code by the busiest lane's admissions -- about K (1 + ln(P2/K)) for random order -- instead of one
 // insertion for every target that ANY of the 32 queries admits, which early in the scan is nearly every target.
+#include <climits>
+
 #include "pcl_common.cuh"
 
 namespace pcl {
@@ -161,7 +163,8 @@ knn_fwd_kernel(Pts p1, const int64_t *__restrict__ len1, Pts p2, const int64_t *
 }
 
 // Backward: one thread per (n, i).  grad_p1[n, i] = sum_k diff_k in ascending k (fp32, in registers, then one store;
-// padded rows get 0); grad_p2[n, idx] -= diff_k with red.global.add onto the zero-filled grad_p2.
+// padded rows get 0); grad_p2[n, idx] -= diff_k with red.global.add onto the zero-filled grad_p2.  Slots whose idx is -1
+// contribute nothing.
 template <int D>
 __global__ void __launch_bounds__(KNN_BWD_THREADS, 4)
 knn_bwd_kernel(Pts p1, const int64_t *__restrict__ len1, Pts p2, const int64_t *__restrict__ len2, int P1, int P2, int K,
@@ -180,6 +183,7 @@ knn_bwd_kernel(Pts p1, const int64_t *__restrict__ len1, Pts p2, const int64_t *
     const size_t r0 = ((size_t)n * P1 + i) * K;
     for (int k = 0; k < kv; k++) {
         const int j = __ldg(idx + r0 + k);
+        if (j < 0) continue;  // a ball-query pad (pcl_knn_fwd never writes -1)
         const float g2 = __fmul_rn(2.0f, __ldg(grad_dists + r0 + k));
         const int64_t to = (int64_t)n * p2.bs + (int64_t)j * p2.rs;
         float *gt = grad_p2 + ((size_t)n * P2 + j) * D;
@@ -193,6 +197,107 @@ knn_bwd_kernel(Pts p1, const int64_t *__restrict__ len1, Pts p2, const int64_t *
     float *gq = grad_p1 + ((size_t)n * P1 + i) * D;
 #pragma unroll
     for (int c = 0; c < D; c++) gq[c] = acc[c];
+}
+
+// ------------------------------------------------------------------ ball query
+// pytorch3d.ops.ball_query (include/pcl.h, "ball query"): for a query i < len1[n], the first K targets j < len2[n] in
+// ascending index order with sqdist<FMA, D> < radius2, then (0, -1) pads.
+//
+// One lane per query, 32 queries per CTA.  When B * ceil(P1 / 32) warps cannot fill the GPU, `parts` warps of the CTA
+// scan `parts` contiguous, ascending ranges of the targets [0, len2) (range p = [p c, (p+1) c), c = ceil(len2 / parts)),
+// each collecting the first K hits of its own range.  Part 0 appends its hits straight to the output row; part p >= 1
+// keeps the indices of its hits in shared memory (distances are recomputed by the same sqdist when merged, so they are
+// bit-identical).  Warp 0 then appends parts 1, 2, ... in order until the row holds K hits.  Because the ranges are
+// contiguous and ordered, the first K hits of the concatenation are the first K hits of the whole scan: the result does
+// not depend on `parts`.  Split rule (bq_parts_for): double `parts` while the GPU has fewer than 8 query warps per SM,
+// parts <= BQ_MAX_PARTS, every part keeps at least BQ_MIN_RANGE of the P2 targets, and the buffered indices
+// (parts - 1) * 32 * K * 4 bytes fit BQ_BUF_BYTES -- so K <= 960 may split in two and K <= 64 in sixteen.  The unsplit
+// path has no bound on K.
+//
+// Each warp streams its range through its own shared-memory tile (no CTA barrier in the scan) and stops once all its
+// lanes have K hits, or once the lower parts already hold K hits for every lane: per-lane hit counts are published in
+// shared memory after every tile, and since they only grow, a stale read only delays the exit.
+constexpr int BQ_MAX_PARTS = 16;
+constexpr int BQ_TILE = 128;                // targets per warp tile
+constexpr int BQ_MIN_RANGE = 256;           // targets per part at least
+constexpr int BQ_BUF_BYTES = 120 * 1024;    // buffered hit indices of parts 1.. (15 parts x 32 lanes x K = 64 x 4 bytes)
+
+// grid (ceil(P1 / 32), B); block 32 * parts; dynamic shared memory: parts tiles of BQ_TILE x DS floats, hit counts
+// [part][lane], then buffered indices [part - 1][k][lane].
+template <bool FMA, int D>
+__global__ void __launch_bounds__(32 * BQ_MAX_PARTS, 1)
+ball_query_fwd_kernel(Pts p1, const int64_t *__restrict__ len1, Pts p2, const int64_t *__restrict__ len2, int P1, int P2,
+                      int K, float r2, float *__restrict__ dists, int *__restrict__ idx) {
+    constexpr int DS = (D == 3) ? 4 : D;
+    extern __shared__ __align__(16) unsigned char bq_sm[];
+    const int parts = blockDim.x >> 5, part = threadIdx.x >> 5, lane = threadIdx.x & 31, n = blockIdx.y;
+    float *tile = reinterpret_cast<float *>(bq_sm) + part * BQ_TILE * DS;
+    volatile int *counts = reinterpret_cast<volatile int *>(bq_sm + (size_t)parts * BQ_TILE * DS * sizeof(float));
+    int *bufs = const_cast<int *>(counts) + parts * 32;
+    const int i0 = blockIdx.x * 32, i = i0 + lane;
+    const int lq = len_of(len1, n, P1), lt = len_of(len2, n, P2);
+    const size_t out0 = ((size_t)n * P1 + i0) * K;
+    const int nout = min(32, P1 - i0) * K;  // this CTA's rows are one contiguous block of the outputs
+    if (i0 >= lq) {  // CTA-uniform: padded rows only
+        for (int e = threadIdx.x; e < nout; e += blockDim.x) { dists[out0 + e] = 0.f; idx[out0 + e] = -1; }
+        return;
+    }
+    const bool active = i < lq;
+    float q[D];
+#pragma unroll
+    for (int c = 0; c < D; c++) q[c] = active ? ld_pt(p1, (int64_t)n * p1.bs + (int64_t)i * p1.rs + c) : 0.f;
+    float *drow = dists + out0 + (size_t)lane * K;
+    int *irow = idx + out0 + (size_t)lane * K;
+    int *buf = bufs + (size_t)(part - 1) * K * 32 + lane;  // part >= 1: hit k at buf[32 k]
+    const int chunk = (lt + parts - 1) / parts;
+    const int lo = min(lt, part * chunk), hi = min(lt, lo + chunk);
+    int cnt = active ? 0 : K;  // surplus lanes count as done
+    counts[part * 32 + lane] = cnt;
+    __syncthreads();
+    for (int t0 = lo; t0 < hi; t0 += BQ_TILE) {
+        int below = 0;
+        for (int s = 0; s < part; s++) below += counts[s * 32 + lane];
+        if (__all_sync(0xffffffffu, cnt >= K || below >= K)) break;  // warp-uniform
+        const int m = min(BQ_TILE, hi - t0);
+        __syncwarp();  // the previous tile is consumed
+        for (int e = lane; e < m * D; e += 32) {
+            const int j = e / D, c = e - j * D;
+            tile[j * DS + c] = ld_pt(p2, (int64_t)n * p2.bs + (int64_t)(t0 + j) * p2.rs + c);
+        }
+        __syncwarp();
+#pragma unroll 4
+        for (int e = 0; e < m; e++) {
+            const float d = sqdist<FMA, D>(q, tile + e * DS);
+            if (d < r2 && cnt < K) {  // NaN is never < r2
+                if (part == 0) { drow[cnt] = d; irow[cnt] = t0 + e; }
+                else buf[32 * cnt] = t0 + e;
+                cnt++;
+            }
+        }
+        counts[part * 32 + lane] = cnt;
+    }
+    __syncthreads();
+    if (part == 0) {
+        for (int s = 1; s < parts && cnt < K; s++) {
+            const int ns = counts[s * 32 + lane];
+            const int *ob = bufs + (size_t)(s - 1) * K * 32 + lane;
+            for (int k = 0; k < ns && cnt < K; k++) {
+                const int j = ob[32 * k];
+                float t[D];
+#pragma unroll
+                for (int c = 0; c < D; c++) t[c] = ld_pt(p2, (int64_t)n * p2.bs + (int64_t)j * p2.rs + c);
+                drow[cnt] = sqdist<FMA, D>(q, t);
+                irow[cnt] = j;
+                cnt++;
+            }
+        }
+        counts[lane] = cnt;
+    }
+    __syncthreads();
+    for (int e = threadIdx.x; e < nout; e += blockDim.x) {  // pads, coalesced over the CTA's block of rows
+        const int r = e / K, k = e - r * K;
+        if (i0 + r >= lq || k >= counts[r]) { dists[out0 + e] = 0.f; idx[out0 + e] = -1; }
+    }
 }
 
 inline int parts_for(int B, int P1, int P2, int K, int sm_count) {
@@ -238,11 +343,56 @@ int launch_fwd(const Pts &a, const int64_t *len1, const Pts &b, const int64_t *l
     return PCL_E_UNSUPPORTED;
 }
 
-int check_args(const char *who, const void *p1, int dtype1, const void *p2, int dtype2, int B, int P1, int P2, int D, int K) {
+inline int bq_parts_for(int B, int P1, int P2, int K, int sm_count) {
+    const long long qwarps = (long long)B * ((P1 + 31) / 32);
+    int parts = 1;
+    while (parts * 2 <= BQ_MAX_PARTS && qwarps * parts < 8LL * sm_count && P2 / (parts * 2) >= BQ_MIN_RANGE &&
+           (long long)(parts * 2 - 1) * 32 * K * sizeof(int) <= BQ_BUF_BYTES)
+        parts *= 2;
+    return parts;
+}
+
+inline size_t bq_smem(int D, int K, int parts) {
+    return (size_t)parts * BQ_TILE * (D == 3 ? 4 : D) * sizeof(float) + (size_t)parts * 32 * sizeof(int) +
+           (size_t)(parts - 1) * 32 * K * sizeof(int);
+}
+
+template <bool FMA, int D>
+int launch_bq_d(const Pts &a, const int64_t *len1, const Pts &b, const int64_t *len2, int B, int P1, int P2, int K, float r2,
+                int parts, float *dists, int *idx, cudaStream_t st) {
+    static thread_local int attr_dev = -1;  // per instantiation: the opt-in to more than 48 KB of dynamic shared memory
+    int dev = 0;
+    PCL_CUDA(cudaGetDevice(&dev));
+    if (attr_dev != dev) {  // bq_parts_for keeps the buffers within BQ_BUF_BYTES
+        PCL_CUDA(cudaFuncSetAttribute(ball_query_fwd_kernel<FMA, D>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)(bq_smem(D, 0, BQ_MAX_PARTS) + BQ_BUF_BYTES)));
+        attr_dev = dev;
+    }
+    ball_query_fwd_kernel<FMA, D><<<dim3((P1 + 31) / 32, B), 32 * parts, bq_smem(D, K, parts), st>>>(a, len1, b, len2, P1, P2, K,
+                                                                                                    r2, dists, idx);
+    return PCL_OK;
+}
+
+template <bool FMA>
+int launch_bq(const Pts &a, const int64_t *len1, const Pts &b, const int64_t *len2, int B, int P1, int P2, int D, int K, float r2,
+              int parts, float *dists, int *idx, cudaStream_t st) {
+    switch (D) {
+#define PCL_BQ_FWD(DD) case DD: return launch_bq_d<FMA, DD>(a, len1, b, len2, B, P1, P2, K, r2, parts, dists, idx, st)
+        PCL_BQ_FWD(1); PCL_BQ_FWD(2); PCL_BQ_FWD(3); PCL_BQ_FWD(4);
+        PCL_BQ_FWD(5); PCL_BQ_FWD(6); PCL_BQ_FWD(7); PCL_BQ_FWD(8);
+#undef PCL_BQ_FWD
+    }
+    set_error("ball_query: D=%d unsupported (1..8)", D);
+    return PCL_E_UNSUPPORTED;
+}
+
+// kmax: the largest K accepted (KNN_MAX_K for kNN; ball query has no bound but sizes)
+int check_args(const char *who, const void *p1, int dtype1, const void *p2, int dtype2, int B, int P1, int P2, int D, int K,
+               int kmax) {
     if (B < 0 || P1 < 0 || P2 < 0) { set_error("%s: negative size B=%d P1=%d P2=%d", who, B, P1, P2); return PCL_E_SHAPE; }
     if (D < 1 || D > 8) { set_error("%s: D=%d unsupported (1..8)", who, D); return PCL_E_UNSUPPORTED; }
     if (K < 1) { set_error("%s: K=%d must be at least 1", who, K); return PCL_E_SHAPE; }
-    if (K > KNN_MAX_K) { set_error("%s: K=%d > pcl_knn_max_k() = %d", who, K, KNN_MAX_K); return PCL_E_UNSUPPORTED; }
+    if (K > kmax) { set_error("%s: K=%d > pcl_knn_max_k() = %d", who, K, kmax); return PCL_E_UNSUPPORTED; }
     if (B > 65535) { set_error("%s: B=%d > 65535", who, B); return PCL_E_SHAPE; }
     if (!dtype_ok(dtype1) || !dtype_ok(dtype2)) { set_error("%s: bad dtype", who); return PCL_E_ARG; }
     if (B > 0 && ((P1 > 0 && !p1) || (P2 > 0 && !p2))) { set_error("%s: null input", who); return PCL_E_ARG; }
@@ -259,7 +409,7 @@ extern "C" int pcl_knn_max_k(void) { return KNN_MAX_K; }
 extern "C" int pcl_knn_fwd(const void *p1, int dtype1, int64_t bs1, int64_t rs1, const int64_t *len1,
                            const void *p2, int dtype2, int64_t bs2, int64_t rs2, const int64_t *len2,
                            int B, int P1, int P2, int D, int K, int mode, float *dists, int32_t *idx, void *stream) {
-    int rc = check_args("knn", p1, dtype1, p2, dtype2, B, P1, P2, D, K);
+    int rc = check_args("knn", p1, dtype1, p2, dtype2, B, P1, P2, D, K, KNN_MAX_K);
     if (rc) return rc;
     if (mode != PCL_CHAMFER_UNFUSED && mode != PCL_CHAMFER_FMA) { set_error("knn: bad mode %d", mode); return PCL_E_ARG; }
     if (B > 0 && P1 > 0 && (!dists || !idx)) { set_error("knn: null output"); return PCL_E_ARG; }
@@ -276,14 +426,15 @@ extern "C" int pcl_knn_fwd(const void *p1, int dtype1, int64_t bs1, int64_t rs1,
     return PCL_OK;
 }
 
-extern "C" int pcl_knn_bwd(const void *p1, int dtype1, int64_t bs1, int64_t rs1, const int64_t *len1,
-                           const void *p2, int dtype2, int64_t bs2, int64_t rs2, const int64_t *len2,
-                           int B, int P1, int P2, int D, int K, const int32_t *idx, const float *grad_dists,
-                           float *grad_p1, float *grad_p2, void *stream) {
-    int rc = check_args("knn_bwd", p1, dtype1, p2, dtype2, B, P1, P2, D, K);
+namespace {
+// pcl_knn_bwd and pcl_ball_query_bwd: the same kernel, with kNN's or ball query's bound on K
+int bwd_impl(const char *who, int kmax, const void *p1, int dtype1, int64_t bs1, int64_t rs1, const int64_t *len1,
+             const void *p2, int dtype2, int64_t bs2, int64_t rs2, const int64_t *len2, int B, int P1, int P2, int D, int K,
+             const int32_t *idx, const float *grad_dists, float *grad_p1, float *grad_p2, void *stream) {
+    int rc = check_args(who, p1, dtype1, p2, dtype2, B, P1, P2, D, K, kmax);
     if (rc) return rc;
     if (B > 0 && ((P1 > 0 && (!idx || !grad_dists || !grad_p1)) || (P2 > 0 && !grad_p2))) {
-        set_error("knn_bwd: null argument"); return PCL_E_ARG;
+        set_error("%s: null argument", who); return PCL_E_ARG;
     }
     DeviceInfo di;
     if ((rc = device_info(&di))) return rc;
@@ -302,4 +453,42 @@ extern "C" int pcl_knn_bwd(const void *p1, int dtype1, int64_t bs1, int64_t rs1,
     }
     PCL_CUDA(cudaGetLastError());
     return PCL_OK;
+}
+}  // namespace
+
+extern "C" int pcl_knn_bwd(const void *p1, int dtype1, int64_t bs1, int64_t rs1, const int64_t *len1,
+                           const void *p2, int dtype2, int64_t bs2, int64_t rs2, const int64_t *len2,
+                           int B, int P1, int P2, int D, int K, const int32_t *idx, const float *grad_dists,
+                           float *grad_p1, float *grad_p2, void *stream) {
+    return bwd_impl("knn_bwd", KNN_MAX_K, p1, dtype1, bs1, rs1, len1, p2, dtype2, bs2, rs2, len2, B, P1, P2, D, K, idx,
+                    grad_dists, grad_p1, grad_p2, stream);
+}
+
+extern "C" int pcl_ball_query_fwd(const void *p1, int dtype1, int64_t bs1, int64_t rs1, const int64_t *len1,
+                                  const void *p2, int dtype2, int64_t bs2, int64_t rs2, const int64_t *len2,
+                                  int B, int P1, int P2, int D, int K, float radius2, int mode, float *dists, int32_t *idx,
+                                  void *stream) {
+    int rc = check_args("ball_query", p1, dtype1, p2, dtype2, B, P1, P2, D, K, INT_MAX);
+    if (rc) return rc;
+    if (mode != PCL_CHAMFER_UNFUSED && mode != PCL_CHAMFER_FMA) { set_error("ball_query: bad mode %d", mode); return PCL_E_ARG; }
+    if (B > 0 && P1 > 0 && (!dists || !idx)) { set_error("ball_query: null output"); return PCL_E_ARG; }
+    DeviceInfo di;
+    if ((rc = device_info(&di))) return rc;
+    if (B == 0 || P1 == 0) return PCL_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    const Pts a{p1, bs1, rs1, dtype1}, b{p2, bs2, rs2, dtype2};
+    const int parts = bq_parts_for(B, P1, P2, K, di.sm_count);
+    rc = (mode == PCL_CHAMFER_FMA) ? launch_bq<true>(a, len1, b, len2, B, P1, P2, D, K, radius2, parts, dists, (int *)idx, st)
+                                   : launch_bq<false>(a, len1, b, len2, B, P1, P2, D, K, radius2, parts, dists, (int *)idx, st);
+    if (rc) return rc;
+    PCL_CUDA(cudaGetLastError());
+    return PCL_OK;
+}
+
+extern "C" int pcl_ball_query_bwd(const void *p1, int dtype1, int64_t bs1, int64_t rs1, const int64_t *len1,
+                                  const void *p2, int dtype2, int64_t bs2, int64_t rs2, const int64_t *len2,
+                                  int B, int P1, int P2, int D, int K, const int32_t *idx, const float *grad_dists,
+                                  float *grad_p1, float *grad_p2, void *stream) {
+    return bwd_impl("ball_query_bwd", INT_MAX, p1, dtype1, bs1, rs1, len1, p2, dtype2, bs2, rs2, len2, B, P1, P2, D, K, idx,
+                    grad_dists, grad_p1, grad_p2, stream);
 }

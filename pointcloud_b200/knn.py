@@ -24,6 +24,14 @@ def knn_max_k() -> int:
 def _check(p1, p2, K, lengths1=None, lengths2=None, norm=2):
     if norm != 2:
         raise NotImplementedError("only norm=2 (squared L2) is supported")
+    _check_shapes(p1, p2, lengths1, lengths2)
+    kmax = knn_max_k()
+    if isinstance(K, bool) or int(K) != K or not 1 <= int(K) <= kmax:
+        raise ValueError(f"K={K} is not supported (1..{kmax})")
+
+
+def _check_shapes(p1, p2, lengths1=None, lengths2=None):
+    """The shape checks shared by knn_points and ball_query (pytorch3d's messages)."""
     if p1.dim() != 3 or p2.dim() != 3:
         raise ValueError("Expected points to be of shape (N, P, D)")
     if p1.shape[0] != p2.shape[0]:
@@ -35,9 +43,6 @@ def _check(p1, p2, K, lengths1=None, lengths2=None, norm=2):
     for name, ln in (("lengths1", lengths1), ("lengths2", lengths2)):
         if ln is not None and ln.shape != (p1.shape[0],):
             raise ValueError(f"Expected {name} to be of shape (N,).")
-    kmax = knn_max_k()
-    if isinstance(K, bool) or int(K) != K or not 1 <= int(K) <= kmax:
-        raise ValueError(f"K={K} is not supported (1..{kmax})")
 
 
 def _lengths(lengths, dev):
@@ -73,6 +78,7 @@ class _KnnFunction(Function):
     @staticmethod
     def forward(ctx, p1, p2, lengths1, lengths2, K, mode):
         ctx.in_meta = (p1.dtype, p1.device, p2.dtype, p2.device)
+        ctx.n_inputs = 6
         r = knn_forward_raw(p1, p2, lengths1, lengths2, K, mode)
         ctx.save_for_backward(r["p1"], r["p2"], r["idx"])
         ctx.lens = (r["len1"], r["len2"])
@@ -82,21 +88,27 @@ class _KnnFunction(Function):
 
     @staticmethod
     def backward(ctx, grad_dists, grad_idx):
-        p1, p2, idx = ctx.saved_tensors
-        l1, l2 = ctx.lens
-        L = _lib.lib()
-        b, n1, d = p1.shape
-        n2, K = p2.shape[1], idx.shape[2]
-        dev = p1.device
-        g = grad_dists.to(device=dev, dtype=torch.float32).contiguous()  # read on the device: no host sync
-        with _lib.on_device(dev):
-            g1 = torch.empty(b, n1, d, device=dev, dtype=torch.float32)
-            g2 = torch.empty(b, n2, d, device=dev, dtype=torch.float32)
-            rc = L.pcl_knn_bwd(*_lib.pts_args(p1), _lib.ptr(l1), *_lib.pts_args(p2), _lib.ptr(l2), b, n1, n2, d, K,
+        return _backward(ctx, grad_dists, "pcl_knn_bwd")
+
+
+def _backward(ctx, grad_dists, entry):
+    """Gradients of (p1, p2) through dists with `entry` (pcl_knn_bwd or pcl_ball_query_bwd), cast back to the inputs'
+    dtypes and devices; None for the other forward arguments."""
+    p1, p2, idx = ctx.saved_tensors
+    l1, l2 = ctx.lens
+    L = _lib.lib()
+    b, n1, d = p1.shape
+    n2, K = p2.shape[1], idx.shape[2]
+    dev = p1.device
+    g = grad_dists.to(device=dev, dtype=torch.float32).contiguous()  # read on the device: no host sync
+    with _lib.on_device(dev):
+        g1 = torch.empty(b, n1, d, device=dev, dtype=torch.float32)
+        g2 = torch.empty(b, n2, d, device=dev, dtype=torch.float32)
+        rc = getattr(L, entry)(*_lib.pts_args(p1), _lib.ptr(l1), *_lib.pts_args(p2), _lib.ptr(l2), b, n1, n2, d, K,
                                idx.data_ptr(), g.data_ptr(), g1.data_ptr(), g2.data_ptr(), _lib.stream_ptr(dev))
-            _lib.check(rc, "pcl_knn_bwd")
-        dt1, dev1, dt2, dev2 = ctx.in_meta
-        return g1.to(device=dev1, dtype=dt1), g2.to(device=dev2, dtype=dt2), None, None, None, None
+        _lib.check(rc, entry)
+    dt1, dev1, dt2, dev2 = ctx.in_meta
+    return (g1.to(device=dev1, dtype=dt1), g2.to(device=dev2, dtype=dt2)) + (None,) * (ctx.n_inputs - 2)
 
 
 def knn_gather(x, idx, lengths=None):
