@@ -78,7 +78,7 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
         if (rank == 0 && W.nworkers > 0) {  // the mirror the workers load: targets (c = 3: price 0), prices, original target indices
             __syncthreads();
             copy16_out(cl + W.o_tgt, S.tgt, n32);
-            copy16_out(cl + W.o_pf, S.pf, n8 / 4);
+            copy16_out(cl + W.o_pf, S.pf, n32 / 4);
             if (S.tperm) copy16_out(cl + W.o_tperm, S.tperm, n8 / 8);
         }
     }

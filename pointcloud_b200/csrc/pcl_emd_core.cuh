@@ -46,7 +46,7 @@ constexpr int EMD_F_COLD = 4;  // bids / per-object maxima / assignment arrays l
 struct EmdSmem {
     float4 *tgt;            // n32 {x, y, z, c = RU(3 - price)}, internal (sorted) target order, padded with far sentinels
     uint2 *pub;             // 2N  published bids {object | second<<16, increment bits}, double-buffered (sort scratch at init)
-    float *pf;              // N   price (fp32, as in the reference)
+    float *pf;              // n32 price (fp32, as in the reference); padding targets keep price 0
     float *maxinc;          // N   per-object running max increment (reference: max_increments)
     int *maxidx;            // N   per-object winning bidder, ORIGINAL index (reference: max_idx), -1 = none
     unsigned *last;         // N   previous bid of every bidder (object | second<<16), NOLAST = never bid
@@ -71,7 +71,7 @@ __host__ __device__ inline size_t emd_cold_bytes(int N) {
 }
 __host__ __device__ inline size_t emd_smem_bytes(int N, int flags, int pcap = EMD_THREADS) {
     const size_t n8 = (size_t)(N + 7) / 8 * 8, n32 = (size_t)(N + 31) / 32 * 32, nt = n32 / 32;
-    return n32 * 16 + n8 * 4 + ((flags & EMD_F_COLD) ? 0 : emd_cold_bytes(N)) + (size_t)pcap * 16 + 64 * 4 + 16 + nt * 32 +
+    return n32 * 16 + n32 * 4 + ((flags & EMD_F_COLD) ? 0 : emd_cold_bytes(N)) + (size_t)pcap * 16 + 64 * 4 + 16 + nt * 32 +
            ((flags & EMD_F_SORT) ? n8 * 4 : 0) + ((flags & EMD_F_X1) ? n8 * 16 : 0) + 64;
 }
 
@@ -85,7 +85,7 @@ __device__ inline EmdSmem carve(unsigned char *base, unsigned char *cold, int N,
     s.x1 = (flags & EMD_F_X1) ? (float4 *)p : nullptr; p += (flags & EMD_F_X1) ? n8 * 16 : 0;
     s.tperm = (flags & EMD_F_SORT) ? (unsigned short *)p : nullptr; p += (flags & EMD_F_SORT) ? n8 * 2 : 0;
     s.pperm = (flags & EMD_F_SORT) ? (unsigned short *)p : nullptr; p += (flags & EMD_F_SORT) ? n8 * 2 : 0;
-    s.pf = (float *)p; p += n8 * 4;
+    s.pf = (float *)p; p += n32 * 4;    // n32: the padding targets of the last tile are priced too (0)
     s.pbest = (float *)p; p += (size_t)pcap * 4;
     s.pbetter = (float *)p; p += (size_t)pcap * 4;
     s.pbi = (unsigned *)p; p += (size_t)pcap * 4;
@@ -305,7 +305,10 @@ __device__ __forceinline__ void emd_setup(const EmdSmem &S, const Pts &xyz1, con
             if (S.x1) { const float3 q = ld_xyz(xyz1, cloud, k); S.x1[k] = make_float4(q.x, q.y, q.z, 0.f); }
         }
     }
-    for (int k = N + tid; k < n32; k += T) S.tgt[k] = make_float4(1e18f, 1e18f, 1e18f, -1e30f);  // never a candidate
+    for (int k = N + tid; k < n32; k += T) S.tgt[k] = make_float4(1e18f, 1e18f, 1e18f, -1e30f);  // far away: never a bid
+    // Every lane of a candidate tile evaluates its target, the padding ones of the last tile included: their price must be a
+    // defined 0 (value 3 - sqrt(3e36) -- never a bid) rather than whatever the previous kernel left in shared memory.
+    for (int j = n8 + tid; j < n32; j += T) S.pf[j] = 0.f;
     for (int j = tid; j < n8; j += T) {
         S.pf[j] = 0.f;
         S.asg[j] = (j < N) ? NONE16 : (unsigned short)0;

@@ -35,7 +35,7 @@ __host__ __device__ inline size_t team_cloud_bytes(int N, size_t *o_tgt, size_t 
     const size_t n8 = (size_t)(N + 7) / 8 * 8, n32 = (size_t)(N + 31) / 32 * 32, nt = n32 / 32;
     size_t o = 0;
     auto put = [&](size_t *where, size_t bytes) { if (where) *where = o; o += (bytes + 255) / 256 * 256; };
-    put(o_tgt, n32 * 16); put(o_pf, n8 * 4); put(o_tperm, n8 * 2); put(o_box, nt * 32); put(o_brec, n8 * 16); put(o_pub, n8 * 16);
+    put(o_tgt, n32 * 16); put(o_pf, n32 * 4); put(o_tperm, n8 * 2); put(o_box, nt * 32); put(o_brec, n8 * 16); put(o_pub, n8 * 16);
     put(o_jp, n8 * 2);
     return o;
 }
@@ -381,7 +381,7 @@ __device__ void team_worker(const EmdSmem &S, const TeamWs &W, int B, int N, flo
         const unsigned char *cl = W.clouds + (size_t)c * W.stride;
         if (c != cached_c || t != cached_t) {  // this CTA's copy of the cloud's hot state is for another cloud / iteration
             // targets + prices + boxes (+ original indices for a new cloud): every thread has all its 16-byte loads in flight at once
-            const int c_tgt = n32, c_pf = n8 / 4, c_box = 2 * NT, c_tp = (c != cached_c && S.tperm) ? n8 / 8 : 0;
+            const int c_tgt = n32, c_pf = n32 / 4, c_box = 2 * NT, c_tp = (c != cached_c && S.tperm) ? n8 / 8 : 0;
             const int total = c_tgt + c_pf + c_box + c_tp;
             constexpr int PER = 8;  // 16 B x 8 x 512 threads = 64 KB per round
             for (int base = 0; base < total; base += PER * THREADS) {

@@ -49,7 +49,7 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
     __syncthreads();
     // the mirror of the hot state: targets (c = 3: price 0), prices, original target indices, tile boxes
     copy16_out(g_tgt, S.tgt, n32);
-    copy16_out(g_pf, S.pf, n8 / 4);
+    copy16_out(g_pf, S.pf, n32 / 4);
     if (S.tperm) copy16_out(cl + W.o_tperm, S.tperm, n8 / 8);
 
     auto pred_xyz = [&](int jp) -> float3 {

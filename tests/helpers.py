@@ -54,6 +54,14 @@ class RefEmdFunction(torch.autograd.Function):
         return None, gradxyz1, gradxyz2, None, None
 
 
+def reference_structure(eps, its, num_classes=None):
+    """The reference's own op-by-op loss structure (oracle/loss_oracle.py, utils.py:253-309) on top of the CUDA emdModule."""
+    import pointcloud_b200 as pcl
+    from oracle import loss_oracle
+    mod = pcl.emdModule()
+    return loss_oracle.EarthMoverDistance(eps, its, num_classes, emd_fn=lambda a, b, e, i: mod(a, b, e, i))
+
+
 def npy(t):
     return t.detach().cpu().numpy()
 

@@ -11,7 +11,7 @@ import torch.nn.functional as F
 import pointcloud_b200 as pcl
 from oracle import loss_oracle
 from pointcloud_b200 import synth
-from helpers import npy
+from helpers import npy, reference_structure
 
 pytestmark = pytest.mark.gpu
 REL = 1e-5
@@ -19,12 +19,6 @@ REL = 1e-5
 
 def _t(a):
     return torch.from_numpy(np.asarray(a))
-
-
-def reference_structure(eps, its, num_classes=None):
-    """The reference's own op-by-op loss structure (oracle/loss_oracle.py, utils.py:253-309) on top of the CUDA emdModule."""
-    mod = pcl.emdModule()
-    return loss_oracle.EarthMoverDistance(eps, its, num_classes, emd_fn=lambda a, b, e, i: mod(a, b, e, i))
 
 
 @pytest.mark.parametrize("fused", [True, False])
@@ -270,6 +264,123 @@ def test_fused_feature_term_entry_points():
     ref.backward()
     assert float(s2[0] / s2[1]) == pytest.approx(float(ref), rel=REL) and float(s2[1]) == b * n * 3
     np.testing.assert_allclose(npy(predf.grad), npy(q.grad), rtol=REL, atol=1e-10)
+
+
+def _seg_ce(L, logits, matched, cw, grad_sum):
+    """pcl_emd_seg_ce_fwd + _bwd through the C ABI -> (rc of the forward, sums, argmax histogram, fp32 gradient)."""
+    b, n, c = logits.shape
+    sums = torch.full((2,), float("nan"), device="cuda")
+    hist = torch.empty(c, device="cuda", dtype=torch.int64)
+    grad = torch.full((b, n, c), float("nan"), device="cuda")
+    g = torch.tensor([grad_sum], device="cuda")
+    wsb = L.pcl_emd_feature_workspace_bytes()
+    ws = torch.empty(wsb, device="cuda", dtype=torch.uint8)
+    st = torch.cuda.current_stream().cuda_stream
+    rc = L.pcl_emd_seg_ce_fwd(*pcl._lib.pts_args(logits), matched.data_ptr(), cw.data_ptr(), b, n, c, sums.data_ptr(), hist.data_ptr(),
+                              ws.data_ptr(), wsb, st)
+    if rc:
+        return rc, None, None, None
+    assert L.pcl_emd_seg_ce_bwd(*pcl._lib.pts_args(logits), matched.data_ptr(), cw.data_ptr(), b, n, c, g.data_ptr(), grad.data_ptr(), st) == 0
+    torch.cuda.synchronize()
+    return rc, npy(sums), npy(hist), npy(grad)
+
+
+@pytest.mark.parametrize("dt", [torch.float32, torch.float16])
+@pytest.mark.parametrize("C", [1, 2, 33, 64])
+def test_seg_cross_entropy_kernels_at_their_limits(C, dt):
+    """pcl_emd_seg_ce_fwd / _bwd against float64 torch up to EP_MAX_C = 64 classes, logits spread over +-50, fp16 logits,
+    matched labels outside [0, C) (no weight, no gradient), and rows whose maximum is tied: the argmax histogram counts the
+    FIRST maximum, like torch.argmax."""
+    L = pcl._lib.lib()
+    g = torch.Generator().manual_seed(60 + C)
+    b, n = 4, 1000
+    z = (torch.rand(b, n, 3 + C, generator=g) * 100 - 50).to(dt)
+    ties = torch.rand(b, n, generator=g) < 0.3
+    if C > 1:                                            # copy each tied row's maximum to another, random class
+        zf = z.float()
+        am = zf[:, :, 3:].argmax(2, keepdim=True)
+        other = torch.randint(0, C, (b, n, 1), generator=g)
+        row_max = zf[:, :, 3:].gather(2, am)
+        z[:, :, 3:].scatter_(2, other, torch.where(ties[..., None], row_max, zf[:, :, 3:].gather(2, other)).to(dt))
+    logits = z.cuda()[:, :, 3:]                          # strided view, row stride 3 + C
+    matched = torch.randint(0, C, (b, n), generator=g, dtype=torch.int32)
+    matched[:, ::97] = -1
+    matched[:, 5::89] = C
+    cw = torch.rand(C, generator=g) + 0.1
+    rc, sums, hist, grad = _seg_ce(L, logits, matched.cuda(), cw.cuda(), 0.7)
+    assert rc == 0, L.pcl_last_error()
+    q = logits.cpu().double()
+    lab = matched.long()
+    ok = (lab >= 0) & (lab < C)
+    lse = torch.logsumexp(q, 2)
+    w = torch.where(ok, cw.double()[lab.clamp(0, C - 1)], torch.zeros((), dtype=torch.float64))
+    nll = lse - q.gather(2, lab.clamp(0, C - 1)[..., None])[..., 0]
+    num, den = float((w * nll).sum()), float(w.sum())
+    assert abs(float(sums[0]) - num) <= REL * abs(num) + 1e-6 and float(sums[1]) == pytest.approx(den, rel=1e-6)
+    first_max = q.argmax(2)                              # torch.argmax: the first maximal index
+    if C > 1:
+        last_max = C - 1 - q.flip(2).argmax(2)
+        assert (first_max != last_max).sum() > 100       # the tie rule decides the histogram
+    assert np.array_equal(hist, np.bincount(first_max.view(-1).numpy(), minlength=C))
+    want = 0.7 * w[..., None] * (torch.softmax(q, 2) - F.one_hot(lab.clamp(0, C - 1), C).double() * ok[..., None])
+    np.testing.assert_allclose(grad, want.numpy(), rtol=REL, atol=1e-6 * max(float(want.abs().max()), 1e-30))
+    assert not grad[~ok.numpy()].any()
+    if C == 64:                                          # one class more than the kernels hold
+        z65 = torch.rand(b, n, 65, generator=g).cuda()
+        from pointcloud_b200._lib import PclError
+        from pointcloud_b200.losses import _SegCrossEntropySums
+        with pytest.raises(PclError):
+            _SegCrossEntropySums.apply(z65, matched.cuda(), torch.rand(65).cuda())
+        gbuf, one = torch.empty(b, n, 65, device="cuda"), torch.ones(1, device="cuda")
+        assert L.pcl_emd_seg_ce_bwd(*pcl._lib.pts_args(z65), matched.cuda().data_ptr(), torch.rand(65).cuda().data_ptr(), b, n, 65,
+                                    one.data_ptr(), gbuf.data_ptr(), torch.cuda.current_stream().cuda_stream) != 0
+
+
+@pytest.mark.parametrize("F_", [1, 5, 13])
+def test_matched_feature_mse_kernels_feature_widths(F_):
+    """pcl_emd_feat_mse_fwd / _bwd against float64 torch for F = 1, 5, 13 feature channels (strided views, a non-bijective
+    assignment): sums[0] within 1e-5, sums[1] = B*N*F exactly, gradient 2 * g * (feat - tfeat[assignment])."""
+    from pointcloud_b200.losses import _MatchedFeatureMSESums
+    g = torch.Generator().manual_seed(70 + F_)
+    b, n = 3, 1500
+    pred = torch.rand(b, n, 3 + F_, generator=g).cuda().requires_grad_()
+    target = torch.rand(b, n, 3 + F_, generator=g).cuda()
+    asg = torch.randint(0, n, (b, n), generator=g).int().cuda()
+    s = _MatchedFeatureMSESums.apply(pred[:, :, 3:], target[:, :, 3:], asg)
+    (s[0] * 0.37).backward()
+    diff = pred.detach().double()[:, :, 3:] - target.double().take_along_dim(asg.long().unsqueeze(-1), 1)[:, :, 3:]
+    num = float((diff ** 2).sum())
+    assert abs(float(s[0]) - num) <= REL * num and float(s[1]) == b * n * F_
+    np.testing.assert_allclose(npy(pred.grad[:, :, 3:]), npy(0.37 * 2 * diff), rtol=REL, atol=1e-12)
+    assert not pred.grad[:, :, :3].any()
+
+
+@pytest.mark.parametrize("dt", [torch.float32, torch.float16])
+def test_match_hist_truncates_labels_like_long(dt):
+    """pcl_emd_match_hist at C = 64 with labels that are negative, fractional (-0.5 truncates to 0) or >= C, and unassigned
+    points: hist = torch.bincount of the matched targets' labels .long(), restricted to [0, C); matched = those labels."""
+    L = pcl._lib.lib()
+    g = torch.Generator().manual_seed(80)
+    b, n, c = 5, 900, 64
+    values = torch.tensor([-3.0, -1.0, -0.5, 0.0, 0.7, 1.0, 5.5, 31.0, 62.9, 63.0, 64.0, 65.0, 100.0])
+    lab = torch.where(torch.rand(b, n, generator=g) < 0.5, values[torch.randint(0, len(values), (b, n), generator=g)],
+                      torch.randint(0, c, (b, n), generator=g).float())
+    target = torch.rand(b, n, 4, generator=g)
+    target[:, :, 3] = lab
+    tl = target.to(dt).cuda()[:, :, 3:4]
+    asg = torch.randint(0, n, (b, n), generator=g, dtype=torch.int32)
+    asg[:, ::50] = -1
+    hist = torch.empty(c, device="cuda", dtype=torch.int64)
+    matched = torch.empty(b, n, device="cuda", dtype=torch.int32)
+    rc = L.pcl_emd_match_hist(*pcl._lib.pts_args(tl), asg.cuda().data_ptr(), b, n, c, hist.data_ptr(), matched.data_ptr(),
+                              torch.cuda.current_stream().cuda_stream)
+    assert rc == 0, L.pcl_last_error()
+    lab_long = tl[..., 0].cpu().float().long()
+    want = torch.where(asg >= 0, lab_long.gather(1, asg.long().clamp(min=0)), torch.full((), -1, dtype=torch.long))
+    assert torch.equal(matched.cpu().long(), want)
+    inside = want[(want >= 0) & (want < c)]
+    assert torch.equal(hist.cpu(), torch.bincount(inside, minlength=c)[:c])
+    assert (lab.gather(1, asg.long().clamp(min=0))[asg >= 0] == -0.5).any()   # some matched label truncates from -0.5 to class 0
 
 
 def test_class_filter_kernel_matches_the_reference_loop():
