@@ -66,6 +66,15 @@ def npy(t):
     return t.detach().cpu().numpy()
 
 
+def same_bits(a, b):
+    """Bitwise equality of float32 arrays, with any NaN equal to any NaN (the payload is not specified)."""
+    a, b = np.asarray(a, np.float32), np.asarray(b, np.float32)
+    if a.shape != b.shape:
+        return False
+    nan_a, nan_b = np.isnan(a), np.isnan(b)
+    return bool(np.array_equal(nan_a, nan_b) and np.array_equal(a.view(np.int32)[~nan_a], b.view(np.int32)[~nan_b]))
+
+
 def sqdist_to_match(x1, x2, asg):
     m = np.take_along_axis(np.asarray(x2), np.asarray(asg).astype(np.int64)[..., None], 1)
     return ((np.asarray(x1, dtype=np.float64) - m) ** 2).sum(-1)

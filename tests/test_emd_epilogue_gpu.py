@@ -17,7 +17,7 @@ import pointcloud_b200 as pcl
 from oracle import loss_oracle
 from pointcloud_b200 import _lib, synth
 from emd_epilogue_ref import epilogue_grad, epilogue_sum, float32_neighbours
-from helpers import npy, reference_structure
+from helpers import npy, reference_structure, same_bits
 
 pytestmark = pytest.mark.gpu
 EPS = 0.005
@@ -91,15 +91,6 @@ def fused_call(x1, x2, iters, grad_scale):
     assert rc == 0, L.pcl_last_error()
     torch.cuda.synchronize()
     return npy(dist), npy(asg), npy(stats), npy(grad), npy(sums)
-
-
-def same_bits(a, b):
-    """Bitwise equality of float32 arrays, with any NaN equal to any NaN (the payload is not specified)."""
-    a, b = np.asarray(a, np.float32), np.asarray(b, np.float32)
-    if a.shape != b.shape:
-        return False
-    nan_a, nan_b = np.isnan(a), np.isnan(b)
-    return bool(np.array_equal(nan_a, nan_b) and np.array_equal(a.view(np.int32)[~nan_a], b.view(np.int32)[~nan_b]))
 
 
 def check_sums(sums, dist):
