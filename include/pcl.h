@@ -96,6 +96,39 @@ PCL_API int pcl_chamfer_bwd(const void *x, int x_dtype, int64_t x_bs, int64_t x_
                     const void *y, int y_dtype, int64_t y_bs, int64_t y_rs, const int64_t *y_len,
                     int B, int P1, int P2, int D, const int32_t *idx_x, const int32_t *idx_y,
                     const float *grad_out, float *grad_x, float *grad_y, void *stream);
+/*
+ * pcl_chamfer_fwd plus what the rest of pytorch3d's chamfer_distance needs: per-cloud results (weights, batch_reduction None /
+ * "sum") and the normal-consistency term (x_normals / y_normals).  pcl_chamfer_fwd is this call with every new pointer NULL.
+ *   cloud_sums: nullable DEVICE float[2*B]: cloud_sums[d*B + n] = sum_{i < len} dist (d = 0: x -> y, d = 1: y -> x),
+ *     un-normalised, the per-cloud sums loss_xy is made of.
+ *   x_nrm / y_nrm: (B,P1,3) / (B,P2,3) normals, strided like the points (pointer, dtype, batch stride, row stride); read only
+ *     when normal_sums is not NULL, and then both are required.
+ *   normal_sums: nullable DEVICE float[2*B]: normal_sums[d*B + n] = sum_{i < len} (1 - |cos(n_i, n'_{idx[i]})|), the cosine as
+ *     F.cosine_similarity(eps=1e-6) forms it; a query whose target cloud is empty adds 1 (its neighbour's normal is taken as 0).
+ * It still writes dist / idx and loss_xy, and uses the same workspace (pcl_chamfer_workspace_bytes).  With normal_sums a second
+ * kernel runs after the search.
+ */
+PCL_API int pcl_chamfer_cloud_fwd(const void *x, int x_dtype, int64_t x_bs, int64_t x_rs, const int64_t *x_len,
+                    const void *y, int y_dtype, int64_t y_bs, int64_t y_rs, const int64_t *y_len,
+                    int B, int P1, int P2, int D, int mode,
+                    float *dist_x, int32_t *idx_x, float *dist_y, int32_t *idx_y, float *loss_xy, float *cloud_sums,
+                    const void *x_nrm, int x_nrm_dtype, int64_t x_nrm_bs, int64_t x_nrm_rs,
+                    const void *y_nrm, int y_nrm_dtype, int64_t y_nrm_bs, int64_t y_nrm_rs, float *normal_sums,
+                    void *workspace, size_t workspace_bytes, void *stream);
+/*
+ * Backward of pcl_chamfer_cloud_fwd.  grad_cloud: DEVICE float[2*B] (may be NULL when B = 0), the upstream gradients of cloud_sums:
+ *   grad_x[i] += 2*grad_cloud[n]*(x_i - y[idx_x[i]]);  grad_y[idx_x[i]] -= same;  symmetrically with grad_cloud[B + n].
+ * grad_normal: nullable DEVICE float[2*B], the upstream gradients of normal_sums; when given, x_nrm / y_nrm are required and
+ * grad_x_nrm (B,P1,3), grad_y_nrm (B,P2,3) receive the normal term's gradient (each query's own normal and, scattered, its
+ * neighbour's; 0 where the target cloud is empty).  All gradient outputs are dense fp32 and are overwritten.  No host sync.
+ */
+PCL_API int pcl_chamfer_cloud_bwd(const void *x, int x_dtype, int64_t x_bs, int64_t x_rs, const int64_t *x_len,
+                    const void *y, int y_dtype, int64_t y_bs, int64_t y_rs, const int64_t *y_len,
+                    int B, int P1, int P2, int D, const int32_t *idx_x, const int32_t *idx_y,
+                    const float *grad_cloud, float *grad_x, float *grad_y,
+                    const void *x_nrm, int x_nrm_dtype, int64_t x_nrm_bs, int64_t x_nrm_rs,
+                    const void *y_nrm, int y_nrm_dtype, int64_t y_nrm_bs, int64_t y_nrm_rs,
+                    const float *grad_normal, float *grad_x_nrm, float *grad_y_nrm, void *stream);
 
 /* ------------------------------------------------------------------ EMD (auction) ------------------------- */
 /*

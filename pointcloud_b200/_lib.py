@@ -28,6 +28,10 @@ _SIGNATURES = {
     "pcl_chamfer_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "pcl_chamfer_fwd": (c_int, _PTS + [c_void_p] + _PTS + [c_void_p] + [c_int] * 5 + [c_void_p] * 5 + [c_void_p, c_size_t, c_void_p]),
     "pcl_chamfer_bwd": (c_int, _PTS + [c_void_p] + _PTS + [c_void_p] + [c_int] * 4 + [c_void_p] * 5 + [c_void_p]),
+    "pcl_chamfer_cloud_fwd": (c_int, _PTS + [c_void_p] + _PTS + [c_void_p] + [c_int] * 5 + [c_void_p] * 6 + _PTS + _PTS + [c_void_p]
+                              + [c_void_p, c_size_t, c_void_p]),
+    "pcl_chamfer_cloud_bwd": (c_int, _PTS + [c_void_p] + _PTS + [c_void_p] + [c_int] * 4 + [c_void_p] * 5 + _PTS + _PTS + [c_void_p] * 3
+                              + [c_void_p]),
     "pcl_emd_max_points": (c_int, []),
     "pcl_emd_set_path": (c_int, [c_int]),
     "pcl_emd_workspace_bytes": (c_size_t, [c_int, c_int]),

@@ -60,12 +60,14 @@ __device__ __forceinline__ float sqdist3(float qx, float qy, float qz, const flo
     else return __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz));
 }
 
-// Tail of both forward kernels: the CTA's partial sum goes to the workspace; the CTA that takes the LAST ticket of the grid
+// Tail of the forward kernels: the CTA's partial sum goes to the workspace; the CTA that takes the LAST ticket of the grid
 // (zeroed by the host call) then forms  loss_xy[dir] = sum_n (sum_i dist / clamp(len,1)) / max(B,1)  from all partials in a
 // fixed order (deterministic scalar, fp64) -- no memset of the partials and no second launch.  Needs >= 64 threads per CTA.
+// cloud_sums (nullable, (2, B)) receives every cloud's un-normalised sum; loss_xy is nullable for the normal-term pass.
 __device__ __forceinline__ void finish_block(float s /* valid on thread 0 */, float *__restrict__ partial, int nblk, int dir, int n,
                                              unsigned *__restrict__ ticket, int P1, int P2, const int64_t *__restrict__ x_len,
-                                             const int64_t *__restrict__ y_len, float *__restrict__ loss_xy) {
+                                             const int64_t *__restrict__ y_len, float *__restrict__ loss_xy,
+                                             float *__restrict__ cloud_sums) {
     __shared__ int last_flag;
     const int B = (int)gridDim.y;
     if (threadIdx.x == 0) {
@@ -82,12 +84,13 @@ __device__ __forceinline__ void finish_block(float s /* valid on thread 0 */, fl
     for (int c = lane; c < B; c += 32) {
         double t = 0.0;
         for (int k = 0; k < (int)gridDim.x; k++) t += (double)__ldcg(&partial[((size_t)d * B + c) * nblk + k]);
+        if (cloud_sums) cloud_sums[d * B + c] = (float)t;
         const int len = d ? len_of(y_len, c, P2) : len_of(x_len, c, P1);
         a += t / (double)(len > 1 ? len : 1);
     }
     acc[d][lane] = a;
     __syncwarp();
-    if (lane == 0) {
+    if (lane == 0 && loss_xy) {
         double t = 0.0;
         for (int k = 0; k < 32; k++) t += acc[d][k];
         loss_xy[d] = (float)(t / (double)(B > 1 ? B : 1));
@@ -164,7 +167,7 @@ __global__ void __launch_bounds__(C3_THREADS, PCL_C3_MINB)
 chamfer_nn3_kernel(Pts x, const int64_t *__restrict__ x_len, Pts y, const int64_t *__restrict__ y_len, int P1, int P2,
                    float *__restrict__ dist_x, int *__restrict__ idx_x, float *__restrict__ dist_y,
                    int *__restrict__ idx_y, float *__restrict__ partial, int nblk, unsigned *__restrict__ ticket,
-                   float *__restrict__ loss_xy) {
+                   float *__restrict__ loss_xy, float *__restrict__ cloud_sums) {
     __shared__ float4 tA[C3_TILE / 2 + C3_GROUP];  // per pair of targets {x0, x1, y0, y1} (+ slack for the read-ahead)
     __shared__ float4 tB[C3_TILE / 2 + C3_GROUP];  //                     {z0, z1, |t0|^2, |t1|^2}
     constexpr int C3_PPT = C3_TILE / C3_THREADS;   // staged points per thread and tile
@@ -176,7 +179,7 @@ chamfer_nn3_kernel(Pts x, const int64_t *__restrict__ x_len, Pts y, const int64_
     const int PQ = dir ? P2 : P1;
     const int q0 = blockIdx.x * C3_QUERIES;
     if (q0 >= PQ) {  // block-uniform: beyond the shorter cloud -- contributes a zero partial (and may be the last CTA)
-        finish_block(0.f, partial, nblk, dir, n, ticket, P1, P2, x_len, y_len, loss_xy);
+        finish_block(0.f, partial, nblk, dir, n, ticket, P1, P2, x_len, y_len, loss_xy, cloud_sums);
         return;
     }
     const int lq = dir ? len_of(y_len, n, P2) : len_of(x_len, n, P1);
@@ -334,7 +337,7 @@ chamfer_nn3_kernel(Pts x, const int64_t *__restrict__ x_len, Pts y, const int64_
         }
     }
     s = block_sum<C3_THREADS / 32>(s, red);
-    finish_block(s, partial, nblk, dir, n, ticket, P1, P2, x_len, y_len, loss_xy);
+    finish_block(s, partial, nblk, dir, n, ticket, P1, P2, x_len, y_len, loss_xy, cloud_sums);
 }
 
 
@@ -487,7 +490,8 @@ template <bool FMA>
 __global__ void __launch_bounds__(PR_NN_WARPS * 32)
 chamfer_nn3_pruned_kernel(const int64_t *__restrict__ x_len, const int64_t *__restrict__ y_len, int P1, int P2, PruneWs W,
                           float *__restrict__ dist_x, int *__restrict__ idx_x, float *__restrict__ dist_y, int *__restrict__ idx_y,
-                          float *__restrict__ partial, int nblk, unsigned *__restrict__ ticket, float *__restrict__ loss_xy) {
+                          float *__restrict__ partial, int nblk, unsigned *__restrict__ ticket, float *__restrict__ loss_xy,
+                          float *__restrict__ cloud_sums) {
     __shared__ float red[PR_NN_WARPS];
     const int dir = blockIdx.z, n = blockIdx.y, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int PQ = dir ? P2 : P1;
@@ -583,7 +587,7 @@ chamfer_nn3_pruned_kernel(const int64_t *__restrict__ x_len, const int64_t *__re
         }
     }
     s = block_sum<PR_NN_WARPS>(s, red);
-    finish_block(s, partial, nblk, dir, n, ticket, P1, P2, x_len, y_len, loss_xy);
+    finish_block(s, partial, nblk, dir, n, ticket, P1, P2, x_len, y_len, loss_xy, cloud_sums);
 }
 
 // Generic feature width (ChamferDistance over all channels, utils.py:209-211).  One query per thread.
@@ -592,7 +596,7 @@ __global__ void __launch_bounds__(CH_THREADS)
 chamfer_nnD_kernel(Pts x, const int64_t *__restrict__ x_len, Pts y, const int64_t *__restrict__ y_len, int P1, int P2,
                    float *__restrict__ dist_x, int *__restrict__ idx_x, float *__restrict__ dist_y,
                    int *__restrict__ idx_y, float *__restrict__ partial, int nblk, unsigned *__restrict__ ticket,
-                   float *__restrict__ loss_xy) {
+                   float *__restrict__ loss_xy, float *__restrict__ cloud_sums) {
     constexpr int TILE = 512;
     __shared__ float tile[TILE * D];
     __shared__ float red[4];
@@ -601,7 +605,7 @@ chamfer_nnD_kernel(Pts x, const int64_t *__restrict__ x_len, Pts y, const int64_
     const int PQ = dir ? P2 : P1;
     const int q0 = blockIdx.x * CH_THREADS;
     if (q0 >= PQ) {
-        finish_block(0.f, partial, nblk, dir, n, ticket, P1, P2, x_len, y_len, loss_xy);
+        finish_block(0.f, partial, nblk, dir, n, ticket, P1, P2, x_len, y_len, loss_xy, cloud_sums);
         return;
     }
     const int lq = dir ? len_of(y_len, n, P2) : len_of(x_len, n, P1);
@@ -643,16 +647,66 @@ chamfer_nnD_kernel(Pts x, const int64_t *__restrict__ x_len, Pts y, const int64_
         dist[i] = s; idx[i] = valid ? bi : 0;
     }
     s = block_sum<4>(s, red);
-    finish_block(s, partial, nblk, dir, n, ticket, P1, P2, x_len, y_len, loss_xy);
+    finish_block(s, partial, nblk, dir, n, ticket, P1, P2, x_len, y_len, loss_xy, cloud_sums);
+}
+
+// ---- normal consistency (pytorch3d's x_normals / y_normals) ---------------------------------------------------------------------
+// The cosine exactly as F.cosine_similarity(a, b, dim, eps=1e-6) forms it: each vector divided by max(|v|, eps), then the dot
+// product.  Its gradient (torch's, where the clamp of the norm carries no gradient) is  dc/da = (b/mb - c a/|a|) / ma  with
+// a/|a| = 0 for a = 0 (the norm's subgradient there).
+constexpr float NRM_EPS = 1e-6f;
+struct NrmCos {
+    float c, ma, mb, ia, ib;  // cosine, max(|a|, eps), max(|b|, eps), 1/|a| and 1/|b| (0 for a zero vector)
+};
+__device__ __forceinline__ NrmCos nrm_cos(float3 a, float3 b) {
+    NrmCos r;
+    const float na = sqrtf(fmaf(a.z, a.z, fmaf(a.y, a.y, a.x * a.x))), nb = sqrtf(fmaf(b.z, b.z, fmaf(b.y, b.y, b.x * b.x)));
+    r.ma = fmaxf(na, NRM_EPS); r.mb = fmaxf(nb, NRM_EPS);
+    r.ia = na > 0.f ? 1.f / na : 0.f; r.ib = nb > 0.f ? 1.f / nb : 0.f;
+    r.c = (a.x / r.ma) * (b.x / r.mb) + (a.y / r.ma) * (b.y / r.mb) + (a.z / r.ma) * (b.z / r.mb);
+    return r;
+}
+
+// Forward of the normal term: grid (ceil(maxP / 128), B, 2), one thread per query, launched after the search on the same stream.
+// normal_sums[dir * B + n] = sum over the valid queries i of 1 - |cos(nq_i, nt_idx[i])|; 1 per query when the target cloud is
+// empty (pytorch3d's knn_gather pads the missing neighbour's normal with zeros, so the cosine is 0).  The per-CTA partials and
+// the ticket are the search's workspace regions, consumed by the search's last CTA before this launch starts; the host re-zeroes
+// the ticket.
+__global__ void __launch_bounds__(CH_THREADS)
+chamfer_normal_kernel(Pts xn, const int64_t *__restrict__ x_len, Pts yn, const int64_t *__restrict__ y_len, int P1, int P2,
+                      const int *__restrict__ idx_x, const int *__restrict__ idx_y, float *__restrict__ partial, int nblk,
+                      unsigned *__restrict__ ticket, float *__restrict__ normal_sums) {
+    __shared__ float red[CH_THREADS / 32];
+    const int dir = blockIdx.z, n = blockIdx.y, i = blockIdx.x * CH_THREADS + threadIdx.x;
+    const Pts q = dir ? yn : xn, t = dir ? xn : yn;
+    const int PQ = dir ? P2 : P1;
+    const int lq = dir ? len_of(y_len, n, P2) : len_of(x_len, n, P1);
+    const int lt = dir ? len_of(x_len, n, P1) : len_of(y_len, n, P2);
+    float s = 0.f;
+    if (i < lq) {
+        s = 1.f;
+        if (lt > 0) {
+            const int j = __ldg((dir ? idx_y : idx_x) + (size_t)n * PQ + i);
+            s = 1.f - fabsf(nrm_cos(ld_xyz(q, n, i), ld_xyz(t, n, j)).c);
+        }
+    }
+    s = block_sum<CH_THREADS / 32>(s, red);
+    finish_block(s, partial, nblk, dir, n, ticket, P1, P2, x_len, y_len, nullptr, normal_sums);
 }
 
 // Backward: grid (ceil(maxP/256), B, 2).  All contributions go through fp32 red.global.add onto
 // zero-filled outputs (same accumulation model as pytorch3d's CUDA knn backward).
+// The factor of a cloud's distances is grad_cloud[dir * B + n] (the upstream gradient of its un-normalised sum) when given, else
+// g / max(B,1) / clamp(len,1).  With grad_normal, the thread also adds the normal term's gradient to its query's normal and
+// scatters the target's share to the neighbour's normal (NRM: a separate instantiation, so that the plain backward keeps its
+// register count).
+template <bool NRM>
 __global__ void __launch_bounds__(256)
 chamfer_bwd_kernel(Pts x, const int64_t *__restrict__ x_len, Pts y, const int64_t *__restrict__ y_len, int B, int P1,
                    int P2, int D, const int *__restrict__ idx_x, const int *__restrict__ idx_y,
-                   const float *__restrict__ grad_out, float g_imm_x, float g_imm_y, float *__restrict__ grad_x,
-                   float *__restrict__ grad_y) {
+                   const float *__restrict__ grad_out, float g_imm_x, float g_imm_y, const float *__restrict__ grad_cloud,
+                   float *__restrict__ grad_x, float *__restrict__ grad_y, Pts xn, Pts yn, const float *__restrict__ grad_normal,
+                   float *__restrict__ grad_xn, float *__restrict__ grad_yn) {
     const int dir = blockIdx.z, n = blockIdx.y;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     const Pts q = dir ? y : x, t = dir ? x : y;
@@ -660,8 +714,13 @@ chamfer_bwd_kernel(Pts x, const int64_t *__restrict__ x_len, Pts y, const int64_
     const int lq = dir ? len_of(y_len, n, P2) : len_of(x_len, n, P1);
     const int lt = dir ? len_of(x_len, n, P1) : len_of(y_len, n, P2);
     if (i >= lq || lt <= 0) return;
-    const float g = grad_out ? __ldg(grad_out + dir) : (dir ? g_imm_y : g_imm_x);  // upstream gradient: device scalar or immediate
-    const float gd = g / (float)(B > 1 ? B : 1) / (float)(lq > 1 ? lq : 1);
+    float gd;
+    if (grad_cloud) {
+        gd = __ldg(grad_cloud + dir * B + n);
+    } else {
+        const float g = grad_out ? __ldg(grad_out + dir) : (dir ? g_imm_y : g_imm_x);  // upstream gradient: device scalar or immediate
+        gd = g / (float)(B > 1 ? B : 1) / (float)(lq > 1 ? lq : 1);
+    }
     const int j = (dir ? idx_y : idx_x)[(size_t)n * PQ + i];
     float *gq = (dir ? grad_y : grad_x) + ((size_t)n * PQ + i) * D;
     float *gt = (dir ? grad_x : grad_y) + ((size_t)n * PT + j) * D;
@@ -671,20 +730,34 @@ chamfer_bwd_kernel(Pts x, const int64_t *__restrict__ x_len, Pts y, const int64_
         atomicAdd(gq + c, diff);
         atomicAdd(gt + c, -diff);
     }
+    if constexpr (NRM) {
+        const float3 a = ld_xyz(dir ? yn : xn, n, i), b = ld_xyz(dir ? xn : yn, n, j);
+        const NrmCos r = nrm_cos(a, b);
+        const float gn = __ldg(grad_normal + dir * B + n);
+        const float sg = r.c > 0.f ? -gn : (r.c < 0.f ? gn : 0.f);  // d(1 - |c|)/dc = -sign(c), sign(0) = 0
+        const float av[3] = {a.x, a.y, a.z}, bv[3] = {b.x, b.y, b.z};
+        float *gqn = (dir ? grad_yn : grad_xn) + ((size_t)n * PQ + i) * 3;
+        float *gtn = (dir ? grad_xn : grad_yn) + ((size_t)n * PT + j) * 3;
+#pragma unroll
+        for (int c = 0; c < 3; c++) {
+            atomicAdd(gqn + c, sg * ((bv[c] / r.mb - r.c * (av[c] * r.ia)) / r.ma));
+            atomicAdd(gtn + c, sg * ((av[c] / r.ma - r.c * (bv[c] * r.ib)) / r.mb));
+        }
+    }
 }
 
 template <bool FMA>
 int launch_fwd(const Pts &x, const int64_t *x_len, const Pts &y, const int64_t *y_len, int B, int P1, int P2, int D,
                float *dist_x, int *idx_x, float *dist_y, int *idx_y, float *partial, int nblk, unsigned *ticket, float *loss_xy,
-               cudaStream_t st) {
+               float *cloud_sums, cudaStream_t st) {
     const int maxP = P1 > P2 ? P1 : P2;
     if (D == 3) {
         dim3 grid((maxP + C3_QUERIES - 1) / C3_QUERIES, B, 2);
-        chamfer_nn3_kernel<FMA><<<grid, C3_THREADS, 0, st>>>(x, x_len, y, y_len, P1, P2, dist_x, idx_x, dist_y, idx_y, partial, nblk, ticket, loss_xy);
+        chamfer_nn3_kernel<FMA><<<grid, C3_THREADS, 0, st>>>(x, x_len, y, y_len, P1, P2, dist_x, idx_x, dist_y, idx_y, partial, nblk, ticket, loss_xy, cloud_sums);
     } else {
         dim3 grid((maxP + CH_THREADS - 1) / CH_THREADS, B, 2);
 #define PCL_LAUNCH_NND(DD) \
-    case DD: chamfer_nnD_kernel<FMA, DD><<<grid, CH_THREADS, 0, st>>>(x, x_len, y, y_len, P1, P2, dist_x, idx_x, dist_y, idx_y, partial, nblk, ticket, loss_xy); break
+    case DD: chamfer_nnD_kernel<FMA, DD><<<grid, CH_THREADS, 0, st>>>(x, x_len, y, y_len, P1, P2, dist_x, idx_x, dist_y, idx_y, partial, nblk, ticket, loss_xy, cloud_sums); break
         switch (D) {
             PCL_LAUNCH_NND(1); PCL_LAUNCH_NND(2); PCL_LAUNCH_NND(4); PCL_LAUNCH_NND(5);
             PCL_LAUNCH_NND(6); PCL_LAUNCH_NND(7); PCL_LAUNCH_NND(8);
@@ -752,15 +825,27 @@ extern "C" size_t pcl_chamfer_workspace_bytes(int B, int P1, int P2) {
     return 256 + align_up((size_t)2 * B * nblk_for(P1, P2) * sizeof(float), 256) + prune_bytes(B, P1, P2);  // [ticket][per-CTA partial sums][sorted clouds + tile boxes of the pruned path]
 }
 
-extern "C" int pcl_chamfer_fwd(const void *x, int x_dtype, int64_t x_bs, int64_t x_rs, const int64_t *x_len,
-                               const void *y, int y_dtype, int64_t y_bs, int64_t y_rs, const int64_t *y_len, int B,
-                               int P1, int P2, int D, int mode, float *dist_x, int32_t *idx_x, float *dist_y,
-                               int32_t *idx_y, float *loss_xy, void *workspace, size_t workspace_bytes, void *stream) {
+// A nullable (B, P, 3) normals array: valid when absent (normal term off) or when its dtype is known and it is there whenever
+// its cloud has rows.
+static bool normals_ok(const void *nx, int nx_dtype, const void *ny, int ny_dtype, int B, int P1, int P2) {
+    return dtype_ok(nx_dtype) && dtype_ok(ny_dtype) && !(B > 0 && ((P1 > 0 && !nx) || (P2 > 0 && !ny)));
+}
+
+extern "C" int pcl_chamfer_cloud_fwd(const void *x, int x_dtype, int64_t x_bs, int64_t x_rs, const int64_t *x_len,
+                                     const void *y, int y_dtype, int64_t y_bs, int64_t y_rs, const int64_t *y_len, int B,
+                                     int P1, int P2, int D, int mode, float *dist_x, int32_t *idx_x, float *dist_y,
+                                     int32_t *idx_y, float *loss_xy, float *cloud_sums,
+                                     const void *x_nrm, int x_nrm_dtype, int64_t x_nrm_bs, int64_t x_nrm_rs,
+                                     const void *y_nrm, int y_nrm_dtype, int64_t y_nrm_bs, int64_t y_nrm_rs, float *normal_sums,
+                                     void *workspace, size_t workspace_bytes, void *stream) {
     int rc = check_args(x, x_dtype, y, y_dtype, B, P1, P2, D);
     if (rc) return rc;
     if (mode != PCL_CHAMFER_UNFUSED && mode != PCL_CHAMFER_FMA) { set_error("chamfer: bad mode %d", mode); return PCL_E_ARG; }
     if (!loss_xy || (B > 0 && ((P1 > 0 && (!dist_x || !idx_x)) || (P2 > 0 && (!dist_y || !idx_y))))) {
         set_error("chamfer: null output"); return PCL_E_ARG;
+    }
+    if (normal_sums && !normals_ok(x_nrm, x_nrm_dtype, y_nrm, y_nrm_dtype, B, P1, P2)) {
+        set_error("chamfer: normal_sums needs both normals arrays (fp32 / fp16 / bf16)"); return PCL_E_ARG;
     }
     if (workspace_bytes < pcl_chamfer_workspace_bytes(B, P1, P2) || !workspace) {
         set_error("chamfer: workspace too small (%zu < %zu)", workspace_bytes, pcl_chamfer_workspace_bytes(B, P1, P2));
@@ -771,18 +856,20 @@ extern "C" int pcl_chamfer_fwd(const void *x, int x_dtype, int64_t x_bs, int64_t
     if ((rc = device_info(&di))) return rc;
     if (B == 0 || (P1 == 0 && P2 == 0)) {
         PCL_CUDA(cudaMemsetAsync(loss_xy, 0, 4 * sizeof(float), st));
+        if (B > 0 && cloud_sums) PCL_CUDA(cudaMemsetAsync(cloud_sums, 0, 2 * (size_t)B * sizeof(float), st));
+        if (B > 0 && normal_sums) PCL_CUDA(cudaMemsetAsync(normal_sums, 0, 2 * (size_t)B * sizeof(float), st));
         return PCL_OK;
     }
     const Pts xp{x, x_bs, x_rs, x_dtype}, yp{y, y_bs, y_rs, y_dtype};
     unsigned *ticket = (unsigned *)workspace;
     float *partial = (float *)((unsigned char *)workspace + 256);
     const int nblk = nblk_for(P1, P2);
+    const int maxP = P1 > P2 ? P1 : P2;
     PCL_CUDA(cudaMemsetAsync(ticket, 0, sizeof(unsigned), st));  // every CTA writes its partial (zeros beyond the shorter cloud); the last one sums
     const int pmin = P1 < P2 ? P1 : P2;
     if (D == 3 && prune_min() > 0 && pmin >= prune_min() && prune_bytes(B, P1, P2) > 0) {
         // large clouds: Morton order + tile boxes, then a nearest-neighbour scan that only visits the tiles that can matter
         const PruneWs W = prune_ws((unsigned char *)workspace + 256 + align_up((size_t)2 * B * nblk * sizeof(float), 256), B, P1, P2);
-        const int maxP = P1 > P2 ? P1 : P2;
         const size_t smem = (size_t)(PR_CELLS + 32) * sizeof(int) + (size_t)maxP * sizeof(unsigned);
         static thread_local int attr_dev = -1;
         int dev = 0;
@@ -795,16 +882,70 @@ extern "C" int pcl_chamfer_fwd(const void *x, int x_dtype, int64_t x_bs, int64_t
         PCL_CUDA(cudaGetLastError());
         const dim3 grid((maxP + PR_NN_WARPS * 32 - 1) / (PR_NN_WARPS * 32), B, 2);
         if (mode == PCL_CHAMFER_FMA)
-            chamfer_nn3_pruned_kernel<true><<<grid, PR_NN_WARPS * 32, 0, st>>>(x_len, y_len, P1, P2, W, dist_x, (int *)idx_x, dist_y, (int *)idx_y, partial, nblk, ticket, loss_xy);
+            chamfer_nn3_pruned_kernel<true><<<grid, PR_NN_WARPS * 32, 0, st>>>(x_len, y_len, P1, P2, W, dist_x, (int *)idx_x, dist_y, (int *)idx_y, partial, nblk, ticket, loss_xy, cloud_sums);
         else
-            chamfer_nn3_pruned_kernel<false><<<grid, PR_NN_WARPS * 32, 0, st>>>(x_len, y_len, P1, P2, W, dist_x, (int *)idx_x, dist_y, (int *)idx_y, partial, nblk, ticket, loss_xy);
-        PCL_CUDA(cudaGetLastError());
-        return PCL_OK;
+            chamfer_nn3_pruned_kernel<false><<<grid, PR_NN_WARPS * 32, 0, st>>>(x_len, y_len, P1, P2, W, dist_x, (int *)idx_x, dist_y, (int *)idx_y, partial, nblk, ticket, loss_xy, cloud_sums);
+    } else {
+        rc = (mode == PCL_CHAMFER_FMA)
+                 ? launch_fwd<true>(xp, x_len, yp, y_len, B, P1, P2, D, dist_x, idx_x, dist_y, idx_y, partial, nblk, ticket, loss_xy, cloud_sums, st)
+                 : launch_fwd<false>(xp, x_len, yp, y_len, B, P1, P2, D, dist_x, idx_x, dist_y, idx_y, partial, nblk, ticket, loss_xy, cloud_sums, st);
+        if (rc) return rc;
     }
-    rc = (mode == PCL_CHAMFER_FMA)
-             ? launch_fwd<true>(xp, x_len, yp, y_len, B, P1, P2, D, dist_x, idx_x, dist_y, idx_y, partial, nblk, ticket, loss_xy, st)
-             : launch_fwd<false>(xp, x_len, yp, y_len, B, P1, P2, D, dist_x, idx_x, dist_y, idx_y, partial, nblk, ticket, loss_xy, st);
+    PCL_CUDA(cudaGetLastError());
+    if (normal_sums) {
+        // a separate pass over the found neighbours: the search kernels' register budget stays as it is (DESIGN.md 3.2)
+        const Pts xn{x_nrm, x_nrm_bs, x_nrm_rs, x_nrm_dtype}, yn{y_nrm, y_nrm_bs, y_nrm_rs, y_nrm_dtype};
+        PCL_CUDA(cudaMemsetAsync(ticket, 0, sizeof(unsigned), st));
+        const dim3 grid((maxP + CH_THREADS - 1) / CH_THREADS, B, 2);
+        chamfer_normal_kernel<<<grid, CH_THREADS, 0, st>>>(xn, x_len, yn, y_len, P1, P2, idx_x, idx_y, partial, nblk, ticket, normal_sums);
+        PCL_CUDA(cudaGetLastError());
+    }
+    return PCL_OK;
+}
+
+extern "C" int pcl_chamfer_fwd(const void *x, int x_dtype, int64_t x_bs, int64_t x_rs, const int64_t *x_len,
+                               const void *y, int y_dtype, int64_t y_bs, int64_t y_rs, const int64_t *y_len, int B,
+                               int P1, int P2, int D, int mode, float *dist_x, int32_t *idx_x, float *dist_y,
+                               int32_t *idx_y, float *loss_xy, void *workspace, size_t workspace_bytes, void *stream) {
+    return pcl_chamfer_cloud_fwd(x, x_dtype, x_bs, x_rs, x_len, y, y_dtype, y_bs, y_rs, y_len, B, P1, P2, D, mode, dist_x, idx_x, dist_y,
+                                 idx_y, loss_xy, nullptr, nullptr, PCL_F32, 0, 0, nullptr, PCL_F32, 0, 0, nullptr, workspace, workspace_bytes,
+                                 stream);
+}
+
+// every backward entry point: the upstream gradients of the distances come from grad_cloud (per cloud), grad_out (device
+// float[2] of the batch means) or the immediates; grad_normal != nullptr adds the normal term's gradient
+static int chamfer_bwd_run(const void *x, int x_dtype, int64_t x_bs, int64_t x_rs, const int64_t *x_len, const void *y, int y_dtype,
+                           int64_t y_bs, int64_t y_rs, const int64_t *y_len, int B, int P1, int P2, int D, const int32_t *idx_x,
+                           const int32_t *idx_y, const float *grad_out, float g_imm_x, float g_imm_y, const float *grad_cloud,
+                           float *grad_x, float *grad_y, const Pts &xn, const Pts &yn, const float *grad_normal, float *grad_xn,
+                           float *grad_yn, cudaStream_t st, bool outputs_are_zero) {
+    int rc = check_args(x, x_dtype, y, y_dtype, B, P1, P2, D);
     if (rc) return rc;
+    if (B > 0 && ((P1 > 0 && (!grad_x || !idx_x)) || (P2 > 0 && (!grad_y || !idx_y)))) {
+        set_error("chamfer_bwd: null argument"); return PCL_E_ARG;
+    }
+    if (grad_normal && (!normals_ok(xn.p, xn.dtype, yn.p, yn.dtype, B, P1, P2) || (B > 0 && ((P1 > 0 && !grad_xn) || (P2 > 0 && !grad_yn))))) {
+        set_error("chamfer_bwd: grad_normal needs both normals arrays (fp32 / fp16 / bf16) and both normal gradients"); return PCL_E_ARG;
+    }
+    if (B == 0) return PCL_OK;
+    if (!outputs_are_zero) {
+        if (P1 > 0) PCL_CUDA(cudaMemsetAsync(grad_x, 0, (size_t)B * P1 * D * sizeof(float), st));
+        if (P2 > 0) PCL_CUDA(cudaMemsetAsync(grad_y, 0, (size_t)B * P2 * D * sizeof(float), st));
+    }
+    if (grad_normal) {
+        if (P1 > 0) PCL_CUDA(cudaMemsetAsync(grad_xn, 0, (size_t)B * P1 * 3 * sizeof(float), st));
+        if (P2 > 0) PCL_CUDA(cudaMemsetAsync(grad_yn, 0, (size_t)B * P2 * 3 * sizeof(float), st));
+    }
+    if (P1 == 0 || P2 == 0) return PCL_OK;
+    const Pts xp{x, x_bs, x_rs, x_dtype}, yp{y, y_bs, y_rs, y_dtype};
+    const int maxP = P1 > P2 ? P1 : P2;
+    dim3 grid((maxP + 255) / 256, B, 2);
+    if (grad_normal)
+        chamfer_bwd_kernel<true><<<grid, 256, 0, st>>>(xp, x_len, yp, y_len, B, P1, P2, D, idx_x, idx_y, grad_out, g_imm_x, g_imm_y, grad_cloud,
+                                                       grad_x, grad_y, xn, yn, grad_normal, grad_xn, grad_yn);
+    else
+        chamfer_bwd_kernel<false><<<grid, 256, 0, st>>>(xp, x_len, yp, y_len, B, P1, P2, D, idx_x, idx_y, grad_out, g_imm_x, g_imm_y, grad_cloud,
+                                                        grad_x, grad_y, xn, yn, nullptr, nullptr, nullptr);
     PCL_CUDA(cudaGetLastError());
     return PCL_OK;
 }
@@ -814,23 +955,9 @@ int pcl::chamfer_bwd_impl(const void *x, int x_dtype, int64_t x_bs, int64_t x_rs
                           int64_t y_bs, int64_t y_rs, const int64_t *y_len, int B, int P1, int P2, int D, const int32_t *idx_x,
                           const int32_t *idx_y, const float *grad_out, float g_imm_x, float g_imm_y, float *grad_x, float *grad_y,
                           cudaStream_t st, bool outputs_are_zero) {
-    int rc = check_args(x, x_dtype, y, y_dtype, B, P1, P2, D);
-    if (rc) return rc;
-    if (B > 0 && ((P1 > 0 && (!grad_x || !idx_x)) || (P2 > 0 && (!grad_y || !idx_y)))) {
-        set_error("chamfer_bwd: null argument"); return PCL_E_ARG;
-    }
-    if (B == 0) return PCL_OK;
-    if (!outputs_are_zero) {
-        if (P1 > 0) PCL_CUDA(cudaMemsetAsync(grad_x, 0, (size_t)B * P1 * D * sizeof(float), st));
-        if (P2 > 0) PCL_CUDA(cudaMemsetAsync(grad_y, 0, (size_t)B * P2 * D * sizeof(float), st));
-    }
-    if (P1 == 0 || P2 == 0) return PCL_OK;
-    const Pts xp{x, x_bs, x_rs, x_dtype}, yp{y, y_bs, y_rs, y_dtype};
-    const int maxP = P1 > P2 ? P1 : P2;
-    dim3 grid((maxP + 255) / 256, B, 2);
-    chamfer_bwd_kernel<<<grid, 256, 0, st>>>(xp, x_len, yp, y_len, B, P1, P2, D, idx_x, idx_y, grad_out, g_imm_x, g_imm_y, grad_x, grad_y);
-    PCL_CUDA(cudaGetLastError());
-    return PCL_OK;
+    const Pts none{nullptr, 0, 0, PCL_F32};
+    return chamfer_bwd_run(x, x_dtype, x_bs, x_rs, x_len, y, y_dtype, y_bs, y_rs, y_len, B, P1, P2, D, idx_x, idx_y, grad_out, g_imm_x, g_imm_y,
+                           nullptr, grad_x, grad_y, none, none, nullptr, nullptr, nullptr, st, outputs_are_zero);
 }
 
 extern "C" int pcl_chamfer_bwd(const void *x, int x_dtype, int64_t x_bs, int64_t x_rs, const int64_t *x_len,
@@ -840,4 +967,17 @@ extern "C" int pcl_chamfer_bwd(const void *x, int x_dtype, int64_t x_bs, int64_t
     if (!grad_out) { set_error("chamfer_bwd: null argument"); return PCL_E_ARG; }
     return chamfer_bwd_impl(x, x_dtype, x_bs, x_rs, x_len, y, y_dtype, y_bs, y_rs, y_len, B, P1, P2, D, idx_x, idx_y, grad_out, 0.f, 0.f,
                             grad_x, grad_y, (cudaStream_t)stream);
+}
+
+extern "C" int pcl_chamfer_cloud_bwd(const void *x, int x_dtype, int64_t x_bs, int64_t x_rs, const int64_t *x_len,
+                                     const void *y, int y_dtype, int64_t y_bs, int64_t y_rs, const int64_t *y_len, int B,
+                                     int P1, int P2, int D, const int32_t *idx_x, const int32_t *idx_y,
+                                     const float *grad_cloud, float *grad_x, float *grad_y,
+                                     const void *x_nrm, int x_nrm_dtype, int64_t x_nrm_bs, int64_t x_nrm_rs,
+                                     const void *y_nrm, int y_nrm_dtype, int64_t y_nrm_bs, int64_t y_nrm_rs,
+                                     const float *grad_normal, float *grad_x_nrm, float *grad_y_nrm, void *stream) {
+    if (B > 0 && !grad_cloud) { set_error("chamfer_bwd: null grad_cloud"); return PCL_E_ARG; }
+    const Pts xn{x_nrm, x_nrm_bs, x_nrm_rs, x_nrm_dtype}, yn{y_nrm, y_nrm_bs, y_nrm_rs, y_nrm_dtype};
+    return chamfer_bwd_run(x, x_dtype, x_bs, x_rs, x_len, y, y_dtype, y_bs, y_rs, y_len, B, P1, P2, D, idx_x, idx_y, nullptr, 0.f, 0.f,
+                           grad_cloud, grad_x, grad_y, xn, yn, grad_normal, grad_x_nrm, grad_y_nrm, (cudaStream_t)stream, false);
 }
