@@ -356,6 +356,36 @@ PCL_API int pcl_ball_query_bwd(const void *p1, int dtype1, int64_t bs1, int64_t 
                 int B, int P1, int P2, int D, int K, const int32_t *idx,
                 const float *grad_dists, float *grad_p1, float *grad_p2, void *stream);
 
+/* ------------------------------------------------------------------ normals and local frames -------------- */
+/*
+ * Replaces pytorch3d.ops.estimate_pointcloud_local_coord_frames / estimate_pointcloud_normals (0.7.2) forward and their
+ * autograd backward (third-party code, restated from memory [3P-memory]: parity with pytorch3d itself is unpinned).
+ * p (B,P,3) strided fp32 / fp16 / bf16 points, len nullable int64[B] (entries clamped to [0,P]), 1 <= K <= pcl_knn_max_k(),
+ * knn_idx (B,P,K) int32: what pcl_knn_fwd(p, p, len, len, K) wrote (read only; an entry outside [0, n_b) is clamped into it).
+ * For cloud b with n_b = len[b] points (P without len) and n_b > K, every point i < n_b with neighbours N_i = knn_idx[b,i,:]:
+ *   mu = mean_{j in N_i} p_j,  C = mean_{j in N_i} (p_j - mu)(p_j - mu)^T,  C = V diag(lam) V^T with lam ascending;
+ *   curvatures[b,i,:] = lam (B,P,3) fp32;  frames[b,i,:,c] = v_c (B,P,3,3) fp32, column c = eigenvector of lam_c.
+ *   disambiguate != 0: v0 and v2 are each negated when 2 * #{j in N_i : v . (p_j - p_i) > 0} < K, and column 1 is v0 x v2.
+ * All of it runs in fp64 on the up-cast coordinates (cyclic Jacobi until the off-diagonal is <= 2^-52 ||C||_F) and is
+ * rounded to fp32 once.  Rows i >= n_b, and every row of a cloud with n_b <= K, are 0.  Repeated eigenvalues give a finite,
+ * orthonormal, deterministic frame.  No atomics: results are bit-reproducible.  No workspace, no host synchronisation.
+ */
+PCL_API int pcl_frames_fwd(const void *p, int dtype, int64_t bs, int64_t rs, const int64_t *len,
+                int B, int P, int K, int disambiguate, const int32_t *knn_idx,
+                float *curvatures, float *frames, void *stream);
+/*
+ * Backward from the saved curvatures and frames and the upstream gradients grad_curvatures (B,P,3) and grad_frames (B,P,3,3)
+ * (DEVICE fp32, each nullable: NULL = zero).  With V = frames[b,i], lam = curvatures[b,i], M = V^T grad_frames[b,i] and
+ * F_ij = 1 / (lam_j - lam_i) for i != j, 0 on the diagonal (a term whose M_ij is exactly 0 is 0):
+ *   Cbar = V (diag(grad_curvatures[b,i]) + F o M) V^T,  grad_p[b,j] += (Cbar + Cbar^T) (p_j - mu) / K  for every j in N_i.
+ * The sign flips carry no gradient; column 1 of a disambiguated frame is the unit eigenvector of lam_1 and is treated as one.
+ * Equal eigenvalues whose vectors carry gradient give a non-finite gradient, as torch.linalg.eigh's backward does.
+ * grad_p (B,P,3) fp32 is overwritten: zero-filled on `stream`, then accumulated with fp32 atomics.
+ */
+PCL_API int pcl_frames_bwd(const void *p, int dtype, int64_t bs, int64_t rs, const int64_t *len,
+                int B, int P, int K, const int32_t *knn_idx, const float *curvatures, const float *frames,
+                const float *grad_curvatures, const float *grad_frames, float *grad_p, void *stream);
+
 /* ------------------------------------------------------------------ composite step ------------------------ */
 /*
  * One pass of the whole hot path over a batch that is already on the device: Chamfer fwd+bwd (upstream gradient 1)

@@ -12,6 +12,7 @@ from .emd_module import emdFunction, emdModule, emd_forward_raw, set_emd_path
 from .knn import knn_forward_raw, knn_gather, knn_points
 from .losses import (ChamferDistance, EarthMoverDistance, FilterClasses, FilteringChamferDistance,
                      SegmentingChamferDistance, chamfer_emd_loss)
+from .normals import estimate_pointcloud_local_coord_frames, estimate_pointcloud_normals, frames_forward_raw
 from .sampling import farthest_point_sample, fps_forward_raw, query_ball_point, sample_farthest_points
 from .sharded import ShardedChamferEmdStep, ShardedLoss, shard_bounds
 
@@ -21,4 +22,5 @@ __all__ = [
     "FilterClasses", "chamfer_emd_loss", "ShardedLoss", "ShardedChamferEmdStep", "shard_bounds",
     "farthest_point_sample", "sample_farthest_points", "fps_forward_raw", "query_ball_point", "knn_points", "knn_gather", "knn_forward_raw",
     "ball_query", "ball_query_forward_raw",
+    "estimate_pointcloud_normals", "estimate_pointcloud_local_coord_frames", "frames_forward_raw",
 ]

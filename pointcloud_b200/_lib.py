@@ -56,6 +56,8 @@ _SIGNATURES = {
     "pcl_knn_bwd": (c_int, _PTS + [c_void_p] + _PTS + [c_void_p] + [c_int] * 5 + [c_void_p] * 4 + [c_void_p]),
     "pcl_ball_query_fwd": (c_int, _PTS + [c_void_p] + _PTS + [c_void_p] + [c_int] * 5 + [c_float, c_int] + [c_void_p] * 2 + [c_void_p]),
     "pcl_ball_query_bwd": (c_int, _PTS + [c_void_p] + _PTS + [c_void_p] + [c_int] * 5 + [c_void_p] * 4 + [c_void_p]),
+    "pcl_frames_fwd": (c_int, _PTS + [c_void_p] + [c_int] * 4 + [c_void_p] * 3 + [c_void_p]),
+    "pcl_frames_bwd": (c_int, _PTS + [c_void_p] + [c_int] * 3 + [c_void_p] * 6 + [c_void_p]),
     "pcl_chamfer_emd_step_scratch_bytes":(c_size_t, [c_int, c_int]),
     "pcl_chamfer_emd_step": (c_int, _PTS + _PTS + [c_int, c_int, c_float, c_int, c_int] + [c_void_p] * 3 + [c_void_p, c_size_t, c_void_p]),
     "pcl_loss_host_scratch_bytes": (c_size_t, [c_int, c_int]),
