@@ -13,6 +13,8 @@ from .knn import knn_forward_raw, knn_gather, knn_points
 from .losses import (ChamferDistance, EarthMoverDistance, FilterClasses, FilteringChamferDistance,
                      SegmentingChamferDistance, chamfer_emd_loss)
 from .normals import estimate_pointcloud_local_coord_frames, estimate_pointcloud_normals, frames_forward_raw
+from .points_alignment import (ICPSolution, SimilarityTransform, corresponding_points_alignment, icp_forward_raw,
+                               iterative_closest_point, points_alignment_forward_raw)
 from .sampling import farthest_point_sample, fps_forward_raw, query_ball_point, sample_farthest_points
 from .sharded import ShardedChamferEmdStep, ShardedLoss, shard_bounds
 
@@ -23,4 +25,6 @@ __all__ = [
     "farthest_point_sample", "sample_farthest_points", "fps_forward_raw", "query_ball_point", "knn_points", "knn_gather", "knn_forward_raw",
     "ball_query", "ball_query_forward_raw",
     "estimate_pointcloud_normals", "estimate_pointcloud_local_coord_frames", "frames_forward_raw",
+    "corresponding_points_alignment", "iterative_closest_point", "SimilarityTransform", "ICPSolution", "icp_forward_raw",
+    "points_alignment_forward_raw",
 ]

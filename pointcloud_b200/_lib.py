@@ -18,6 +18,7 @@ PCL_CHAMFER_UNFUSED, PCL_CHAMFER_FMA = 0, 1
 _DTYPES = {torch.float32: PCL_F32, torch.float16: PCL_F16, torch.bfloat16: PCL_BF16}
 
 c_void_p, c_int, c_int64, c_size_t, c_float = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_size_t, ctypes.c_float
+c_double = ctypes.c_double
 
 _PTS = [c_void_p, c_int, c_int64, c_int64]  # pointer, dtype, batch stride, row stride
 _SIGNATURES = {
@@ -58,6 +59,12 @@ _SIGNATURES = {
     "pcl_ball_query_bwd": (c_int, _PTS + [c_void_p] + _PTS + [c_void_p] + [c_int] * 5 + [c_void_p] * 4 + [c_void_p]),
     "pcl_frames_fwd": (c_int, _PTS + [c_void_p] + [c_int] * 4 + [c_void_p] * 3 + [c_void_p]),
     "pcl_frames_bwd": (c_int, _PTS + [c_void_p] + [c_int] * 3 + [c_void_p] * 6 + [c_void_p]),
+    "pcl_points_alignment_workspace_bytes": (c_size_t, [c_int, c_int]),
+    "pcl_points_alignment_fwd": (c_int, _PTS + _PTS + [c_void_p] * 2 + [c_int] * 4 + [c_double] + [c_void_p] * 4 + [c_void_p, c_size_t, c_void_p]),
+    "pcl_points_alignment_bwd": (c_int, _PTS + _PTS + [c_void_p] * 2 + [c_int] * 3 + [c_double] + [c_void_p] * 7 + [c_void_p]),
+    "pcl_icp_workspace_bytes": (c_size_t, [c_int] * 4),
+    "pcl_icp": (c_int, _PTS + [c_void_p] + _PTS + [c_void_p] + [c_int] * 3 + [c_void_p] * 3 + [c_int, c_float, c_int, c_int, c_int]
+                + [c_void_p] * 6 + [c_void_p, c_size_t, c_void_p]),
     "pcl_chamfer_emd_step_scratch_bytes":(c_size_t, [c_int, c_int]),
     "pcl_chamfer_emd_step": (c_int, _PTS + _PTS + [c_int, c_int, c_float, c_int, c_int] + [c_void_p] * 3 + [c_void_p, c_size_t, c_void_p]),
     "pcl_loss_host_scratch_bytes": (c_size_t, [c_int, c_int]),

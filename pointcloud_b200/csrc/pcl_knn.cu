@@ -21,6 +21,7 @@
 #include <climits>
 
 #include "pcl_common.cuh"
+#include "pcl_nn.cuh"
 
 namespace pcl {
 namespace {
@@ -47,24 +48,7 @@ __device__ __forceinline__ float ld_pt(const Pts &a, int64_t i) {
     return (a.dtype == PCL_F16) ? __half2float(__ushort_as_half(h)) : __uint_as_float((unsigned)h << 16);
 }
 
-__device__ __forceinline__ u64 knn_key(float d, int j) {
-    const unsigned b = (d != d) ? 0x7fffffffu : __float_as_uint(d);
-    return ((u64)b << 32) | (unsigned)j;
-}
-__device__ __forceinline__ float key_dist(u64 k) { return __uint_as_float((unsigned)(k >> 32)); }  // KNN_NONE -> NaN
-
-// the Chamfer arithmetic (sqdist3 / chamfer_nnD_kernel of pcl_chamfer.cu): d = 0; per channel d = d + df*df or fma(df, df, d)
-template <bool FMA, int D>
-__device__ __forceinline__ float sqdist(const float (&q)[D], const float *t) {
-    float d = 0.f;
-#pragma unroll
-    for (int c = 0; c < D; c++) {
-        const float df = __fsub_rn(q[c], t[c]);
-        if constexpr (FMA) d = __fmaf_rn(df, df, d);
-        else d = __fadd_rn(d, __fmul_rn(df, df));
-    }
-    return d;
-}
+// knn_key, key_dist and sqdist<FMA, D>: pcl_nn.cuh (shared with pcl_icp.cu)
 
 // insert `key` (< my[K-1]) into the ascending list my[0], my[32], ..., my[32 (K-1)]; returns the new K-th key
 __device__ __forceinline__ u64 list_insert(u64 *my, int K, u64 key) {
