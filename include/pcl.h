@@ -450,6 +450,44 @@ PCL_API int pcl_icp(const void *x, int x_dtype, int64_t x_bs, int64_t x_rs, cons
                 int estimate_scale, int allow_reflection, int mode, float *Xt, float *R_hist, float *T_hist, float *s_hist,
                 float *rmse_hist, int32_t *status, void *workspace, size_t workspace_bytes, void *stream);
 
+/* ------------------------------------------------------------------ points to volumes -------------------- */
+/*
+ * Replaces pytorch3d.ops.add_points_features_to_volume_densities_features (0.7.2) forward, unscaled, and its autograd backward
+ * (third-party code, restated from memory [3P-memory]: parity with pytorch3d itself is unpinned; tests/volumes_ref.py is
+ * the specification).  points (B,P,3) and features (B,P,C), C >= 1, strided fp32 / fp16 / bf16 (pointer, dtype, batch
+ * stride, row stride); mask nullable fp32 (B,P), used as a weight m (1 without); grid_sizes nullable DEVICE int64 (B,3)
+ * = (D_b, H_b, W_b) (the padded D, H, W without); 0 <= D, H, W <= 2^24.  mode PCL_P2V_TRILINEAR or PCL_P2V_NEAREST.
+ * Per axis (x -> W, y -> H, z -> D) with cloud size S, in fp32 with every operation rounded:
+ *   t = ((p + 1) * (S - s) - o) * 0.5,   (s, o) = (1, 0) with align_corners, (0, 1) without.
+ * Trilinear: f = floor(t), r = t - f; corner f + d (d in {0,1}^3) has weight w = m * (wz * wy) * wx, w_a = d_a ? r_a : 1 - r_a.
+ * Nearest: the voxel roundf(t) (half away from zero), weight m.  A vote lands at [b, :, z, y, x] when 0 <= index <
+ * min(S_axis, padded axis) on every axis (tested in float: non-finite coordinates and 0 or oversize grid_sizes never index
+ * out of bounds) and w != 0; a point with m == 0 is skipped entirely.
+ *   volume_densities (B,1,D,H,W) += w;  volume_features (B,C,D,H,W)[c] += w * feature[c]
+ * Both volumes are contiguous fp32 and are accumulated into in place with fp32 reductions (red.global.add, subnormals
+ * flushed) in no fixed order: not bit-reproducible.  One launch; B = 0, P = 0 or an empty grid launch nothing.
+ */
+enum { PCL_P2V_TRILINEAR = 0, PCL_P2V_NEAREST = 1 };
+PCL_API int pcl_points_to_volumes_fwd(const void *points, int p_dtype, int64_t p_bs, int64_t p_rs,
+                const void *features, int f_dtype, int64_t f_bs, int64_t f_rs, const float *mask, const int64_t *grid_sizes,
+                int B, int P, int C, int D, int H, int W, int mode, int align_corners,
+                float *volume_densities, float *volume_features, void *stream);
+/*
+ * Backward.  grad_densities (B,1,D,H,W) and grad_features (B,C,D,H,W): contiguous DEVICE fp32, each nullable (NULL = zero).
+ * grad_points (B,P,3) and grad_point_features (B,P,C): dense fp32, each nullable (NULL = not computed), overwritten.
+ * With the forward's in-bounds corners v_k and weights w_k (zero-weight corners included):
+ *   grad_point_features[c] = sum_k w_k grad_features[c, v_k];
+ *   grad_points[a] = (S_a - s)/2 * sum_k dw_k/dt_a * (grad_densities[v_k] + sum_c feature[c] grad_features[c, v_k])
+ * (trilinear, floor convention dr/dt = 1); 0 in nearest mode.  Points with m == 0 get 0.  One thread per point sums in a
+ * fixed order in fp32 with no atomics: bit-reproducible, and a cloud's gradients do not depend on the rest of the batch.
+ * One launch, none when both outputs are NULL.
+ */
+PCL_API int pcl_points_to_volumes_bwd(const void *points, int p_dtype, int64_t p_bs, int64_t p_rs,
+                const void *features, int f_dtype, int64_t f_bs, int64_t f_rs, const float *mask, const int64_t *grid_sizes,
+                int B, int P, int C, int D, int H, int W, int mode, int align_corners,
+                const float *grad_densities, const float *grad_features, float *grad_points, float *grad_point_features,
+                void *stream);
+
 /* ------------------------------------------------------------------ composite step ------------------------ */
 /*
  * One pass of the whole hot path over a batch that is already on the device: Chamfer fwd+bwd (upstream gradient 1)

@@ -15,6 +15,7 @@ from .losses import (ChamferDistance, EarthMoverDistance, FilterClasses, Filteri
 from .normals import estimate_pointcloud_local_coord_frames, estimate_pointcloud_normals, frames_forward_raw
 from .points_alignment import (ICPSolution, SimilarityTransform, corresponding_points_alignment, icp_forward_raw,
                                iterative_closest_point, points_alignment_forward_raw)
+from .points_to_volumes import add_points_features_to_volume_densities_features, points_to_volumes_forward_raw
 from .sampling import farthest_point_sample, fps_forward_raw, query_ball_point, sample_farthest_points
 from .sharded import ShardedChamferEmdStep, ShardedLoss, shard_bounds
 
@@ -26,5 +27,5 @@ __all__ = [
     "ball_query", "ball_query_forward_raw",
     "estimate_pointcloud_normals", "estimate_pointcloud_local_coord_frames", "frames_forward_raw",
     "corresponding_points_alignment", "iterative_closest_point", "SimilarityTransform", "ICPSolution", "icp_forward_raw",
-    "points_alignment_forward_raw",
+    "points_alignment_forward_raw", "add_points_features_to_volume_densities_features", "points_to_volumes_forward_raw",
 ]

@@ -65,6 +65,8 @@ _SIGNATURES = {
     "pcl_icp_workspace_bytes": (c_size_t, [c_int] * 4),
     "pcl_icp": (c_int, _PTS + [c_void_p] + _PTS + [c_void_p] + [c_int] * 3 + [c_void_p] * 3 + [c_int, c_float, c_int, c_int, c_int]
                 + [c_void_p] * 6 + [c_void_p, c_size_t, c_void_p]),
+    "pcl_points_to_volumes_fwd": (c_int, _PTS + _PTS + [c_void_p] * 2 + [c_int] * 8 + [c_void_p] * 2 + [c_void_p]),
+    "pcl_points_to_volumes_bwd": (c_int, _PTS + _PTS + [c_void_p] * 2 + [c_int] * 8 + [c_void_p] * 4 + [c_void_p]),
     "pcl_chamfer_emd_step_scratch_bytes":(c_size_t, [c_int, c_int]),
     "pcl_chamfer_emd_step": (c_int, _PTS + _PTS + [c_int, c_int, c_float, c_int, c_int] + [c_void_p] * 3 + [c_void_p, c_size_t, c_void_p]),
     "pcl_loss_host_scratch_bytes": (c_size_t, [c_int, c_int]),
