@@ -25,7 +25,7 @@
 // Only the two largest values of a scan matter, so the expensive part (IEEE sqrt, two F2F conversions, two
 // DADDs -- the XU pipe runs at 16 lanes/clk/SM on B200 and bounds the reference's Bid) is evaluated only
 // for candidates that pass an exact-safe FP32 filter in the squared domain:
-//   skip k  <=>  s_k > (c_k - (T - margin))^2,  c_k = RU(3 - price_k) kept in the target tile's .w,
+//   skip k  <=>  s_k > u^2,  u = RU(c_k - RD(T - margin)),  c_k = RU(3 - price_k) kept in the target tile's .w,
 // where T is a proven lower bound of the bidder's final second-best value (its running second best, seeded
 // with the exact current values of the two objects it preferred at its previous bid); a whole tile is skipped with
 // the same inequality on bounds (distance to the tile's box, tile maximum of c).  Skipped candidates are strictly
@@ -293,7 +293,7 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                                     v2 = __shfl_sync(0xffffffffu, v, 2), v3 = __shfl_sync(0xffffffffu, v, 3);
                         const float hi01 = fmaxf(v0, v1), lo01 = fminf(v0, v1), hi23 = fmaxf(v2, v3), lo23 = fminf(v2, v3);
                         const float second = fmaxf(fminf(hi01, hi23), fmaxf(lo01, lo23));
-                        tm = __fsub_rn(second, FILTER_MARGIN);
+                        tm = filter_threshold(second);
                     }
                 }
                 float best = -1e9f, better = -1e9f;
@@ -321,7 +321,7 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                             const float4 tq = S.tgt[tix[i] * TILE + lane];
                             sq[i] = sq3_ref(__fsub_rn(tq.x, a.x), __fsub_rn(tq.y, a.y), __fsub_rn(tq.z, a.z));
                             cw[i] = tq.w;
-                            const float u = __fsub_rn(tq.w, tm);
+                            const float u = filter_u(tq.w, tm);
                             pass[i] = have[i] && !(__fmaf_rn(u, u, -sq[i]) < 0.f);
                             any |= pass[i];
                         }
@@ -385,11 +385,11 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                                 else if (vl > better) { k4 = k3; k3 = bi2; better = vl; bi2 = kl; }
                                 else { k4 = k3; k3 = kl; }
                             }
-                            tm = fmaxf(tm, __fsub_rn(better, FILTER_MARGIN));  // re-test the leftovers against the tightened threshold
+                            tm = fmaxf(tm, filter_threshold(better));  // re-test the leftovers against the tightened threshold
                             any = false;
 #pragma unroll
                             for (int i = 0; i < WC; i++) {
-                                const float u = __fsub_rn(cw[i], tm);
+                                const float u = filter_u(cw[i], tm);
                                 pass[i] = pass[i] && !(__fmaf_rn(u, u, -sq[i]) < 0.f);
                                 any |= pass[i];
                             }

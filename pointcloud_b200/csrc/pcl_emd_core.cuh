@@ -36,7 +36,7 @@ constexpr int TILE = 32;  // targets per spatial tile (one bounding box per tile
 constexpr int EMD_WPB_MAX = 6 * EMD_WARPS;  // at most this many bidders per CTA: warp-per-bidder scan (swept on config 2: 48..128)
 constexpr unsigned short NONE16 = 0xffffu;
 constexpr unsigned NOLAST = 0xffffffffu;
-constexpr float FILTER_MARGIN = 2e-6f;  // > 4.2e-7 worst-case rounding slack of the filter (DESIGN.md)
+constexpr float FILTER_MARGIN = 2e-6f;  // keeps T_m below T; the directed rounding below, not this size, makes skipping exact
 
 // flags of the launch (what fits into shared memory for this N)
 constexpr int EMD_F_SORT = 1;  // clouds are re-ordered along a Morton curve inside the kernel
@@ -133,6 +133,13 @@ __device__ __forceinline__ unsigned morton18(float3 p) {
     return spread6(qx) | (spread6(qy) << 1) | (spread6(qz) << 2);
 }
 
+// The skip rule of every Bid scan (DESIGN.md "Why skipping is exact"): for T a proven lower bound of the bidder's final second
+// best, c >= 3 - price and s (a lower bound of) the squared distance, u = filter_u(c, filter_threshold(T)) and
+// fma(u, u, -s) < 0 prove value < T.  Both subtractions round in the safe direction -- T_m down, u up -- so that the proof
+// needs no bound on the magnitude of coordinates, prices or values.
+__device__ __forceinline__ float filter_threshold(float T) { return __fsub_rd(T, FILTER_MARGIN); }
+__device__ __forceinline__ float filter_u(float c, float tm) { return __fsub_ru(c, tm); }
+
 struct Top2 {
     float best, better;  // emd_cuda.cu:112
     int bi, bi2;         // internal index of the bid (first argmax in ORIGINAL index order) and of the runner-up
@@ -149,16 +156,16 @@ __device__ __forceinline__ void top2_exact(const EmdSmem &S, Top2 &r, float s, i
     if (v > r.best || (v == r.best && ko < r.bio)) { r.k4 = r.k3; r.k3 = r.bi2; r.better = r.best; r.bi2 = r.bi; r.best = v; r.bi = k; r.bio = ko; }
     else if (v > r.better) { r.k4 = r.k3; r.k3 = r.bi2; r.better = v; r.bi2 = k; }
     else { r.k4 = r.k3; r.k3 = k; }
-    r.tm = fmaxf(r.tm, __fsub_rn(r.better, FILTER_MARGIN));
+    r.tm = fmaxf(r.tm, filter_threshold(r.better));
 }
 
-// One tile of 32 targets for the bidder at (ax,ay,az).  e = u*u - s with u = c_k - tm: e < 0 proves
+// One tile of 32 targets for the bidder at (ax,ay,az).  e = u*u - s with u = filter_u(c_k, tm): e < 0 proves
 // value_k < (final second best), so the candidate cannot change best / second best / argmax.
 __device__ __forceinline__ void scan_tile(const EmdSmem &S, int k0, float ax, float ay, float az, Top2 &r) {
 #define PCL_FILTER(T_, S_, E_)                                                                   \
     const float4 T_ = S.tgt[k_];                                                                 \
     const float S_ = sq3_ref(__fsub_rn(T_.x, ax), __fsub_rn(T_.y, ay), __fsub_rn(T_.z, az));     \
-    const float u_##E_ = __fsub_rn(T_.w, r.tm);                                                   \
+    const float u_##E_ = filter_u(T_.w, r.tm);                                                   \
     const float E_ = __fmaf_rn(u_##E_, u_##E_, -S_);
 #pragma unroll kScanUnroll
     for (int k = k0; k < k0 + TILE; k += 4) {
@@ -178,13 +185,13 @@ __device__ __forceinline__ void scan_tile(const EmdSmem &S, int k0, float ax, fl
 }
 
 // Can the whole tile be skipped for this bidder?  Lower bound of s over the tile = squared distance to the
-// tile's box (shrunk by 1e-6 relative against fp32 rounding of both sides), upper bound of c = tile max.
+// tile's box (the same monotone fp32 operations as s, shrunk by 1e-6 relative on top), upper bound of c = tile max.
 __device__ __forceinline__ bool tile_skippable(const float4 &lo, const float4 &hi, float ax, float ay, float az, float tm) {
     const float dx = fmaxf(fmaxf(__fsub_rn(lo.x, ax), __fsub_rn(ax, hi.x)), 0.f);
     const float dy = fmaxf(fmaxf(__fsub_rn(lo.y, ay), __fsub_rn(ay, hi.y)), 0.f);
     const float dz = fmaxf(fmaxf(__fsub_rn(lo.z, az), __fsub_rn(az, hi.z)), 0.f);
     const float d2 = __fmul_rn(__fmaf_rn(dz, dz, __fmaf_rn(dx, dx, __fmul_rn(dy, dy))), 0.999999f);
-    const float u = __fsub_rn(lo.w, tm);
+    const float u = filter_u(lo.w, tm);
     return (u < 0.f) || (__fmaf_rn(u, u, -d2) < 0.f);
 }
 
@@ -220,7 +227,7 @@ __device__ __forceinline__ float seed_threshold(const EmdSmem &S, unsigned lastp
             const float v = seed_value(S, k4, ax, ay, az);
             if (v > hi) { lo = hi; hi = v; } else if (v > lo) lo = v;
         }
-        tm = __fsub_rn(lo, FILTER_MARGIN);
+        tm = filter_threshold(lo);
     }
     return tm;
 }

@@ -114,7 +114,7 @@ __device__ __forceinline__ WarpBid warp_scan_bidder(const EmdSmem &S, int NT, fl
                 const float4 tq = S.tgt[tix[i] * TILE + lane];
                 sq[i] = sq3_ref(__fsub_rn(tq.x, ax), __fsub_rn(tq.y, ay), __fsub_rn(tq.z, az));
                 cw[i] = tq.w;
-                const float u = __fsub_rn(tq.w, tm);
+                const float u = filter_u(tq.w, tm);
                 pass[i] = have[i] && !(__fmaf_rn(u, u, -sq[i]) < 0.f);
                 any |= pass[i];
             }
@@ -172,11 +172,11 @@ __device__ __forceinline__ WarpBid warp_scan_bidder(const EmdSmem &S, int NT, fl
                     else if (vl > better) { k4 = k3; k3 = bi2; better = vl; bi2 = kl; }
                     else { k4 = k3; k3 = kl; }
                 }
-                tm = fmaxf(tm, __fsub_rn(better, FILTER_MARGIN));
+                tm = fmaxf(tm, filter_threshold(better));
                 any = false;
 #pragma unroll
                 for (int i = 0; i < WC; i++) {
-                    const float u = __fsub_rn(cw[i], tm);
+                    const float u = filter_u(cw[i], tm);
                     pass[i] = pass[i] && !(__fmaf_rn(u, u, -sq[i]) < 0.f);
                     any |= pass[i];
                 }

@@ -161,7 +161,7 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
                         const float v0 = __shfl_sync(0xffffffffu, v, 0), v1 = __shfl_sync(0xffffffffu, v, 1),
                                     v2 = __shfl_sync(0xffffffffu, v, 2), v3 = __shfl_sync(0xffffffffu, v, 3);
                         const float hi01 = fmaxf(v0, v1), lo01 = fminf(v0, v1), hi23 = fmaxf(v2, v3), lo23 = fminf(v2, v3);
-                        tm = __fsub_rn(fmaxf(fminf(hi01, hi23), fmaxf(lo01, lo23)), FILTER_MARGIN);
+                        tm = filter_threshold(fmaxf(fminf(hi01, hi23), fmaxf(lo01, lo23)));
                     }
                 }
                 const WarpBid w = warp_scan_bidder(S, NT, a.x, a.y, a.z, tm, my_evals);

@@ -1,9 +1,11 @@
 """EMD approximation module (auction algorithm) -- B200 drop-in for
 pointcloud_vision/loss/emd/emd_module.py (same names, arguments, outputs and gradient behaviour).
 
-Input:  xyz1, xyz2: [#batch, #points, 3]; xyz1 is the predicted cloud, xyz2 the ground truth, both
-        normalised to [0, 1] (emd_module.py:6-9).  Any CUDA float dtype / strided view is accepted
-        without a copy (the reference copies with .contiguous().float().cuda(), :43-44).
+Input:  xyz1, xyz2: [#batch, #points, 3]; xyz1 is the predicted cloud, xyz2 the ground truth.  Any finite
+        coordinates give the oracle's results bit for bit as long as pairwise distances stay below 1e9 (the
+        reference's initial bid value is -1e9); [0, 1] (emd_module.py:6-9) is only the range for which the
+        reference tuned eps.  Any CUDA float dtype / strided view is accepted without a copy (the reference copies
+        with .contiguous().float().cuda(), :43-44).
 Output: dist [#batch, #points] (squared distance to the match, fp32), assignment [#batch, #points]
         (int32 index into xyz2; not guaranteed to be a bijection, :16-19).
 Only xyz1 receives a gradient; xyz2 gets zeros; eps / iters get None (:63-72).
