@@ -89,10 +89,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
     bool told_workers = false;   // this cloud has no more exported iterations: said so once (rank 0)
     cluster.sync();  // every CTA's arrays exist before anyone writes remote bids
 
-    auto pred_xyz = [&](int jp) -> float3 {
-        if (S.x1) { const float4 q = S.x1[jp]; return make_float3(q.x, q.y, q.z); }
-        return ld_xyz(xyz1, cloud, S.pperm ? (int)S.pperm[jp] : jp);
-    };
     long long sum_u = 0;
     unsigned long long my_evals = 0ull;  // evaluations this lane really executed (tiles that were not skipped)
     int iters_run = 0, extra_qualifiers = 0, cur = 0;
@@ -102,26 +98,7 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
     for (int t = 0; t < iters; t++) {
         const bool last = (t == iters - 1);
         // ---- 1. list of unassigned bidders (emd_cuda.cu:23-93), ascending, identical in every CTA -------
-        if (t > 0 && (!have_list || (t & 3) == 0)) {  // prices moved in the previous iteration: refresh the per-tile upper bound of c (a stale, higher bound stays valid: with few bidders left only every fourth iteration)
-            for (int t0 = wid; t0 < NT; t0 += 4 * NW) {  // four independent tiles per trip
-                // warp maximum with one REDUX on an order-preserving integer image of the float (c may be negative: padding)
-                int b[4];
-#pragma unroll
-                for (int i = 0; i < 4; i++) {
-                    const int tl = min(t0 + i * NW, NT - 1);
-                    b[i] = __float_as_int(S.tgt[tl * TILE + lane].w);
-                    b[i] ^= (b[i] >> 31) & 0x7fffffff;
-                }
-#pragma unroll
-                for (int i = 0; i < 4; i++) b[i] = __reduce_max_sync(0xffffffffu, b[i]);
-#pragma unroll
-                for (int i = 0; i < 4; i++) {
-                    const int tl = t0 + i * NW;
-                    b[i] ^= (b[i] >> 31) & 0x7fffffff;
-                    if (lane == 0 && tl < NT) S.tlo[tl].w = __int_as_float(b[i]);
-                }
-            }
-        }
+        refresh_tile_bounds<THREADS>(S, NT, t, have_list);
         int U = 0;
         if (have_list) {
             // At most 32 bidders were left: warp 0 wrote the next list (the losers in list order, then the evicted owners)
@@ -252,7 +229,7 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                     unsigned short *const g_jp = reinterpret_cast<unsigned short *>(cl + W.o_jp);
                     for (int i = tid; i < Ux; i += T) {
                         const int jp = S.unass[Ud + i];
-                        const float3 a = pred_xyz(jp);
+                        const float3 a = pred_xyz(S, xyz1, cloud, jp);
                         unsigned lp = S.last[jp], lp34 = S.last34[jp];
                         if (flags & EMD_F_SORT) first_seeds(jp, N, lp, lp34);
                         g_brec[i] = make_float4(a.x, a.y, a.z, seed_threshold(S, lp, lp34, N, a.x, a.y, a.z));
@@ -270,32 +247,15 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
             }
         }
         if (wpb) {
-            // ---- few bidders: one WARP per bidder, one lane per target of a tile.  The tile tests are exact per
-            // bidder (no other lane's neighbourhood keeps a tile alive), 32 boxes are tested per ballot, and the
-            // rare candidates are folded into a warp-uniform top 2 in any order (the update is order-independent).
+            // ---- few bidders: one WARP per bidder, one lane per target of a tile: the scan of warp_scan_bidder (pcl_emd_tasks.cuh),
+            // written out here because routing it through the shared function slowed this kernel (profiles/r10_emd_shared_phases_ab.txt)
             for (int b = wid;;) {
                 if (b >= Uc) break;
                 const int jp = S.unass[pos(b)];
-                const float3 a = pred_xyz(jp);
+                const float3 a = pred_xyz(S, xyz1, cloud, jp);
                 unsigned lp = S.last[jp], lp34 = S.last34[jp];
                 if (flags & EMD_F_SORT) first_seeds(jp, N, lp, lp34);
-                float tm = -1e9f;
-                {
-                    const int k1 = (int)(lp & 0xffffu), k2 = (int)(lp >> 16);
-                    if (lp != NOLAST && k1 < N && k2 < N && k1 != k2) {  // seeds: lanes 0..3 evaluate up to four of them in parallel
-                        const int k3 = (int)(lp34 & 0xffffu), k4 = (int)(lp34 >> 16);
-                        const bool ok3 = k3 < N && k3 != k1 && k3 != k2, ok4 = k4 < N && k4 != k1 && k4 != k2 && k4 != k3;
-                        float v = -3e38f;
-                        const int ks = lane == 0 ? k1 : lane == 1 ? k2 : lane == 2 ? k3 : k4;
-                        if (lane < 2 || (lane == 2 && ok3) || (lane == 3 && ok4)) v = seed_value(S, ks, a.x, a.y, a.z);
-                        // second largest of the (up to) four values
-                        const float v0 = __shfl_sync(0xffffffffu, v, 0), v1 = __shfl_sync(0xffffffffu, v, 1),
-                                    v2 = __shfl_sync(0xffffffffu, v, 2), v3 = __shfl_sync(0xffffffffu, v, 3);
-                        const float hi01 = fmaxf(v0, v1), lo01 = fminf(v0, v1), hi23 = fmaxf(v2, v3), lo23 = fminf(v2, v3);
-                        const float second = fmaxf(fminf(hi01, hi23), fmaxf(lo01, lo23));
-                        tm = filter_threshold(second);
-                    }
-                }
+                float tm = warp_seed_threshold(S, lp, lp34, N, a.x, a.y, a.z);
                 float best = -1e9f, better = -1e9f;
                 int bi = -1, bi2 = -1, bio = 0x7fffffff, k3 = -1, k4 = -1;
                 for (int tb = 0; tb < NT; tb += 32) {
@@ -330,8 +290,6 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                             for (int i = 0; i < WC; i++) my_evals += have[i] ? TILE : 0;
                         }
                         if (!__any_sync(0xffffffffu, any)) continue;
-                        // Every lane takes ITS first surviving slot, so that one pass through the sqrt/F2F/DADD chain serves
-                        // all lanes (a lane rarely has two survivors among its 4 targets; leftovers loop).
                         do {
                             int sel = -1;
 #pragma unroll
@@ -347,11 +305,7 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
                             if (sel >= 0) { v = bid_value_exact(ssel, S.pf[ksel]); ko = S.tperm ? (int)S.tperm[ksel] : ksel; }
                             unsigned pm = __ballot_sync(0xffffffffu, sel >= 0);
                             if (__popc(pm) > 3) {
-                                // Many survivors (a weak threshold, e.g. after an eviction): only the two largest of them can change
-                                // (best, better), so pick those with warp reductions instead of folding every survivor serially.
-                                // Largest value, lowest ORIGINAL index among equal maxima; then the largest of the remaining lanes
-                                // (duplicates of the maximum count, as in the serial rule).  NaN never updates anything: left out.
-                                const float vc = __fadd_rn(v, 0.f);  // -0 -> +0: equal floats get equal keys
+                                const float vc = __fadd_rn(v, 0.f);
                                 int key = __float_as_int(vc);
                                 key ^= (key >> 31) & 0x7fffffff;
                                 if (!(sel >= 0 && vc == vc)) key = (int)0x80000000;
@@ -406,7 +360,7 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
         // bid slot, which nobody else touches before this CTA publishes that bid
         for (int b = tid; b < Uc; b += T) {
             const int jp = S.unass[pos(b)];
-            const float3 a = pred_xyz(jp);
+            const float3 a = pred_xyz(S, xyz1, cloud, jp);
             unsigned lp = S.last[jp], lp34 = S.last34[jp];
             if (flags & EMD_F_SORT) first_seeds(jp, N, lp, lp34);
             pub_cur[jp].y = __float_as_uint(seed_threshold(S, lp, lp34, N, a.x, a.y, a.z));
@@ -418,7 +372,7 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
             const int b = min(g * 32 + lane, Uc - 1);          // surplus lanes shadow the last bidder (results discarded)
             const bool active = (g * 32 + lane) < Uc;
             const int jp = S.unass[pos(b)];
-            const float3 a = pred_xyz(jp);
+            const float3 a = pred_xyz(S, xyz1, cloud, jp);
             Top2 r = top2_init(__uint_as_float(pub_cur[jp].y));
             const int ntl = (NT - sl + KS - 1) / KS;           // tiles of this slice: sl, sl+KS, ...
             const int home = min(max((__shfl_sync(0xffffffffu, jp, 0) / TILE - sl + KS / 2) / KS, 0), ntl - 1);
@@ -443,43 +397,7 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
         }
         }
         if (!wpb && KS > 1) {
-            __syncthreads();
-            // Tree merge of the KS slice partials of every bidder (log2 KS steps); same order-independent rule as
-            // top2_exact, i.e. the reference's ascending merge (emd_cuda.cu:165-173).
-            int span = 1;
-            while (span < KS) span <<= 1;
-            for (int st = span >> 1; st >= 1; st >>= 1) {
-                const int rows = min(st, KS - st);  // slices c in [0, rows) absorb slice c + st
-                for (int idx = tid; idx < rows * Uc; idx += T) {
-                    const int c = idx / Uc, b = idx - c * Uc;
-                    const int me = c * GS + b, ot = (c + st) * GS + b;
-                    float best = S.pbest[me], better = S.pbetter[me];
-                    unsigned pk = S.pbi[me], pk34 = S.pbi34[me];
-                    const float ob = S.pbest[ot], obt = S.pbetter[ot];
-                    const unsigned opk = S.pbi[ot];
-                    bool other_wins = ob > best;
-                    if (ob == best && (opk & 0xffffu) != 0xffffu) {
-                        const unsigned mine = pk & 0xffffu;
-                        if (mine == 0xffffu) other_wins = true;
-                        else {
-                            const unsigned mo = S.tperm ? S.tperm[mine] : mine, oo = S.tperm ? S.tperm[opk & 0xffffu] : (opk & 0xffffu);
-                            other_wins = oo < mo;
-                        }
-                    }
-                    if (other_wins) {
-                        const unsigned second = (best >= obt) ? (pk & 0xffffu) : (opk >> 16);
-                        better = fmaxf(best, obt);
-                        best = ob;
-                        pk = (opk & 0xffffu) | (second << 16);
-                        pk34 = S.pbi34[ot];  // also-rans of the slice that holds the best: spatially closest extra seeds
-                    } else if (ob > better) {
-                        better = ob;
-                        pk = (pk & 0xffffu) | ((opk & 0xffffu) << 16);
-                    }
-                    S.pbest[me] = best; S.pbetter[me] = better; S.pbi[me] = pk; S.pbi34[me] = pk34;
-                }
-                __syncthreads();
-            }
+            merge_slices<THREADS>(S, KS, Uc, GS);
             for (int b = tid; b < Uc; b += T) publish(S.unass[pos(b)], S.pbest[b], S.pbetter[b], S.pbi[b], S.pbi34[b]);
         }
         if constexpr (EXPORT) {
@@ -615,7 +533,7 @@ emd_auction_kernel(Pts xyz1, Pts xyz2, int N, float eps, int iters, int flags, i
         float d = 0.f;
         float3 gr = make_float3(0.f, 0.f, 0.f);
         if (k != NONE16) {
-            const float3 a = pred_xyz(jp);
+            const float3 a = pred_xyz(S, xyz1, cloud, jp);
             const float4 tp = S.tgt[k];
             const float dx = __fsub_rn(a.x, tp.x), dy = __fsub_rn(a.y, tp.y), dz = __fsub_rn(a.z, tp.z);
             d = sq3_ref(dx, dy, dz);

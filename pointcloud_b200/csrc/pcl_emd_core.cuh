@@ -231,10 +231,63 @@ __device__ __forceinline__ float seed_threshold(const EmdSmem &S, unsigned lastp
     }
     return tm;
 }
+// The same threshold for a bidder scanned by a whole warp: lanes 0..3 evaluate up to four seeds in parallel (warp-uniform result).
+__device__ __forceinline__ float warp_seed_threshold(const EmdSmem &S, unsigned lastpack, unsigned last34, int N, float ax, float ay, float az) {
+    const int lane = threadIdx.x & 31;
+    float tm = -1e9f;
+    const int k1 = (int)(lastpack & 0xffffu), k2 = (int)(lastpack >> 16);
+    if (lastpack != NOLAST && k1 < N && k2 < N && k1 != k2) {
+        const int k3 = (int)(last34 & 0xffffu), k4 = (int)(last34 >> 16);
+        const bool ok3 = k3 < N && k3 != k1 && k3 != k2, ok4 = k4 < N && k4 != k1 && k4 != k2 && k4 != k3;
+        float v = -3e38f;
+        const int ks = lane == 0 ? k1 : lane == 1 ? k2 : lane == 2 ? k3 : k4;
+        if (lane < 2 || (lane == 2 && ok3) || (lane == 3 && ok4)) v = seed_value(S, ks, ax, ay, az);
+        // second largest of the (up to) four values
+        const float v0 = __shfl_sync(0xffffffffu, v, 0), v1 = __shfl_sync(0xffffffffu, v, 1),
+                    v2 = __shfl_sync(0xffffffffu, v, 2), v3 = __shfl_sync(0xffffffffu, v, 3);
+        const float hi01 = fmaxf(v0, v1), lo01 = fminf(v0, v1), hi23 = fmaxf(v2, v3), lo23 = fminf(v2, v3);
+        tm = filter_threshold(fmaxf(fminf(hi01, hi23), fmaxf(lo01, lo23)));
+    }
+    return tm;
+}
 __device__ __forceinline__ Top2 top2_init(float tm) {
     Top2 r;
     r.best = -1e9f; r.better = -1e9f; r.bi = -1; r.bi2 = -1; r.bio = 0x7fffffff; r.k3 = -1; r.k4 = -1; r.tm = tm;
     return r;
+}
+
+// prediction jp (internal index) of the cloud: from the shared-memory copy, else from global memory / L2
+__device__ __forceinline__ float3 pred_xyz(const EmdSmem &S, const Pts &xyz1, int cloud, int jp) {
+    if (S.x1) { const float4 q = S.x1[jp]; return make_float3(q.x, q.y, q.z); }
+    return ld_xyz(xyz1, cloud, S.pperm ? (int)S.pperm[jp] : jp);
+}
+
+// Start of iteration t: prices moved in the previous iteration, so refresh the per-tile upper bound of c.  A stale, higher bound
+// stays valid, so with at most 32 bidders left (have_list) only every fourth iteration does it.
+template <int THREADS>
+__device__ __forceinline__ void refresh_tile_bounds(const EmdSmem &S, int NT, int t, bool have_list) {
+    constexpr int NW = THREADS / 32;
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    if (t > 0 && (!have_list || (t & 3) == 0)) {
+        for (int t0 = wid; t0 < NT; t0 += 4 * NW) {  // four independent tiles per trip
+            // warp maximum with one REDUX on an order-preserving integer image of the float (c may be negative: padding)
+            int b[4];
+#pragma unroll
+            for (int i = 0; i < 4; i++) {
+                const int tl = min(t0 + i * NW, NT - 1);
+                b[i] = __float_as_int(S.tgt[tl * TILE + lane].w);
+                b[i] ^= (b[i] >> 31) & 0x7fffffff;
+            }
+#pragma unroll
+            for (int i = 0; i < 4; i++) b[i] = __reduce_max_sync(0xffffffffu, b[i]);
+#pragma unroll
+            for (int i = 0; i < 4; i++) {
+                const int tl = t0 + i * NW;
+                b[i] ^= (b[i] >> 31) & 0x7fffffff;
+                if (lane == 0 && tl < NT) S.tlo[tl].w = __int_as_float(b[i]);
+            }
+        }
+    }
 }
 
 // Set-up of one CTA's replica (emd_module.py:45-56 + the internal order): both clouds in Morton order, target tiles with their

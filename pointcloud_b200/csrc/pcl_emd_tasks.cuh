@@ -84,8 +84,9 @@ __device__ __forceinline__ void copy16_out(void *dst, const void *src, int n16) 
     for (int i = threadIdx.x; i < n16; i += (int)blockDim.x) reinterpret_cast<uint4 *>(dst)[i] = reinterpret_cast<const uint4 *>(src)[i];
 }
 
-// One bidder scanned by one warp, one lane per target of a tile (the warp-per-bidder mode of pcl_emd.cu): 32 boxes per ballot, up to
-// PCL_WPB_CHUNK candidate tiles per step, rare filter survivors folded into a warp-uniform top two.  Returns the bid of the bidder.
+// One bidder scanned by one warp, one lane per target of a tile (the warp-per-bidder mode, for few bidders): 32 boxes per ballot, up
+// to PCL_WPB_CHUNK candidate tiles per step, rare filter survivors folded into a warp-uniform top two in any order (the update is
+// order-independent).  The tile tests are exact per bidder: no other lane's neighbourhood keeps a tile alive.  Returns the bid.
 struct WarpBid { float best, better; int bi, bi2, k3, k4; };
 __device__ __forceinline__ WarpBid warp_scan_bidder(const EmdSmem &S, int NT, float ax, float ay, float az, float tm, unsigned long long &my_evals) {
     const int lane = threadIdx.x & 31;
@@ -97,14 +98,14 @@ __device__ __forceinline__ WarpBid warp_scan_bidder(const EmdSmem &S, int NT, fl
         if (tl < NT) cand = !tile_skippable(S.tlo[tl], S.thi[tl], ax, ay, az, tm);
         unsigned cm = __ballot_sync(0xffffffffu, cand);
         constexpr int WC = PCL_WPB_CHUNK;
-        while (cm) {
+        while (cm) {  // up to WC candidate tiles per step: WC independent filter chains per lane, one vote
             int tix[WC];
             bool have[WC];
 #pragma unroll
             for (int i = 0; i < WC; i++) {
                 have[i] = cm != 0;
                 tix[i] = tb + (have[i] ? __ffs(cm) - 1 : 0);
-                cm &= cm - 1;
+                cm &= cm - 1;  // cm == 0 stays 0
             }
             float sq[WC], cw[WC];
             bool pass[WC];
@@ -123,6 +124,8 @@ __device__ __forceinline__ WarpBid warp_scan_bidder(const EmdSmem &S, int NT, fl
                 for (int i = 0; i < WC; i++) my_evals += have[i] ? TILE : 0;
             }
             if (!__any_sync(0xffffffffu, any)) continue;
+            // Every lane takes ITS first surviving slot, so that one pass through the sqrt/F2F/DADD chain serves all lanes (a lane
+            // rarely has two survivors among its targets; leftovers loop).
             do {
                 int sel = -1;
 #pragma unroll
@@ -137,8 +140,12 @@ __device__ __forceinline__ WarpBid warp_scan_bidder(const EmdSmem &S, int NT, fl
                 int ko = 0;
                 if (sel >= 0) { v = bid_value_exact(ssel, S.pf[ksel]); ko = S.tperm ? (int)S.tperm[ksel] : ksel; }
                 unsigned pm = __ballot_sync(0xffffffffu, sel >= 0);
-                if (__popc(pm) > 3) {  // many survivors: only the two largest can change (best, better)
-                    const float vc = __fadd_rn(v, 0.f);
+                if (__popc(pm) > 3) {
+                    // Many survivors (a weak threshold, e.g. after an eviction): only the two largest of them can change (best,
+                    // better), so pick those with warp reductions instead of folding every survivor serially.  Largest value, lowest
+                    // ORIGINAL index among equal maxima; then the largest of the remaining lanes (duplicates of the maximum count, as
+                    // in the serial rule).  NaN never updates anything: left out.
+                    const float vc = __fadd_rn(v, 0.f);  // -0 -> +0: equal floats get equal keys
                     int key = __float_as_int(vc);
                     key ^= (key >> 31) & 0x7fffffff;
                     if (!(sel >= 0 && vc == vc)) key = (int)0x80000000;
@@ -172,7 +179,7 @@ __device__ __forceinline__ WarpBid warp_scan_bidder(const EmdSmem &S, int NT, fl
                     else if (vl > better) { k4 = k3; k3 = bi2; better = vl; bi2 = kl; }
                     else { k4 = k3; k3 = kl; }
                 }
-                tm = fmaxf(tm, filter_threshold(better));
+                tm = fmaxf(tm, filter_threshold(better));  // re-test the leftovers against the tightened threshold
                 any = false;
 #pragma unroll
                 for (int i = 0; i < WC; i++) {
@@ -203,10 +210,52 @@ __device__ __forceinline__ TaskHdr task_policy(int U, bool wpb, int tasks_target
     return h;
 }  // bidders of the iteration, bidders per task, tile slices per group, scan mode
 
+// Tree merge of the KS slice partials of nb bidders (log2 KS steps, slots b, GS + b, ...): the same order-independent rule as
+// top2_exact, i.e. the reference's ascending merge (emd_cuda.cu:165-173).  Leaves the bid of bidder b in slot b.  Starts and ends
+// with a barrier.
+template <int THREADS>
+__device__ __forceinline__ void merge_slices(const EmdSmem &S, int KS, int nb, int GS) {
+    __syncthreads();
+    int span = 1;
+    while (span < KS) span <<= 1;
+    for (int st = span >> 1; st >= 1; st >>= 1) {
+        const int rows = min(st, KS - st);  // slices c in [0, rows) absorb slice c + st
+        for (int idx = threadIdx.x; idx < rows * nb; idx += THREADS) {
+            const int c = idx / nb, b = idx - c * nb;
+            const int me = c * GS + b, ot = (c + st) * GS + b;
+            float best = S.pbest[me], better = S.pbetter[me];
+            unsigned pk = S.pbi[me], pk34 = S.pbi34[me];
+            const float ob = S.pbest[ot], obt = S.pbetter[ot];
+            const unsigned opk = S.pbi[ot];
+            bool other_wins = ob > best;
+            if (ob == best && (opk & 0xffffu) != 0xffffu) {
+                const unsigned mine = pk & 0xffffu;
+                if (mine == 0xffffu) other_wins = true;
+                else {
+                    const unsigned mo = S.tperm ? S.tperm[mine] : mine, oo = S.tperm ? S.tperm[opk & 0xffffu] : (opk & 0xffffu);
+                    other_wins = oo < mo;
+                }
+            }
+            if (other_wins) {
+                const unsigned second = (best >= obt) ? (pk & 0xffffu) : (opk >> 16);
+                better = fmaxf(best, obt);
+                best = ob;
+                pk = (opk & 0xffffu) | (second << 16);
+                pk34 = S.pbi34[ot];  // also-rans of the slice that holds the best: spatially closest extra seeds
+            } else if (ob > better) {
+                better = ob;
+                pk = (pk & 0xffffu) | ((opk & 0xffffu) << 16);
+            }
+            S.pbest[me] = best; S.pbetter[me] = better; S.pbi[me] = pk; S.pbi34[me] = pk34;
+        }
+        __syncthreads();
+    }
+}
+
 // One task of a cloud's Bid phase, executed by a whole CTA whose shared memory holds the cloud's targets / prices / boxes (the
 // owner's replica or a worker's copy of the mirror): TB consecutive bidders of the list.  mode 0: lane-per-bidder -- groups of 32
 // neighbouring bidders, every group scanned in KS tile slices (TB/32*KS work items for the 16 warps, dynamic queue, slice partials
-// merged by the tree of pcl_emd.cu == emd_cuda.cu:165-173).  mode 1: warp-per-bidder -- one bidder per warp at a time.
+// merged by merge_slices).  mode 1: warp-per-bidder -- one bidder per warp at a time.
 // Bids go to pub[list position] = {object | second << 16, increment bits, third | fourth << 16, 0}.
 template <int THREADS>
 __device__ __forceinline__ void team_run_task(const EmdSmem &S, int NT, float eps, const TaskHdr &h, int task,
@@ -265,41 +314,7 @@ __device__ __forceinline__ void team_run_task(const EmdSmem &S, int NT, float ep
         it = __shfl_sync(0xffffffffu, it, 0);
     }
     if (KS > 1) {
-        __syncthreads();
-        int span = 1;
-        while (span < KS) span <<= 1;
-        for (int st = span >> 1; st >= 1; st >>= 1) {
-            const int rows = min(st, KS - st);  // slices c in [0, rows) absorb slice c + st
-            for (int idx = tid; idx < rows * nb; idx += THREADS) {
-                const int c = idx / nb, b = idx - c * nb;
-                const int me = c * GS + b, ot = (c + st) * GS + b;
-                float best = S.pbest[me], better = S.pbetter[me];
-                unsigned pk = S.pbi[me], pk34 = S.pbi34[me];
-                const float ob = S.pbest[ot], obt = S.pbetter[ot];
-                const unsigned opk = S.pbi[ot];
-                bool other_wins = ob > best;
-                if (ob == best && (opk & 0xffffu) != 0xffffu) {
-                    const unsigned mine = pk & 0xffffu;
-                    if (mine == 0xffffu) other_wins = true;
-                    else {
-                        const unsigned mo = S.tperm ? S.tperm[mine] : mine, oo = S.tperm ? S.tperm[opk & 0xffffu] : (opk & 0xffffu);
-                        other_wins = oo < mo;
-                    }
-                }
-                if (other_wins) {
-                    const unsigned second = (best >= obt) ? (pk & 0xffffu) : (opk >> 16);
-                    better = fmaxf(best, obt);
-                    best = ob;
-                    pk = (opk & 0xffffu) | (second << 16);
-                    pk34 = S.pbi34[ot];
-                } else if (ob > better) {
-                    better = ob;
-                    pk = (pk & 0xffffu) | ((opk & 0xffffu) << 16);
-                }
-                S.pbest[me] = best; S.pbetter[me] = better; S.pbi[me] = pk; S.pbi34[me] = pk34;
-            }
-            __syncthreads();
-        }
+        merge_slices<THREADS>(S, KS, nb, GS);
         for (int b = tid; b < nb; b += THREADS)
             pub[b0 + b] = make_uint4(S.pbi[b], __float_as_uint(__fadd_rn(__fsub_rn(S.pbest[b], S.pbetter[b]), eps)), S.pbi34[b], 0u);
     }

@@ -52,10 +52,6 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
     copy16_out(g_pf, S.pf, n32 / 4);
     if (S.tperm) copy16_out(cl + W.o_tperm, S.tperm, n8 / 8);
 
-    auto pred_xyz = [&](int jp) -> float3 {
-        if (S.x1) { const float4 q = S.x1[jp]; return make_float3(q.x, q.y, q.z); }
-        return ld_xyz(xyz1, cloud, S.pperm ? (int)S.pperm[jp] : jp);
-    };
     long long sum_u = 0;
     unsigned long long my_evals = 0ull;
     int iters_run = 0, extra_qualifiers = 0;
@@ -67,25 +63,7 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
     for (int t = 0; t < iters; t++) {
         const bool last = (t == iters - 1);
         // ---- 1. list of unassigned bidders (emd_cuda.cu:23-93) and the per-tile upper bound of c ----------------
-        if (t > 0 && (!have_list || (t & 3) == 0)) {
-            for (int t0 = wid; t0 < NT; t0 += 4 * EMD_WARPS) {
-                int b[4];
-#pragma unroll
-                for (int i = 0; i < 4; i++) {
-                    const int tl = min(t0 + i * EMD_WARPS, NT - 1);
-                    b[i] = __float_as_int(S.tgt[tl * TILE + lane].w);
-                    b[i] ^= (b[i] >> 31) & 0x7fffffff;
-                }
-#pragma unroll
-                for (int i = 0; i < 4; i++) b[i] = __reduce_max_sync(0xffffffffu, b[i]);
-#pragma unroll
-                for (int i = 0; i < 4; i++) {
-                    const int tl = t0 + i * EMD_WARPS;
-                    b[i] ^= (b[i] >> 31) & 0x7fffffff;
-                    if (lane == 0 && tl < NT) S.tlo[tl].w = __int_as_float(b[i]);
-                }
-            }
-        }
+        refresh_tile_bounds<EMD_THREADS>(S, NT, t, have_list);
         int U = 0;
         if (have_list) {
             U = S.wsum[40];
@@ -146,24 +124,10 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
             for (int b = wid;;) {
                 if (b >= U) break;
                 const int jp = S.unass[b];
-                const float3 a = pred_xyz(jp);
+                const float3 a = pred_xyz(S, xyz1, cloud, jp);
                 unsigned lp = S.last[jp], lp34 = S.last34[jp];
                 if (flags & EMD_F_SORT) first_seeds(jp, N, lp, lp34);
-                float tm = -1e9f;
-                {
-                    const int k1 = (int)(lp & 0xffffu), k2 = (int)(lp >> 16);
-                    if (lp != NOLAST && k1 < N && k2 < N && k1 != k2) {  // seeds: lanes 0..3 evaluate up to four of them in parallel
-                        const int k3 = (int)(lp34 & 0xffffu), k4 = (int)(lp34 >> 16);
-                        const bool ok3 = k3 < N && k3 != k1 && k3 != k2, ok4 = k4 < N && k4 != k1 && k4 != k2 && k4 != k3;
-                        float v = -3e38f;
-                        const int ks = lane == 0 ? k1 : lane == 1 ? k2 : lane == 2 ? k3 : k4;
-                        if (lane < 2 || (lane == 2 && ok3) || (lane == 3 && ok4)) v = seed_value(S, ks, a.x, a.y, a.z);
-                        const float v0 = __shfl_sync(0xffffffffu, v, 0), v1 = __shfl_sync(0xffffffffu, v, 1),
-                                    v2 = __shfl_sync(0xffffffffu, v, 2), v3 = __shfl_sync(0xffffffffu, v, 3);
-                        const float hi01 = fmaxf(v0, v1), lo01 = fminf(v0, v1), hi23 = fmaxf(v2, v3), lo23 = fminf(v2, v3);
-                        tm = filter_threshold(fmaxf(fminf(hi01, hi23), fmaxf(lo01, lo23)));
-                    }
-                }
+                float tm = warp_seed_threshold(S, lp, lp34, N, a.x, a.y, a.z);
                 const WarpBid w = warp_scan_bidder(S, NT, a.x, a.y, a.z, tm, my_evals);
                 if (lane == 0) {
                     pub_cur[jp] = make_uint2((unsigned)(w.bi & 0xffff) | ((unsigned)(w.bi2 & 0xffff) << 16),
@@ -178,7 +142,7 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
             // bidder records {x, y, z, seed threshold} by list position + the internal index (scan start hint) ...
             for (int b = tid; b < U; b += T) {
                 const int jp = S.unass[b];
-                const float3 a = pred_xyz(jp);
+                const float3 a = pred_xyz(S, xyz1, cloud, jp);
                 unsigned lp = S.last[jp], lp34 = S.last34[jp];
                 if (flags & EMD_F_SORT) first_seeds(jp, N, lp, lp34);
                 g_brec[b] = make_float4(a.x, a.y, a.z, seed_threshold(S, lp, lp34, N, a.x, a.y, a.z));
@@ -296,7 +260,7 @@ emd_team_kernel(Pts xyz1, Pts xyz2, int B, int N, float eps, int iters, int flag
         float d = 0.f;
         float3 gr = make_float3(0.f, 0.f, 0.f);
         if (k != NONE16) {
-            const float3 a = pred_xyz(jp);
+            const float3 a = pred_xyz(S, xyz1, cloud, jp);
             const float4 tp = S.tgt[k];
             const float dx = __fsub_rn(a.x, tp.x), dy = __fsub_rn(a.y, tp.y), dz = __fsub_rn(a.z, tp.z);
             d = sq3_ref(dx, dy, dz);
