@@ -490,6 +490,71 @@ PCL_API int pcl_points_to_volumes_bwd(const void *points, int p_dtype, int64_t p
                 const float *grad_densities, const float *grad_features, float *grad_points, float *grad_point_features,
                 void *stream);
 
+/* ------------------------------------------------------------------ rasterize points / compositing -------- */
+/*
+ * Replaces pytorch3d.renderer.points.rasterize_points (0.7.2) forward and its autograd backward (third-party code, restated
+ * from memory [3P-memory]: parity with pytorch3d itself is unpinned; tests/raster_ref.py is the specification).
+ * points (B,P,3) strided fp32 / fp16 / bf16 in NDC (+X left, +Y up, +Z away); lengths nullable int64[B] (entries clamped to
+ * [0,P]); radius nullable DEVICE fp32 (B,P) contiguous, one radius per point, else radius_scalar for every point.
+ * B*P < 2^31, B <= 65535, 1 <= H, W <= 16384, 1 <= K <= pcl_raster_max_k() (150).
+ * Pixel (row r, column c) has the fp32 centre xf = ndc(W-1-c, W, H), yf = ndc(H-1-r, H, W), with
+ *   ndc(i, S1, S2) = -off + (range*i + off) / S1,  range = S1 > S2 ? (S1*2)/S2 : 2,  off = range/2,
+ * every operation rounded (no contraction).  Point i of cloud b hits it when i < lengths[b], x, y, z and r are finite,
+ * z >= 0 and d2 = (xf-x)*(xf-x) + (yf-y)*(yf-y) <= r*r (fp32, every operation rounded).  The pixel keeps the K hits of
+ * smallest key (z + 0, i) (so -0.0 ties +0.0 and the index decides), ascending:
+ *   idx (B,H,W,K) int32 = offset_b + i with offset_b = sum of lengths[0..b-1] (b*P without lengths): pytorch3d's packed index;
+ *   zbuf (B,H,W,K) fp32 = z;  dists (B,H,W,K) fp32 = d2;  unused slots -1 in all three.
+ * The key is a total order, so the outputs are bit-identical whatever bin_size and max_points_per_bin are, and a cloud's
+ * outputs do not depend on the rest of the batch (apart from offset_b).
+ * bin_size = 0: one launch; each 16 x TH pixel block scans its whole cloud.  bin_size > 0 (a multiple of 16, else PCL_E_ARG):
+ * a memset and two launches; a coarse pass puts every point into each bin_size x bin_size pixel bin its conservative box
+ * reaches, at most max_points_per_bin per (cloud, bin) (<= 0: max(10000, P/5), as pytorch3d; never more than P), and the
+ * fine pass reads its bin -- or, when the bin overflowed, the whole cloud.  Overflow costs time only: no error, no host read.
+ * Workspace: pcl_rasterize_points_workspace_bytes(B, P, H, W, bin_size, max_points_per_bin) (0 for bin_size = 0), else
+ * PCL_E_WORKSPACE.  The call can be captured in a CUDA graph.
+ */
+PCL_API int pcl_raster_max_k(void);
+PCL_API size_t pcl_rasterize_points_workspace_bytes(int B, int P, int H, int W, int bin_size, int max_points_per_bin);
+PCL_API int pcl_rasterize_points_fwd(const void *points, int dtype, int64_t bs, int64_t rs, const int64_t *lengths,
+                const float *radius, float radius_scalar, int B, int P, int H, int W, int K, int bin_size,
+                int max_points_per_bin, int32_t *idx, float *zbuf, float *dists, void *workspace, size_t workspace_bytes,
+                void *stream);
+/*
+ * Backward through zbuf and dists (each grad nullable = zero; DEVICE fp32 (B,H,W,K) contiguous): for every slot whose idx is
+ * offset_b + i with 0 <= i < lengths[b] (other values, -1 included, are skipped),
+ *   grad_points[b,i,2] += grad_zbuf;  grad_points[b,i,0:2] += 2*grad_dists*(p_xy - pixel_xy)
+ * with the forward's fp32 pixel centre.  grad_points (B,P,3) dense fp32 is zero-filled (one memset) and accumulated with
+ * fp32 red.add by one thread per (pixel, slot): not bit-reproducible.  A memset and at most one launch.
+ */
+PCL_API int pcl_rasterize_points_bwd(const void *points, int dtype, int64_t bs, int64_t rs, const int64_t *lengths, int B,
+                int P, int H, int W, int K, const int32_t *idx, const float *grad_zbuf, const float *grad_dists,
+                float *grad_points, void *stream);
+/*
+ * Replaces pytorch3d.renderer.compositing's alpha_composite / norm_weighted_sum / weighted_sum and their backward
+ * [3P-memory].  idx (N,K,H,W) int32 (idx_int64 = 0) or int64 (1), alphas (N,K,H,W) fp32 and features (C, P_total) fp32 are
+ * read through their element strides (idx_strides_host / alpha_strides_host: 4 HOST int64, feature_strides_host: 2 HOST
+ * int64), so permuted views need no copy.  out (N,C,H,W) contiguous fp32.  A slot with idx < 0 or idx >= P_total
+ * contributes nothing.  Sums in fp32 in slot order, every operation rounded:
+ *   WEIGHTED:       out = sum_k a_k F[:, idx_k]
+ *   NORM_WEIGHTED:  out = sum_k (a_k F[:, idx_k]) / w,  w = max(sum of the valid a_k, 1e-4)
+ *   ALPHA:          out = sum_k ((T_k a_k) F[:, idx_k]),  T_0 = 1, T_{k+1} = T_k (1 - a_k) over every slot, valid or not.
+ * One launch, one thread per (pixel, 4 channels): bit-reproducible.
+ */
+enum { PCL_COMPOSITE_ALPHA = 0, PCL_COMPOSITE_NORM_WEIGHTED = 1, PCL_COMPOSITE_WEIGHTED = 2 };
+PCL_API int pcl_composite_fwd(int mode, const void *idx, int idx_int64, const int64_t *idx_strides_host, const float *alphas,
+                const int64_t *alpha_strides_host, const float *features, const int64_t *feature_strides_host, int N, int K,
+                int H, int W, int C, int64_t P_total, float *out, void *stream);
+/*
+ * Backward: grad_out (N,C,H,W) contiguous fp32.  grad_alphas (N,K,H,W) contiguous fp32, nullable, written by one thread per
+ * pixel with no atomics (the alpha derivative is formed from products of (1 - a_t), never by dividing by 1 - a_k, so a = 1
+ * stays finite); grad_features (C, P_total) contiguous fp32, nullable, zero-filled (one memset) and accumulated with fp32
+ * red.add.  At most a memset and one launch.
+ */
+PCL_API int pcl_composite_bwd(int mode, const void *idx, int idx_int64, const int64_t *idx_strides_host, const float *alphas,
+                const int64_t *alpha_strides_host, const float *features, const int64_t *feature_strides_host, int N, int K,
+                int H, int W, int C, int64_t P_total, const float *grad_out, float *grad_alphas, float *grad_features,
+                void *stream);
+
 /* ------------------------------------------------------------------ composite step ------------------------ */
 /*
  * One pass of the whole hot path over a batch that is already on the device: Chamfer fwd+bwd (upstream gradient 1)

@@ -16,6 +16,8 @@ from .normals import estimate_pointcloud_local_coord_frames, estimate_pointcloud
 from .points_alignment import (ICPSolution, SimilarityTransform, corresponding_points_alignment, icp_forward_raw,
                                iterative_closest_point, points_alignment_forward_raw)
 from .points_to_volumes import add_points_features_to_volume_densities_features, points_to_volumes_forward_raw
+from .compositing import alpha_composite, composite_forward_raw, norm_weighted_sum, weighted_sum
+from .rasterize_points import rasterize_points, rasterize_points_backward_raw, rasterize_points_forward_raw
 from .sampling import farthest_point_sample, fps_forward_raw, query_ball_point, sample_farthest_points
 from .sharded import ShardedChamferEmdStep, ShardedLoss, shard_bounds
 
@@ -28,4 +30,6 @@ __all__ = [
     "estimate_pointcloud_normals", "estimate_pointcloud_local_coord_frames", "frames_forward_raw",
     "corresponding_points_alignment", "iterative_closest_point", "SimilarityTransform", "ICPSolution", "icp_forward_raw",
     "points_alignment_forward_raw", "add_points_features_to_volume_densities_features", "points_to_volumes_forward_raw",
+    "rasterize_points", "rasterize_points_forward_raw", "rasterize_points_backward_raw", "alpha_composite", "norm_weighted_sum",
+    "weighted_sum", "composite_forward_raw",
 ]

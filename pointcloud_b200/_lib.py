@@ -67,6 +67,12 @@ _SIGNATURES = {
                 + [c_void_p] * 6 + [c_void_p, c_size_t, c_void_p]),
     "pcl_points_to_volumes_fwd": (c_int, _PTS + _PTS + [c_void_p] * 2 + [c_int] * 8 + [c_void_p] * 2 + [c_void_p]),
     "pcl_points_to_volumes_bwd": (c_int, _PTS + _PTS + [c_void_p] * 2 + [c_int] * 8 + [c_void_p] * 4 + [c_void_p]),
+    "pcl_raster_max_k": (c_int, []),
+    "pcl_rasterize_points_workspace_bytes": (c_size_t, [c_int] * 6),
+    "pcl_rasterize_points_fwd": (c_int, _PTS + [c_void_p, c_void_p, c_float] + [c_int] * 7 + [c_void_p] * 3 + [c_void_p, c_size_t, c_void_p]),
+    "pcl_rasterize_points_bwd": (c_int, _PTS + [c_void_p] + [c_int] * 5 + [c_void_p] * 4 + [c_void_p]),
+    "pcl_composite_fwd": (c_int, [c_int, c_void_p, c_int] + [c_void_p] * 5 + [c_int] * 5 + [c_int64, c_void_p, c_void_p]),
+    "pcl_composite_bwd": (c_int, [c_int, c_void_p, c_int] + [c_void_p] * 5 + [c_int] * 5 + [c_int64] + [c_void_p] * 4),
     "pcl_chamfer_emd_step_scratch_bytes":(c_size_t, [c_int, c_int]),
     "pcl_chamfer_emd_step": (c_int, _PTS + _PTS + [c_int, c_int, c_float, c_int, c_int] + [c_void_p] * 3 + [c_void_p, c_size_t, c_void_p]),
     "pcl_loss_host_scratch_bytes": (c_size_t, [c_int, c_int]),

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.environ.get("PCL_LIB_OVERRIDE") or os.path.join(HERE, "libpcl_b200.so")  # override: development A/B builds
-SOURCES = ["pcl_api.cu", "pcl_chamfer.cu", "pcl_emd.cu", "pcl_emd_team.cu", "pcl_epilogue.cu", "pcl_sampling.cu", "pcl_knn.cu", "pcl_normals.cu", "pcl_icp.cu", "pcl_volumes.cu"]
+SOURCES = ["pcl_api.cu", "pcl_chamfer.cu", "pcl_emd.cu", "pcl_emd_team.cu", "pcl_epilogue.cu", "pcl_sampling.cu", "pcl_knn.cu", "pcl_normals.cu", "pcl_icp.cu", "pcl_volumes.cu", "pcl_raster.cu"]
 HEADERS = [os.path.join(CSRC, "pcl_common.cuh"), os.path.join(CSRC, "pcl_nn.cuh"), os.path.join(CSRC, "pcl_emd_core.cuh"), os.path.join(CSRC, "pcl_emd_tasks.cuh"), os.path.join(HERE, "..", "include", "pcl.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr"]
